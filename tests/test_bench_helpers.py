@@ -1,5 +1,5 @@
 """Host-side helpers of bench.py: the algorithmic-byte formula of SURVEY.md section 8(d), the DOF-balanced x-slab
-cut, and the nvidia-smi clock sampler's parsing. No GPU."""
+cut, the nvidia-smi clock sampler's parsing and the files of --dump-outputs. No GPU."""
 import importlib.util
 import os
 
@@ -51,3 +51,33 @@ def test_clock_sampler_summary_parses_nvidia_smi_rows():
     assert out["reasons"] == ["sw_power_cap"]                      # the sample outside the timed window is ignored
     s.samples = []
     assert s.summary(0, 1)["samples"] == 0
+
+
+def test_dump_outputs_sample_is_fixed_and_fits(tmp_path):
+    """--dump-outputs: outputs of two builds are compared row for row, so the sample must not depend on the run."""
+    assert np.array_equal(bench.dump_rows(1000, 16), np.arange(1000))
+    n = 50_000_000                                                  # ~ pillbox-256 B-field rows
+    rows = bench.dump_rows(n, 8)
+    assert np.array_equal(rows, bench.dump_rows(n, 8))
+    assert len(rows) * 8 <= bench.DUMP_BYTES < 64 << 20
+    assert rows[0] >= 0 and rows[-1] < n and np.all(np.diff(rows) > 0)
+    y = np.array([[1 + 2j], [3 - 4j]])
+    bench.write_outputs(str(tmp_path / "d"), {"y": y, "ev": [2.5, 7.0]})
+    got = np.load(tmp_path / "d" / "y.npy")
+    assert got.dtype == np.float64 and got.shape == (2, 1, 2) and np.array_equal(got[..., 0] + 1j * got[..., 1], y)
+    assert np.load(tmp_path / "d" / "ev.npy").tolist() == [2.5, 7.0]
+
+
+def test_dump_outputs_slabs_concatenate_to_the_global_sample(orc):
+    """Every rank dumps the sampled rows of its slab; rank 0 concatenates the pieces in rank order."""
+    n = 16
+    sim = orc.pillbox(n)
+    gids = sim.map("bfield")
+    n_global = sim.num_global("bfield")
+    y = np.arange(len(gids), dtype=np.float64) * 3.0 + 1.0     # stands for the global y = A x
+    rows = bench.dump_rows(len(gids), bench.DUMP_BYTES // (len(gids) // 3))
+    assert 0 < len(rows) < len(gids)                           # a real sample, not every row
+    for nranks in (1, 2, 3, 4):
+        cuts = bench.slab_ranges(gids, n_global, nranks, n)
+        pieces = [y[r0:r1][bench.slab_dump_rows(rows, r0, r1)] for r0, r1 in zip(cuts, cuts[1:])]
+        assert np.array_equal(np.concatenate(pieces), y[rows])
