@@ -6,7 +6,6 @@
 // This translation unit is compiled with -fmad=false: the reference's host code rounds a*b+c twice, and the generated
 // matrices have to carry the very same doubles for the SpMV parity gate to hold downstream.
 #include <algorithm>
-#include <cstdlib>
 #include <cstring>
 #include <string>
 
@@ -127,8 +126,9 @@ extern "C" {
 
 // MxCrsMatrix::fillComplete for an operator assembled on the device (MxCrsMatrix.cpp:325-342): the rows this rank's
 // row map owns become a device operator (pattern dictionary / sliced ELL, halo plan) without the host ever seeing
-// them: the layout is built by kernels too (mxg::crsCreateFromDevice). MXG_LAYOUT_BUILD=host sends the rows through
-// the host layout builder of mxg_crs_create instead (same result; kept for comparison).
+// them: the layout is built by kernels too (mxg::crsCreateFromDevice). A domain map that is not a run of the column
+// field map, and ordered maps, take the host CSR route instead: the rows are downloaded and mxg_crs_create_opts lays
+// them out with the same kernels.
 int mxg_crs_create_from_dcsr(mxg_map* row_map, mxg_map* domain_map, const mxg_dcsr* a, int layout, mxg_crs** out) {
   const CsrHandle* A = reinterpret_cast<const CsrHandle*>(a);
   MXG_REQUIRE(row_map && domain_map && A && out, "mxg_crs_create_from_dcsr: NULL argument");
@@ -160,16 +160,13 @@ int mxg_crs_create_from_dcsr(mxg_map* row_map, mxg_map* domain_map, const mxg_dc
       domIsRun = c0 + domain_map->nLocal <= int64_t(colG.size()) &&
                  std::memcmp(colG.data() + c0, domain_map->gids.data(), size_t(domain_map->nLocal) * sizeof(int64_t)) == 0;
     }
-    const char* how = std::getenv("MXG_LAYOUT_BUILD");
-    const bool onDevice = !(how && std::strcmp(how, "host") == 0) && domIsRun && row_map->perm.empty() && domain_map->perm.empty();
-    if (onDevice) {
-      // layout built on the device (mxg_spmv.cu: hash-table pattern dictionary, sliced ELL, inverse diagonal as kernels)
+    if (domIsRun && row_map->perm.empty() && domain_map->perm.empty()) {
       const int64_t* rp = (A->isComplex ? A->c.rowptr : A->r.rowptr) + r0;
       const int32_t* col = A->isComplex ? A->c.col : A->r.col;
       const void* val = A->isComplex ? static_cast<const void*>(A->c.val) : static_cast<const void*>(A->r.val);
       return mxg::crsCreateFromDevice(row_map, domain_map, rp, col, val, c0, int64_t(colG.size()), colG.data(), A->isComplex, layout, out);
     }
-    // MXG_LAYOUT_BUILD=host (or maps the device builder does not take): the rows pass through the host layout builder
+    // maps the device front end does not take: the rows pass through the host CSR entry point
     const int64_t n = r1 - r0;
     std::vector<int64_t> rowptr(static_cast<size_t>(n) + 1, 0);
     int rc = mxg_dcsr_download(a, r0, r1, rowptr.data(), nullptr, nullptr);

@@ -1,5 +1,5 @@
 // Exclusive prefix scan of int32 counts into int64 offsets (three passes: chunk totals, scan of the totals in one
-// block, scan inside every chunk). Set-up code of the operator assembly and of the device layout builder.
+// block, scan inside every chunk). Set-up code of the operator assembly and of the layout builder.
 #pragma once
 #include <algorithm>
 

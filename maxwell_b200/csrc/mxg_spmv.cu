@@ -1,6 +1,6 @@
 // libmxgpu: sparse operator apply (K1/K2/K4/K16/K20 of SURVEY.md section 2.3).
 //
-// Device layout ("pattern-compressed sliced ELL"), built from host CSR in mxg_crs_create:
+// Device layout ("pattern-compressed sliced ELL"), built by mxg_crs_create (host CSR) and mxg_crs_create_from_dcsr (device CSR):
 //
 //  * Dictionary rows. On a Yee grid almost every row of an assembled operator repeats the
 //    same stencil: identical values and identical column offsets relative to the row.
@@ -21,7 +21,6 @@
 #include <algorithm>
 #include <cstdlib>
 #include <cstring>
-#include <unordered_map>
 
 #include "mxg_internal.h"
 #include "mxg_ilv_model.h"
@@ -221,7 +220,7 @@ __global__ void __launch_bounds__(kBlock) k_spmm_dict(int64_t rowBegin, int64_t 
 // Same rows, different thread -> row assignment for maps whose DOFs come in component triples (GID = comp + 3 cell,
 // the B/E fields): warp w of a 96-row tile takes rows tile + 3 lane + (w mod 3), i.e. 32 consecutive CELLS of ONE field
 // component. All lanes then share one pattern (one broadcast wavefront per entry instead of ~3) and gather x from one
-// neighbourhood instead of three. Chosen per matrix at build time (mxg_crs::ilv), see buildImpl.
+// neighbourhood instead of three. Chosen per matrix at build time (mxg_crs::ilv), see planKernels.
 constexpr int kBlockIlv = 384;   // 4 tiles of 3 warps
 template <class T, bool GHOST, int NV>
 __global__ void __launch_bounds__(kBlockIlv) k_spmm_dict_ilv3(int64_t rowBegin, int64_t rowEnd, DictArgs<T> D,
@@ -1139,7 +1138,7 @@ int planHalo(mxg_crs* A, const std::vector<int64_t>& ghosts, const std::vector<i
 }
 
 // Kernel plans that depend on the row -> pattern map: thread -> row interleave of the gather kernels and the x windows of
-// the windowed kernel. Shared by the host layout builder and the device one (which hands in a host copy of rowPat).
+// the windowed kernel. The layout back end hands in host copies of the row -> pattern map and the pattern table.
 template <class T>
 int planKernels(mxg_crs* A, const std::vector<int32_t>& rowPat, const std::vector<int32_t>& patOff, const std::vector<PatEntry<T>>& pat) {
   mxg_ctx* ctx = A->ctx;
@@ -1201,275 +1200,12 @@ int planKernels(mxg_crs* A, const std::vector<int32_t>& rowPat, const std::vecto
   return rc;
 }
 
-template <class T>
-int buildImpl(mxg_crs* A, const int64_t* rowptr, const int64_t* colGids, const double* valsIn, int layout) {
-  mxg_ctx* ctx = A->ctx;
-  constexpr int w = sizeof(T) / sizeof(double);
-  const T* vals = reinterpret_cast<const T*>(valsIn);
-  const int64_t nRows = A->nRows, nLoc = A->nLoc;
-  const int64_t nnzIn = rowptr[nRows];
-  const mxg_map* dom = A->domMap;
-  MXG_REQUIRE(dom->nGlobal < (int64_t(1) << 31), "mxg_crs_create: global size must fit in 31 bits");
-
-  // GID -> local id of the domain map
-  std::vector<int32_t> lookup(size_t(dom->nGlobal), -1);
-  for (int64_t i = 0; i < nLoc; ++i) lookup[dom->gids[i]] = int32_t(i);
-  const int64_t domLo = nLoc ? dom->gids.front() : 0, domHi = nLoc ? dom->gids.back() : -1;
-
-  // ghosts = referenced GIDs that are not local
-  std::vector<int64_t> ghosts;
-  for (int64_t q = 0; q < nnzIn; ++q) {
-    const int64_t g = colGids[q];
-    MXG_REQUIRE(g >= 0 && g < dom->nGlobal, "mxg_crs_create: column GID %lld out of range", (long long)g);
-    if (lookup[g] < 0) ghosts.push_back(g);
-  }
-  std::sort(ghosts.begin(), ghosts.end());
-  ghosts.erase(std::unique(ghosts.begin(), ghosts.end()), ghosts.end());
-  MXG_REQUIRE(ghosts.empty() || ctx->nranks > 1, "mxg_crs_create: column GID %lld is not in the domain map",
-              (long long)(ghosts.empty() ? 0 : ghosts[0]));
-  A->gLo = int64_t(std::lower_bound(ghosts.begin(), ghosts.end(), domLo) - ghosts.begin());
-  if (nLoc == 0) A->gLo = 0;
-  A->gHi = int64_t(ghosts.size()) - A->gLo;
-  int rc = planHalo(A, ghosts, lookup, domLo, domHi);
-  if (rc) return rc;
-
-  // extended local column index of every entry; rows sorted, duplicates merged
-  std::vector<int64_t> rp(nRows + 1, 0);
-  std::vector<int32_t> ext;
-  std::vector<T> val;
-  ext.reserve(nnzIn);
-  val.reserve(nnzIn);
-  std::vector<uint8_t> needsGhost(nRows, 0);
-  std::vector<std::pair<int32_t, T>> rowBuf;
-  for (int64_t r = 0; r < nRows; ++r) {
-    rowBuf.clear();
-    bool sorted = true;
-    for (int64_t q = rowptr[r]; q < rowptr[r + 1]; ++q) {
-      const int64_t g = colGids[q];
-      int32_t e = lookup[g];
-      if (e < 0) {
-        const int64_t pos = std::lower_bound(ghosts.begin(), ghosts.end(), g) - ghosts.begin();
-        e = pos < A->gLo ? int32_t(pos - A->gLo) : int32_t(nLoc + (pos - A->gLo));
-        needsGhost[r] = 1;
-      }
-      if (!rowBuf.empty() && e <= rowBuf.back().first) sorted = false;
-      rowBuf.emplace_back(e, vals[q]);
-    }
-    if (!sorted) {
-      std::stable_sort(rowBuf.begin(), rowBuf.end(), [](auto& a, auto& b) { return a.first < b.first; });
-      size_t o = 0;
-      for (size_t i = 0; i < rowBuf.size();) {
-        T s = rowBuf[i].second;
-        size_t j = i + 1;
-        while (j < rowBuf.size() && rowBuf[j].first == rowBuf[i].first) s = s + rowBuf[j++].second;
-        rowBuf[o++] = {rowBuf[i].first, s};
-        i = j;
-      }
-      rowBuf.resize(o);
-    }
-    for (auto& t : rowBuf) { ext.push_back(t.first); val.push_back(t.second); }
-    rp[r + 1] = int64_t(ext.size());
-  }
-  A->nnz = int64_t(ext.size());
-  // Ordered maps (mxg_map_create_ordered): rows move to their device positions and owned columns are translated; the
-  // entry order inside a row stays the reference's ascending local column, so sums keep Epetra's order bit for bit.
-  if (!A->rowMap->perm.empty() || !A->domMap->perm.empty()) {
-    MXG_REQUIRE(ctx->nranks == 1 && ghosts.empty(), "mxg_crs_create: ordered maps are supported on single-rank contexts only");
-    std::vector<int32_t> rowPerm = A->rowMap->perm, colInv = A->domMap->inv;
-    if (rowPerm.empty()) { rowPerm.resize(size_t(nRows)); for (int64_t i = 0; i < nRows; ++i) rowPerm[size_t(i)] = int32_t(i); }
-    if (colInv.empty()) { colInv.resize(size_t(nLoc)); for (int64_t i = 0; i < nLoc; ++i) colInv[size_t(i)] = int32_t(i); }
-    std::vector<int64_t> rp2;
-    std::vector<int32_t> ext2;
-    std::vector<T> val2;
-    try {
-      mxg::permuteCsr(rp, ext, val, rowPerm, colInv, nLoc, rp2, ext2, val2);
-    } catch (const std::exception& e) {   // nothing may unwind through the C boundary
-      MXG_REQUIRE(false, "mxg_crs_create: %s", e.what());
-    }
-    rp.swap(rp2);
-    ext.swap(ext2);
-    val.swap(val2);
-  }
-  for (int64_t r = 0; r < nRows; ++r) A->ghostRows += needsGhost[r];
-
-  // interior range = longest run of rows without ghost needs
-  {
-    int64_t bestB = 0, bestE = 0, runB = 0;
-    for (int64_t r = 0; r <= nRows; ++r)
-      if (r == nRows || needsGhost[r]) {
-        if (r - runB > bestE - bestB) { bestB = runB; bestE = r; }
-        runB = r + 1;
-      }
-    A->intBegin = bestB;
-    A->intEnd = bestE;
-  }
-
-  // ---- pattern dictionary ---------------------------------------------------------------
-  std::vector<int32_t> rowPat(nRows, -1);
-  std::vector<int32_t> patOff(1, 0);
-  std::vector<PatEntry<T>> pat;
-  // Rectangular operators on two different maps (div, grad, curl, the multigrid transfers) have no translation-invariant
-  // rows -- column minus row index drifts with the row -- so the dictionary pass would hash tens of millions of unique
-  // rows for nothing: they go straight to sliced ELL.
-  const bool sameMaps = A->rowMap == A->domMap || A->rowMap->gids == A->domMap->gids;
-  if (layout != 1 && sameMaps) {
-    std::unordered_map<uint64_t, std::vector<int32_t>> table;  // hash -> candidate pattern ids
-    table.reserve(1 << 16);
-    struct Cand { int64_t row; int32_t count; };
-    std::vector<Cand> cands;
-    std::vector<int32_t> rowCand(nRows, -1);
-    auto sameRow = [&](int64_t a, int64_t b) {
-      const int64_t la = rp[a + 1] - rp[a];
-      if (la != rp[b + 1] - rp[b]) return false;
-      for (int64_t k = 0; k < la; ++k) {
-        if (ext[rp[a] + k] - a != ext[rp[b] + k] - b) return false;
-        if (std::memcmp(&val[rp[a] + k], &val[rp[b] + k], sizeof(T)) != 0) return false;
-      }
-      return true;
-    };
-    for (int64_t r = 0; r < nRows; ++r) {
-      const int64_t len = rp[r + 1] - rp[r];
-      if (len == 0) continue;  // empty rows go to the general path (y = 0)
-      uint64_t h = mix64(0x1234567ull, uint64_t(len));
-      for (int64_t k = rp[r]; k < rp[r + 1]; ++k) {
-        h = mix64(h, uint64_t(int64_t(ext[k]) - r));
-        uint64_t bits[w];
-        std::memcpy(bits, &val[k], sizeof(T));
-        for (int t = 0; t < w; ++t) h = mix64(h, bits[t]);
-      }
-      auto& bucket = table[h];
-      int32_t found = -1;
-      for (int32_t c : bucket)
-        if (sameRow(cands[c].row, r)) { found = c; break; }
-      if (found < 0) {
-        found = int32_t(cands.size());
-        cands.push_back({r, 0});
-        bucket.push_back(found);
-      }
-      cands[found].count++;
-      rowCand[r] = found;
-    }
-    const int minCount = 4;
-    std::vector<int32_t> candToPat(cands.size(), -1);
-    // most frequent patterns first: the leading ones ride in the kernel parameter block
-    std::vector<size_t> order(cands.size());
-    for (size_t c = 0; c < cands.size(); ++c) order[c] = c;
-    std::stable_sort(order.begin(), order.end(), [&](size_t a, size_t b) { return cands[a].count > cands[b].count; });
-    for (size_t c : order) {
-      if (cands[c].count < minCount) continue;
-      candToPat[c] = int32_t(patOff.size() - 1);
-      const int64_t r = cands[c].row;
-      for (int64_t k = rp[r]; k < rp[r + 1]; ++k) {
-        PatEntry<T> e;
-        std::memset(&e, 0, sizeof(e));
-        std::memcpy(&e, &val[k], sizeof(T));
-        e.d = int32_t(int64_t(ext[k]) - r);
-        pat.push_back(e);
-      }
-      patOff.push_back(int32_t(pat.size()));
-    }
-    for (int64_t r = 0; r < nRows; ++r)
-      if (rowCand[r] >= 0 && candToPat[rowCand[r]] >= 0) { rowPat[r] = candToPat[rowCand[r]]; A->dictRows++; }
-  }
-  A->numPats = int64_t(patOff.size()) - 1;
-  A->patEntries = int64_t(pat.size());
-  // (A constant-bank copy of the most frequent patterns was tried and removed: 0.351 ms vs 0.305 ms per apply on
-  // pillbox-256 -- a warp holds ~3 different patterns and divergent LDC replays cost more than L1 broadcast loads;
-  // the 16 KB parameter block also lengthened every launch. profiles/README_r01.md.)
-
-  if ((rc = planKernels<T>(A, rowPat, patOff, pat))) return rc;
-
-  // ---- general rows in sliced ELL; the three row classes (leading boundary, interior,
-  // trailing boundary) each start on a slice boundary so they can be launched separately
-  std::vector<int32_t> genRow, genLen;
-  auto appendClass = [&](int64_t b, int64_t e) {
-    for (int64_t r = b; r < e; ++r)
-      if (rowPat[r] < 0) { genRow.push_back(int32_t(r)); genLen.push_back(int32_t(rp[r + 1] - rp[r])); }
-    while (genRow.size() % 32) { genRow.push_back(-1); genLen.push_back(0); }
-  };
-  appendClass(0, A->intBegin);
-  A->genIntBegin = int64_t(genRow.size());
-  appendClass(A->intBegin, A->intEnd);
-  A->genIntEnd = int64_t(genRow.size());
-  appendClass(A->intEnd, nRows);
-  A->nGen = int64_t(genRow.size());
-  const int64_t nSlices = A->nGen / 32;
-  std::vector<int64_t> slicePtr(nSlices + 1, 0);
-  for (int64_t s = 0; s < nSlices; ++s) {
-    int32_t wmax = 0;
-    for (int l = 0; l < 32; ++l) wmax = std::max(wmax, genLen[s * 32 + l]);
-    slicePtr[s + 1] = slicePtr[s] + int64_t(wmax) * 32;
-  }
-  A->ellEntries = slicePtr[nSlices];
-  std::vector<int32_t> ellCol(A->ellEntries, 0);
-  std::vector<T> ellVal(A->ellEntries, zeroOf<T>());
-  for (int64_t sIdx = 0; sIdx < nSlices; ++sIdx) {
-    // padding entries point at a column some real entry of the slice uses, so the kernel may
-    // load through them unconditionally (their value is 0 and they are skipped in the sum)
-    int32_t fallback = 0;
-    bool have = false;
-    for (int l = 0; l < 32 && !have; ++l) {
-      const int64_t i = sIdx * 32 + l;
-      if (genRow[i] >= 0 && genLen[i] > 0) { fallback = ext[rp[genRow[i]]]; have = true; }
-    }
-    for (int64_t q = slicePtr[sIdx]; q < slicePtr[sIdx + 1]; ++q) ellCol[q] = fallback;
-  }
-  for (int64_t i = 0; i < A->nGen; ++i) {
-    const int64_t r = genRow[i];
-    if (r < 0) continue;
-    const int64_t base = slicePtr[i >> 5] + (i & 31);
-    for (int64_t k = 0; k < genLen[i]; ++k) {
-      ellCol[base + k * 32] = ext[rp[r] + k];
-      ellVal[base + k * 32] = val[rp[r] + k];
-    }
-  }
-  // slice-padding entries keep row id -1; the kernel skips them
-  if ((rc = uploadVec(rowPat, &A->dRowPat, &A->deviceBytes, ctx))) return rc;
-  if ((rc = uploadVec(patOff, &A->dPatOff, &A->deviceBytes, ctx))) return rc;
-  PatEntry<T>* dPat = nullptr;
-  if ((rc = uploadVec(pat, &dPat, &A->deviceBytes, ctx))) return rc;
-  A->dPat = dPat;
-  if ((rc = uploadVec(genRow, &A->dGenRow, &A->deviceBytes, ctx))) return rc;
-  if ((rc = uploadVec(genLen, &A->dGenLen, &A->deviceBytes, ctx))) return rc;
-  if ((rc = uploadVec(slicePtr, &A->dSlicePtr, &A->deviceBytes, ctx))) return rc;
-  if ((rc = uploadVec(ellCol, &A->dCol, &A->deviceBytes, ctx))) return rc;
-  T* dVal = nullptr;
-  if ((rc = uploadVec(ellVal, &dVal, &A->deviceBytes, ctx))) return rc;
-  A->dVal = dVal;
-  // inverse diagonal for the smoothers (square operators on a single map only)
-  if (nRows == nLoc && A->rowMap->gids == A->domMap->gids) {
-    std::vector<T> inv(nRows, zeroOf<T>());
-    for (int64_t r = 0; r < nRows; ++r)
-      for (int64_t k = rp[r]; k < rp[r + 1]; ++k)
-        if (ext[k] == r) {
-          const T d = val[k];
-          if (!isZero(d)) {
-            if constexpr (sizeof(T) == sizeof(double)) {
-              double dd; std::memcpy(&dd, &d, sizeof(double));
-              dd = 1.0 / dd;
-              std::memcpy(&inv[r], &dd, sizeof(double));
-            } else {
-              double re, im; std::memcpy(&re, &d, sizeof(double)); std::memcpy(&im, reinterpret_cast<const char*>(&d) + 8, 8);
-              const double m2 = re * re + im * im;
-              const double o[2] = {re / m2, -im / m2};
-              std::memcpy(&inv[r], o, 16);
-            }
-          }
-        }
-    T* dInv = nullptr;
-    size_t unused = 0;
-    if ((rc = uploadVec(inv, &dInv, &unused, ctx))) return rc;
-    A->dInvDiag = dInv;
-  }
-  return MXG_OK;
-}
-
-
-// ---- layout built on the device ---------------------------------------------------------------------------------------
-// The same layout as buildImpl, for an operator whose CRS rows already sit in device memory (the operator assembly,
-// mxg_asm.cu): ghost discovery, extended column indices, the pattern dictionary (a device hash table instead of the host
-// unordered_map), sliced ELL and the inverse diagonal are kernels; the host keeps what is small or collective -- pattern
-// ordering (a few thousand candidates), the halo plan and the tile planner on a downloaded row -> pattern map.
+// ---- layout construction ----------------------------------------------------------------------------------------------
+// Two front ends bring a rank's rows into extended local columns: buildImpl from host CSR with global column ids
+// (mxg_crs_create), buildFromDeviceImpl from CRS rows that already sit in device memory (the operator assembly, mxg_asm.cu).
+// One back end, layoutFromDeviceRows, lays those rows out: the pattern dictionary (a device hash table), sliced ELL and the
+// inverse diagonal are kernels; the host keeps what is small or collective -- pattern ordering (a few thousand
+// candidates), the halo plan and the tile planner on a downloaded row -> pattern map.
 struct Scratch {
   std::vector<void*> p;
   ~Scratch() { for (void* q : p) if (q) cudaFree(q); }
@@ -1668,7 +1404,8 @@ __global__ void k_lb_fill_ell(const int32_t* __restrict__ genRow, const int32_t*
 }
 __device__ __forceinline__ double lbInverse(double d) { return 1.0 / d; }
 __device__ __forceinline__ zd lbInverse(zd d) {
-  const double m2 = __dadd_rn(__dmul_rn(d.x, d.x), __dmul_rn(d.y, d.y));    // two roundings, like the host builder
+  // two roundings, no FMA contraction: this pins the bits of the inverse diagonal, and so of every multigrid result
+  const double m2 = __dadd_rn(__dmul_rn(d.x, d.x), __dmul_rn(d.y, d.y));
   return {d.x / m2, -d.y / m2};
 }
 template <class T>
@@ -1679,7 +1416,7 @@ __global__ void k_lb_inv_diag(const int64_t* __restrict__ rp, const int32_t* __r
     for (int64_t q = rp[r]; q < rp[r + 1]; ++q)
       if (ext[q - base] == r) {
         const T d = valG[q];
-        out = isZero(d) ? zeroOf<T>() : lbInverse(d);      // the last matching entry wins, as in buildImpl (rows are merged: one)
+        out = isZero(d) ? zeroOf<T>() : lbInverse(d);      // rows are merged: at most one matching entry
       }
     inv[r] = out;
   }
@@ -1689,9 +1426,10 @@ inline unsigned lbGrid(int64_t n, int block = 256) {
   const int64_t b = (n + block - 1) / block;
   return unsigned(std::max<int64_t>(1, std::min<int64_t>(b, int64_t(1) << 20)));
 }
+// scratch buffer from the enclosing `tmp`; a failure names the entry point `fn`
 #define MXG_LB_ALLOC(var, type, count)                                                          \
   type* var = tmp.get<type>(count);                                                             \
-  MXG_REQUIRE(var != nullptr, "mxg_crs_create_from_dcsr: out of device memory (%s)", #var)
+  MXG_REQUIRE(var != nullptr, "%s: out of device memory (%s)", fn, #var)
 #define MXG_LB_KEEP(dst, type, count)                                                           \
   do {                                                                                          \
     void* q_ = nullptr;                                                                         \
@@ -1700,12 +1438,283 @@ inline unsigned lbGrid(int64_t n, int block = 256) {
     A->deviceBytes += size_t((count) > 0 ? (count) : 1) * sizeof(type);                         \
   } while (0)
 
+// interior range = longest run of rows without ghost needs, and the number of rows that have them (no `needs`: none has)
+void setInterior(mxg_crs* A, const std::vector<uint8_t>& needs) {
+  const int64_t nRows = A->nRows;
+  int64_t bestB = 0, bestE = 0, runB = 0;
+  for (int64_t r = 0; r <= nRows; ++r)
+    if (r == nRows || (!needs.empty() && needs[size_t(r)])) {
+      if (r - runB > bestE - bestB) { bestB = runB; bestE = r; }
+      runB = r + 1;
+    }
+  A->intBegin = bestB;
+  A->intEnd = bestE;
+  for (uint8_t n : needs) A->ghostRows += n;
+}
+
+// Back end of both front ends: pattern dictionary, kernel plans, sliced ELL and inverse diagonal from a rank's rows in
+// device memory. Precondition: the maps, nRows / nLoc, gLo / gHi and the halo plan are set; intBegin / intEnd, ghostRows
+// and nnz are set; dExt[q - base] holds the extended local column of entry q (dRp and dVal index entries from base); rows
+// are merged, one entry per column. fn names the entry point in error messages.
+template <class T>
+int layoutFromDeviceRows(mxg_crs* A, const int64_t* dRp, const int32_t* dExt, const T* dVal, int64_t base, int layout, const char* fn) {
+  mxg_ctx* ctx = A->ctx;
+  cudaStream_t st = ctx->stream;
+  const int64_t nRows = A->nRows, nLoc = A->nLoc;
+  Scratch tmp;
+
+  // ---- pattern dictionary
+  std::vector<int32_t> rowPat(static_cast<size_t>(nRows), -1), patOff(1, 0);
+  std::vector<PatEntry<T>> pat;
+  MXG_LB_KEEP(A->dRowPat, int32_t, nRows);
+  // Rectangular operators on two different maps (div, grad, curl, the multigrid transfers) have no translation-invariant
+  // rows -- column minus row index drifts with the row -- so the dictionary pass would hash tens of millions of unique
+  // rows for nothing: they go straight to sliced ELL.
+  const bool sameMaps = A->rowMap == A->domMap || A->rowMap->gids == A->domMap->gids;
+  bool haveDict = false;
+  if (layout != 1 && sameMaps && nRows > 0) {
+    int64_t tableSize = 1024;
+    while (tableSize < 2 * nRows) tableSize <<= 1;
+    MXG_LB_ALLOC(dKeys, unsigned long long, tableSize);
+    MXG_LB_ALLOC(dRep, int32_t, tableSize);
+    MXG_LB_ALLOC(dCount, int32_t, tableSize);
+    MXG_LB_ALLOC(dRowSlot, int32_t, nRows);
+    MXG_CUDA(cudaMemsetAsync(dKeys, 0xFF, size_t(tableSize) * sizeof(unsigned long long), st));
+    MXG_CUDA(cudaMemsetAsync(dRep, 0x7F, size_t(tableSize) * sizeof(int32_t), st));
+    MXG_CUDA(cudaMemsetAsync(dCount, 0, size_t(tableSize) * sizeof(int32_t), st));
+    k_lb_hash_insert<T><<<lbGrid(nRows), 256, 0, st>>>(dRp, dExt, dVal, base, nRows, dKeys, dRep, dCount, dRowSlot, uint64_t(tableSize - 1));
+    k_lb_verify<T><<<lbGrid(nRows), 256, 0, st>>>(dRp, dExt, dVal, base, nRows, dRep, dCount, dRowSlot);
+    MXG_LB_ALLOC(dOcc, int32_t, tableSize);
+    MXG_LB_ALLOC(dSlotOff, int64_t, tableSize + 1);
+    k_lb_occupied<<<lbGrid(tableSize), 256, 0, st>>>(dKeys, tableSize, dOcc);
+    int64_t nCand = 0;
+    MXG_CUDA(exclusiveScan(ctx, dOcc, dSlotOff, tableSize, &nCand));
+    ctx->launches += 3;
+    MXG_LB_ALLOC(dCandRep, int32_t, nCand);
+    MXG_LB_ALLOC(dCandCount, int32_t, nCand);
+    MXG_LB_ALLOC(dCandLen, int32_t, nCand);
+    MXG_LB_ALLOC(dCandPat, int32_t, nCand);
+    k_lb_cands<<<lbGrid(tableSize), 256, 0, st>>>(dOcc, dSlotOff, tableSize, dRep, dCount, dRp, dCandRep, dCandCount, dCandLen);
+    std::vector<int32_t> candRep(static_cast<size_t>(nCand), 0), candCount(static_cast<size_t>(nCand), 0), candLen(static_cast<size_t>(nCand), 0);
+    MXG_CUDA(cudaMemcpyAsync(candRep.data(), dCandRep, size_t(nCand) * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    MXG_CUDA(cudaMemcpyAsync(candCount.data(), dCandCount, size_t(nCand) * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    MXG_CUDA(cudaMemcpyAsync(candLen.data(), dCandLen, size_t(nCand) * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    MXG_CUDA(cudaStreamSynchronize(st));
+    // pattern numbering: candidates in order of first appearance, most frequent first (stable; the leading ones ride in
+    // the kernel parameter block), at least 4 rows
+    std::vector<int32_t> byRow(static_cast<size_t>(nCand), 0);
+    for (int64_t c = 0; c < nCand; ++c) byRow[size_t(c)] = int32_t(c);
+    std::sort(byRow.begin(), byRow.end(), [&](int32_t a, int32_t b) { return candRep[size_t(a)] < candRep[size_t(b)]; });
+    std::stable_sort(byRow.begin(), byRow.end(), [&](int32_t a, int32_t b) { return candCount[size_t(a)] > candCount[size_t(b)]; });
+    const int minCount = 4;
+    std::vector<int32_t> candPat(static_cast<size_t>(nCand), -1), patRep;
+    for (int32_t c : byRow) {
+      if (candCount[size_t(c)] < minCount) continue;
+      candPat[size_t(c)] = int32_t(patRep.size());
+      patRep.push_back(candRep[size_t(c)]);
+      patOff.push_back(patOff.back() + candLen[size_t(c)]);
+      A->dictRows += candCount[size_t(c)];
+    }
+    A->numPats = int64_t(patRep.size());
+    A->patEntries = patOff.back();
+    MXG_CUDA(cudaMemcpyAsync(dCandPat, candPat.data(), size_t(nCand) * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    k_lb_row_pat<<<lbGrid(nRows), 256, 0, st>>>(dRowSlot, dSlotOff, dCandPat, nRows, A->dRowPat);
+    MXG_LB_ALLOC(dPatRep, int32_t, A->numPats);
+    MXG_LB_KEEP(A->dPatOff, int32_t, A->numPats + 1);
+    PatEntry<T>* dPat = nullptr;
+    MXG_LB_KEEP(dPat, PatEntry<T>, A->patEntries);
+    A->dPat = dPat;
+    MXG_CUDA(cudaMemcpyAsync(dPatRep, patRep.data(), patRep.size() * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    MXG_CUDA(cudaMemcpyAsync(A->dPatOff, patOff.data(), patOff.size() * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    if (A->numPats > 0) k_lb_fill_pat<T><<<lbGrid(A->numPats, 64), 64, 0, st>>>(A->numPats, dPatRep, A->dPatOff, dRp, dExt, dVal, base, dPat);
+    ctx->launches += 3;
+    pat.resize(static_cast<size_t>(A->patEntries));
+    MXG_CUDA(cudaMemcpyAsync(rowPat.data(), A->dRowPat, size_t(nRows) * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    if (A->patEntries > 0) MXG_CUDA(cudaMemcpyAsync(pat.data(), dPat, size_t(A->patEntries) * sizeof(PatEntry<T>), cudaMemcpyDeviceToHost, st));
+    MXG_CUDA(cudaStreamSynchronize(st));      // candPat / patRep / patOff are host temporaries: done with them here
+    haveDict = true;
+  }
+  if (!haveDict) {
+    MXG_CUDA(cudaMemsetAsync(A->dRowPat, 0xFF, size_t(std::max<int64_t>(nRows, 1)) * sizeof(int32_t), st));
+    MXG_LB_KEEP(A->dPatOff, int32_t, 1);
+    MXG_CUDA(cudaMemsetAsync(A->dPatOff, 0, sizeof(int32_t), st));
+    PatEntry<T>* dPat = nullptr;
+    MXG_LB_KEEP(dPat, PatEntry<T>, 1);
+    A->dPat = dPat;
+  }
+  // (A constant-bank copy of the most frequent patterns was tried and removed: 0.351 ms vs 0.305 ms per apply on
+  // pillbox-256 -- a warp holds ~3 different patterns and divergent LDC replays cost more than L1 broadcast loads;
+  // the 16 KB parameter block also lengthened every launch. profiles/README_r01.md.)
+  int rc = planKernels<T>(A, rowPat, patOff, pat);
+  if (rc) return rc;
+
+  // ---- general rows in sliced ELL; the three row classes (leading boundary, interior, trailing boundary) each start on
+  // a slice boundary so they can be launched separately
+  MXG_LB_ALLOC(dIsGen, int32_t, nRows);
+  MXG_LB_ALLOC(dGenOff, int64_t, nRows + 1);
+  if (nRows > 0) k_lb_is_gen<<<lbGrid(nRows), 256, 0, st>>>(A->dRowPat, nRows, dIsGen);
+  int64_t totalGen = 0;
+  MXG_CUDA(exclusiveScan(ctx, dIsGen, dGenOff, nRows, &totalGen));
+  int64_t offs[2] = {0, totalGen};
+  MXG_CUDA(cudaMemcpyAsync(&offs[0], dGenOff + A->intBegin, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+  MXG_CUDA(cudaMemcpyAsync(&offs[1], dGenOff + A->intEnd, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+  MXG_CUDA(cudaStreamSynchronize(st));
+  auto pad32 = [](int64_t v) { return (v + 31) / 32 * 32; };
+  const int64_t n0 = offs[0], n1 = offs[1] - offs[0], n2 = totalGen - offs[1];
+  A->genIntBegin = pad32(n0);
+  A->genIntEnd = A->genIntBegin + pad32(n1);
+  A->nGen = A->genIntEnd + pad32(n2);
+  MXG_LB_KEEP(A->dGenRow, int32_t, A->nGen);
+  MXG_LB_KEEP(A->dGenLen, int32_t, A->nGen);
+  MXG_CUDA(cudaMemsetAsync(A->dGenRow, 0xFF, size_t(std::max<int64_t>(A->nGen, 1)) * sizeof(int32_t), st));
+  MXG_CUDA(cudaMemsetAsync(A->dGenLen, 0, size_t(std::max<int64_t>(A->nGen, 1)) * sizeof(int32_t), st));
+  if (nRows > 0)
+    k_lb_gen_rows<<<lbGrid(nRows), 256, 0, st>>>(dIsGen, dGenOff, dRp, nRows, A->intBegin, A->intEnd, offs[0], offs[1], A->genIntBegin,
+                                                 A->genIntEnd, A->dGenRow, A->dGenLen);
+  const int64_t nSlices = A->nGen / 32;
+  MXG_LB_ALLOC(dSliceW, int32_t, nSlices);
+  MXG_LB_KEEP(A->dSlicePtr, int64_t, nSlices + 1);
+  if (nSlices > 0) k_lb_slice_width<<<lbGrid(nSlices), 256, 0, st>>>(A->dGenLen, nSlices, dSliceW);
+  int64_t totalW = 0;
+  MXG_CUDA(exclusiveScan(ctx, dSliceW, A->dSlicePtr, nSlices, &totalW));
+  k_lb_times32<<<lbGrid(nSlices + 1), 256, 0, st>>>(A->dSlicePtr, nSlices + 1);
+  A->ellEntries = totalW * 32;
+  MXG_LB_KEEP(A->dCol, int32_t, A->ellEntries);
+  T* dEllVal = nullptr;
+  MXG_LB_KEEP(dEllVal, T, A->ellEntries);
+  A->dVal = dEllVal;
+  if (nSlices > 0) k_lb_fill_ell<T><<<lbGrid(nSlices * 32), 256, 0, st>>>(A->dGenRow, A->dGenLen, A->dSlicePtr, dRp, dExt, dVal, base, nSlices, A->dCol, dEllVal);
+  ctx->launches += 5;
+
+  // ---- inverse diagonal for the smoothers (square operators on a single map only)
+  if (nRows == nLoc && A->rowMap->gids == A->domMap->gids) {
+    T* dInv = nullptr;
+    void* q = nullptr;
+    MXG_CUDA(cudaMalloc(&q, size_t(std::max<int64_t>(nRows, 1)) * sizeof(T)));
+    dInv = static_cast<T*>(q);
+    A->dInvDiag = dInv;
+    if (nRows > 0) k_lb_inv_diag<T><<<lbGrid(nRows), 256, 0, st>>>(dRp, dExt, dVal, base, nRows, dInv);
+    ctx->launches++;
+  }
+  MXG_CUDA(cudaGetLastError());
+  MXG_CUDA(cudaStreamSynchronize(st));
+  return MXG_OK;
+}
+
+// Host front end (mxg_crs_create): host CSR rows with global column ids.
+template <class T>
+int buildImpl(mxg_crs* A, const int64_t* rowptr, const int64_t* colGids, const double* valsIn, int layout) {
+  const char* fn = "mxg_crs_create";
+  mxg_ctx* ctx = A->ctx;
+  const T* vals = reinterpret_cast<const T*>(valsIn);
+  const int64_t nRows = A->nRows, nLoc = A->nLoc;
+  const int64_t nnzIn = rowptr[nRows];
+  const mxg_map* dom = A->domMap;
+  MXG_REQUIRE(dom->nGlobal < (int64_t(1) << 31), "mxg_crs_create: global size must fit in 31 bits");
+
+  // GID -> local id of the domain map
+  std::vector<int32_t> lookup(size_t(dom->nGlobal), -1);
+  for (int64_t i = 0; i < nLoc; ++i) lookup[dom->gids[i]] = int32_t(i);
+  const int64_t domLo = nLoc ? dom->gids.front() : 0, domHi = nLoc ? dom->gids.back() : -1;
+
+  // ghosts = referenced GIDs that are not local
+  std::vector<int64_t> ghosts;
+  for (int64_t q = 0; q < nnzIn; ++q) {
+    const int64_t g = colGids[q];
+    MXG_REQUIRE(g >= 0 && g < dom->nGlobal, "mxg_crs_create: column GID %lld out of range", (long long)g);
+    if (lookup[g] < 0) ghosts.push_back(g);
+  }
+  std::sort(ghosts.begin(), ghosts.end());
+  ghosts.erase(std::unique(ghosts.begin(), ghosts.end()), ghosts.end());
+  MXG_REQUIRE(ghosts.empty() || ctx->nranks > 1, "mxg_crs_create: column GID %lld is not in the domain map",
+              (long long)(ghosts.empty() ? 0 : ghosts[0]));
+  A->gLo = int64_t(std::lower_bound(ghosts.begin(), ghosts.end(), domLo) - ghosts.begin());
+  if (nLoc == 0) A->gLo = 0;
+  A->gHi = int64_t(ghosts.size()) - A->gLo;
+  int rc = planHalo(A, ghosts, lookup, domLo, domHi);
+  if (rc) return rc;
+
+  // extended local column index of every entry; rows sorted, duplicates merged
+  std::vector<int64_t> rp(nRows + 1, 0);
+  std::vector<int32_t> ext;
+  std::vector<T> val;
+  ext.reserve(nnzIn);
+  val.reserve(nnzIn);
+  std::vector<uint8_t> needsGhost(nRows, 0);
+  std::vector<std::pair<int32_t, T>> rowBuf;
+  for (int64_t r = 0; r < nRows; ++r) {
+    rowBuf.clear();
+    bool sorted = true;
+    for (int64_t q = rowptr[r]; q < rowptr[r + 1]; ++q) {
+      const int64_t g = colGids[q];
+      int32_t e = lookup[g];
+      if (e < 0) {
+        const int64_t pos = std::lower_bound(ghosts.begin(), ghosts.end(), g) - ghosts.begin();
+        e = pos < A->gLo ? int32_t(pos - A->gLo) : int32_t(nLoc + (pos - A->gLo));
+        needsGhost[r] = 1;
+      }
+      if (!rowBuf.empty() && e <= rowBuf.back().first) sorted = false;
+      rowBuf.emplace_back(e, vals[q]);
+    }
+    if (!sorted) {
+      std::stable_sort(rowBuf.begin(), rowBuf.end(), [](auto& a, auto& b) { return a.first < b.first; });
+      size_t o = 0;
+      for (size_t i = 0; i < rowBuf.size();) {
+        T s = rowBuf[i].second;
+        size_t j = i + 1;
+        while (j < rowBuf.size() && rowBuf[j].first == rowBuf[i].first) s = s + rowBuf[j++].second;
+        rowBuf[o++] = {rowBuf[i].first, s};
+        i = j;
+      }
+      rowBuf.resize(o);
+    }
+    for (auto& t : rowBuf) { ext.push_back(t.first); val.push_back(t.second); }
+    rp[r + 1] = int64_t(ext.size());
+  }
+  A->nnz = int64_t(ext.size());
+  // Ordered maps (mxg_map_create_ordered): rows move to their device positions and owned columns are translated; the
+  // entry order inside a row stays the reference's ascending local column, so sums keep Epetra's order bit for bit.
+  if (!A->rowMap->perm.empty() || !A->domMap->perm.empty()) {
+    MXG_REQUIRE(ctx->nranks == 1 && ghosts.empty(), "mxg_crs_create: ordered maps are supported on single-rank contexts only");
+    std::vector<int32_t> rowPerm = A->rowMap->perm, colInv = A->domMap->inv;
+    if (rowPerm.empty()) { rowPerm.resize(size_t(nRows)); for (int64_t i = 0; i < nRows; ++i) rowPerm[size_t(i)] = int32_t(i); }
+    if (colInv.empty()) { colInv.resize(size_t(nLoc)); for (int64_t i = 0; i < nLoc; ++i) colInv[size_t(i)] = int32_t(i); }
+    std::vector<int64_t> rp2;
+    std::vector<int32_t> ext2;
+    std::vector<T> val2;
+    try {
+      mxg::permuteCsr(rp, ext, val, rowPerm, colInv, nLoc, rp2, ext2, val2);
+    } catch (const std::exception& e) {   // nothing may unwind through the C boundary
+      MXG_REQUIRE(false, "mxg_crs_create: %s", e.what());
+    }
+    rp.swap(rp2);
+    ext.swap(ext2);
+    val.swap(val2);
+  }
+  setInterior(A, needsGhost);
+
+  // the merged rows go to the device for the common back end
+  Scratch tmp;
+  MXG_LB_ALLOC(dRp, int64_t, nRows + 1);
+  MXG_LB_ALLOC(dExt, int32_t, A->nnz);
+  MXG_LB_ALLOC(dVal, T, A->nnz);
+  cudaStream_t st = ctx->stream;
+  MXG_CUDA(cudaMemcpyAsync(dRp, rp.data(), rp.size() * sizeof(int64_t), cudaMemcpyHostToDevice, st));
+  if (A->nnz > 0) {
+    MXG_CUDA(cudaMemcpyAsync(dExt, ext.data(), ext.size() * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    MXG_CUDA(cudaMemcpyAsync(dVal, val.data(), val.size() * sizeof(T), cudaMemcpyHostToDevice, st));
+  }
+  return layoutFromDeviceRows<T>(A, dRp, dExt, dVal, 0, layout, fn);
+}
+
+// Device front end (mxg_crs_create_from_dcsr): rows [base, base + nnz) of a device CRS whose columns are positions in
+// the column field's map, of which this rank owns [c0, c0 + nLoc).
 template <class T>
 int buildFromDeviceImpl(mxg_crs* A, const int64_t* dRp, const int32_t* dColG, const void* dValRaw, int64_t c0, int64_t colFieldSize,
                         const int64_t* colFieldGids, int layout) {
+  const char* fn = "mxg_crs_create_from_dcsr";
   mxg_ctx* ctx = A->ctx;
   cudaStream_t st = ctx->stream;
-  const T* dValG = static_cast<const T*>(dValRaw);
   const int64_t nRows = A->nRows, nLoc = A->nLoc, c1 = c0 + nLoc;
   const mxg_map* dom = A->domMap;
   MXG_REQUIRE(dom->nGlobal < (int64_t(1) << 31), "mxg_crs_create: global size must fit in 31 bits");
@@ -1770,147 +1779,30 @@ int buildFromDeviceImpl(mxg_crs* A, const int64_t* dRp, const int32_t* dColG, co
   }
   MXG_CUDA(cudaStreamSynchronize(st));
   MXG_REQUIRE(hErr == 0, "mxg_crs_create: a column is not in the domain map (single-rank context)");
-  A->intBegin = 0;
-  A->intEnd = nRows;
-  if (dNeeds) {       // interior range = longest run of rows without ghost needs
-    int64_t bestB = 0, bestE = 0, runB = 0;
-    for (int64_t r = 0; r <= nRows; ++r)
-      if (r == nRows || needs[size_t(r)]) {
-        if (r - runB > bestE - bestB) { bestB = runB; bestE = r; }
-        runB = r + 1;
-      }
-    A->intBegin = bestB;
-    A->intEnd = bestE;
-    for (int64_t r = 0; r < nRows; ++r) A->ghostRows += needs[size_t(r)];
-  }
+  setInterior(A, needs);
+  return layoutFromDeviceRows<T>(A, dRp, dExt, static_cast<const T*>(dValRaw), base, layout, fn);
+}
 
-  // ---- pattern dictionary
-  std::vector<int32_t> rowPat(static_cast<size_t>(nRows), -1), patOff(1, 0);
-  std::vector<PatEntry<T>> pat;
-  MXG_LB_KEEP(A->dRowPat, int32_t, nRows);
-  const bool sameMaps = A->rowMap == A->domMap || A->rowMap->gids == A->domMap->gids;
-  bool haveDict = false;
-  if (layout != 1 && sameMaps && nRows > 0) {
-    int64_t tableSize = 1024;
-    while (tableSize < 2 * nRows) tableSize <<= 1;
-    MXG_LB_ALLOC(dKeys, unsigned long long, tableSize);
-    MXG_LB_ALLOC(dRep, int32_t, tableSize);
-    MXG_LB_ALLOC(dCount, int32_t, tableSize);
-    MXG_LB_ALLOC(dRowSlot, int32_t, nRows);
-    MXG_CUDA(cudaMemsetAsync(dKeys, 0xFF, size_t(tableSize) * sizeof(unsigned long long), st));
-    MXG_CUDA(cudaMemsetAsync(dRep, 0x7F, size_t(tableSize) * sizeof(int32_t), st));
-    MXG_CUDA(cudaMemsetAsync(dCount, 0, size_t(tableSize) * sizeof(int32_t), st));
-    k_lb_hash_insert<T><<<lbGrid(nRows), 256, 0, st>>>(dRp, dExt, dValG, base, nRows, dKeys, dRep, dCount, dRowSlot, uint64_t(tableSize - 1));
-    k_lb_verify<T><<<lbGrid(nRows), 256, 0, st>>>(dRp, dExt, dValG, base, nRows, dRep, dCount, dRowSlot);
-    MXG_LB_ALLOC(dOcc, int32_t, tableSize);
-    MXG_LB_ALLOC(dSlotOff, int64_t, tableSize + 1);
-    k_lb_occupied<<<lbGrid(tableSize), 256, 0, st>>>(dKeys, tableSize, dOcc);
-    int64_t nCand = 0;
-    MXG_CUDA(exclusiveScan(ctx, dOcc, dSlotOff, tableSize, &nCand));
-    ctx->launches += 3;
-    MXG_LB_ALLOC(dCandRep, int32_t, nCand);
-    MXG_LB_ALLOC(dCandCount, int32_t, nCand);
-    MXG_LB_ALLOC(dCandLen, int32_t, nCand);
-    MXG_LB_ALLOC(dCandPat, int32_t, nCand);
-    k_lb_cands<<<lbGrid(tableSize), 256, 0, st>>>(dOcc, dSlotOff, tableSize, dRep, dCount, dRp, dCandRep, dCandCount, dCandLen);
-    std::vector<int32_t> candRep(static_cast<size_t>(nCand), 0), candCount(static_cast<size_t>(nCand), 0), candLen(static_cast<size_t>(nCand), 0);
-    MXG_CUDA(cudaMemcpyAsync(candRep.data(), dCandRep, size_t(nCand) * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-    MXG_CUDA(cudaMemcpyAsync(candCount.data(), dCandCount, size_t(nCand) * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-    MXG_CUDA(cudaMemcpyAsync(candLen.data(), dCandLen, size_t(nCand) * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-    MXG_CUDA(cudaStreamSynchronize(st));
-    // pattern numbering as in buildImpl: candidates in order of first appearance, most frequent first (stable), at least 4 rows
-    std::vector<int32_t> byRow(static_cast<size_t>(nCand), 0);
-    for (int64_t c = 0; c < nCand; ++c) byRow[size_t(c)] = int32_t(c);
-    std::sort(byRow.begin(), byRow.end(), [&](int32_t a, int32_t b) { return candRep[size_t(a)] < candRep[size_t(b)]; });
-    std::stable_sort(byRow.begin(), byRow.end(), [&](int32_t a, int32_t b) { return candCount[size_t(a)] > candCount[size_t(b)]; });
-    const int minCount = 4;
-    std::vector<int32_t> candPat(static_cast<size_t>(nCand), -1), patRep;
-    for (int32_t c : byRow) {
-      if (candCount[size_t(c)] < minCount) continue;
-      candPat[size_t(c)] = int32_t(patRep.size());
-      patRep.push_back(candRep[size_t(c)]);
-      patOff.push_back(patOff.back() + candLen[size_t(c)]);
-      A->dictRows += candCount[size_t(c)];
-    }
-    A->numPats = int64_t(patRep.size());
-    A->patEntries = patOff.back();
-    MXG_CUDA(cudaMemcpyAsync(dCandPat, candPat.data(), size_t(nCand) * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-    k_lb_row_pat<<<lbGrid(nRows), 256, 0, st>>>(dRowSlot, dSlotOff, dCandPat, nRows, A->dRowPat);
-    MXG_LB_ALLOC(dPatRep, int32_t, A->numPats);
-    MXG_LB_KEEP(A->dPatOff, int32_t, A->numPats + 1);
-    PatEntry<T>* dPat = nullptr;
-    MXG_LB_KEEP(dPat, PatEntry<T>, A->patEntries);
-    A->dPat = dPat;
-    MXG_CUDA(cudaMemcpyAsync(dPatRep, patRep.data(), patRep.size() * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-    MXG_CUDA(cudaMemcpyAsync(A->dPatOff, patOff.data(), patOff.size() * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-    if (A->numPats > 0) k_lb_fill_pat<T><<<lbGrid(A->numPats, 64), 64, 0, st>>>(A->numPats, dPatRep, A->dPatOff, dRp, dExt, dValG, base, dPat);
-    ctx->launches += 3;
-    pat.resize(static_cast<size_t>(A->patEntries));
-    MXG_CUDA(cudaMemcpyAsync(rowPat.data(), A->dRowPat, size_t(nRows) * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-    if (A->patEntries > 0) MXG_CUDA(cudaMemcpyAsync(pat.data(), dPat, size_t(A->patEntries) * sizeof(PatEntry<T>), cudaMemcpyDeviceToHost, st));
-    MXG_CUDA(cudaStreamSynchronize(st));      // candPat / patRep / patOff are host temporaries: done with them here
-    haveDict = true;
+// A new operator on (rowMap, domMap), laid out by `build`; released again when that fails.
+template <class Build>
+int crsCreate(mxg_map* rowMap, mxg_map* domMap, int isComplex, mxg_crs** out, Build build) {
+  mxg_ctx* ctx = rowMap->ctx;
+  MXG_CUDA(cudaSetDevice(ctx->device));
+  mxg_crs* A = new mxg_crs;
+  A->ctx = ctx;
+  A->rowMap = rowMap;
+  A->domMap = domMap;
+  rowMap->refs++;
+  domMap->refs++;
+  A->isComplex = isComplex != 0;
+  A->nRows = rowMap->nLocal;
+  A->nLoc = domMap->nLocal;
+  const int rc = build(A);
+  if (rc) {
+    mxg_crs_destroy(A);
+    return rc;
   }
-  if (!haveDict) {
-    MXG_CUDA(cudaMemsetAsync(A->dRowPat, 0xFF, size_t(std::max<int64_t>(nRows, 1)) * sizeof(int32_t), st));
-    MXG_LB_KEEP(A->dPatOff, int32_t, 1);
-    MXG_CUDA(cudaMemsetAsync(A->dPatOff, 0, sizeof(int32_t), st));
-    PatEntry<T>* dPat = nullptr;
-    MXG_LB_KEEP(dPat, PatEntry<T>, 1);
-    A->dPat = dPat;
-  }
-  int rc = planKernels<T>(A, rowPat, patOff, pat);
-  if (rc) return rc;
-
-  // ---- general rows in sliced ELL
-  MXG_LB_ALLOC(dIsGen, int32_t, nRows);
-  MXG_LB_ALLOC(dGenOff, int64_t, nRows + 1);
-  if (nRows > 0) k_lb_is_gen<<<lbGrid(nRows), 256, 0, st>>>(A->dRowPat, nRows, dIsGen);
-  int64_t totalGen = 0;
-  MXG_CUDA(exclusiveScan(ctx, dIsGen, dGenOff, nRows, &totalGen));
-  int64_t offs[2] = {0, totalGen};
-  MXG_CUDA(cudaMemcpyAsync(&offs[0], dGenOff + A->intBegin, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
-  MXG_CUDA(cudaMemcpyAsync(&offs[1], dGenOff + A->intEnd, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
-  MXG_CUDA(cudaStreamSynchronize(st));
-  auto pad32 = [](int64_t v) { return (v + 31) / 32 * 32; };
-  const int64_t n0 = offs[0], n1 = offs[1] - offs[0], n2 = totalGen - offs[1];
-  A->genIntBegin = pad32(n0);
-  A->genIntEnd = A->genIntBegin + pad32(n1);
-  A->nGen = A->genIntEnd + pad32(n2);
-  MXG_LB_KEEP(A->dGenRow, int32_t, A->nGen);
-  MXG_LB_KEEP(A->dGenLen, int32_t, A->nGen);
-  MXG_CUDA(cudaMemsetAsync(A->dGenRow, 0xFF, size_t(std::max<int64_t>(A->nGen, 1)) * sizeof(int32_t), st));
-  MXG_CUDA(cudaMemsetAsync(A->dGenLen, 0, size_t(std::max<int64_t>(A->nGen, 1)) * sizeof(int32_t), st));
-  if (nRows > 0)
-    k_lb_gen_rows<<<lbGrid(nRows), 256, 0, st>>>(dIsGen, dGenOff, dRp, nRows, A->intBegin, A->intEnd, offs[0], offs[1], A->genIntBegin,
-                                                 A->genIntEnd, A->dGenRow, A->dGenLen);
-  const int64_t nSlices = A->nGen / 32;
-  MXG_LB_ALLOC(dSliceW, int32_t, nSlices);
-  MXG_LB_KEEP(A->dSlicePtr, int64_t, nSlices + 1);
-  if (nSlices > 0) k_lb_slice_width<<<lbGrid(nSlices), 256, 0, st>>>(A->dGenLen, nSlices, dSliceW);
-  int64_t totalW = 0;
-  MXG_CUDA(exclusiveScan(ctx, dSliceW, A->dSlicePtr, nSlices, &totalW));
-  k_lb_times32<<<lbGrid(nSlices + 1), 256, 0, st>>>(A->dSlicePtr, nSlices + 1);
-  A->ellEntries = totalW * 32;
-  MXG_LB_KEEP(A->dCol, int32_t, A->ellEntries);
-  T* dEllVal = nullptr;
-  MXG_LB_KEEP(dEllVal, T, A->ellEntries);
-  A->dVal = dEllVal;
-  if (nSlices > 0) k_lb_fill_ell<T><<<lbGrid(nSlices * 32), 256, 0, st>>>(A->dGenRow, A->dGenLen, A->dSlicePtr, dRp, dExt, dValG, base, nSlices, A->dCol, dEllVal);
-  ctx->launches += 5;
-
-  // ---- inverse diagonal for the smoothers (square operators on a single map only)
-  if (nRows == nLoc && A->rowMap->gids == A->domMap->gids) {
-    T* dInv = nullptr;
-    void* q = nullptr;
-    MXG_CUDA(cudaMalloc(&q, size_t(std::max<int64_t>(nRows, 1)) * sizeof(T)));
-    dInv = static_cast<T*>(q);
-    A->dInvDiag = dInv;
-    if (nRows > 0) k_lb_inv_diag<T><<<lbGrid(nRows), 256, 0, st>>>(dRp, dExt, dValG, base, nRows, dInv);
-    ctx->launches++;
-  }
-  MXG_CUDA(cudaGetLastError());
-  MXG_CUDA(cudaStreamSynchronize(st));
+  *out = A;
   return MXG_OK;
 }
 
@@ -1925,26 +1817,11 @@ int crsCreateFromDevice(mxg_map* rowMap, mxg_map* domMap, const int64_t* dRowptr
   MXG_REQUIRE(rowMap && domMap && dRowptr && out, "mxg_crs_create_from_dcsr: NULL argument");
   MXG_REQUIRE(rowMap->ctx == domMap->ctx, "mxg_crs_create_from_dcsr: maps live on different contexts");
   MXG_REQUIRE(layout >= 0 && layout <= 1, "mxg_crs_create_from_dcsr: unknown layout %d", layout);
-  MXG_REQUIRE(rowMap->perm.empty() && domMap->perm.empty(), "mxg_crs_create_from_dcsr: ordered maps are not supported by the device layout builder");
-  mxg_ctx* ctx = rowMap->ctx;
-  MXG_CUDA(cudaSetDevice(ctx->device));
-  mxg_crs* A = new mxg_crs;
-  A->ctx = ctx;
-  A->rowMap = rowMap;
-  A->domMap = domMap;
-  rowMap->refs++;
-  domMap->refs++;
-  A->isComplex = isComplex != 0;
-  A->nRows = rowMap->nLocal;
-  A->nLoc = domMap->nLocal;
-  const int rc = A->isComplex ? buildFromDeviceImpl<zd>(A, dRowptr, dCol, dVal, colBegin, colFieldSize, colFieldGids, layout)
-                              : buildFromDeviceImpl<double>(A, dRowptr, dCol, dVal, colBegin, colFieldSize, colFieldGids, layout);
-  if (rc) {
-    mxg_crs_destroy(A);
-    return rc;
-  }
-  *out = A;
-  return MXG_OK;
+  MXG_REQUIRE(rowMap->perm.empty() && domMap->perm.empty(), "mxg_crs_create_from_dcsr: ordered maps are not supported by the device front end");
+  return crsCreate(rowMap, domMap, isComplex, out, [&](mxg_crs* A) {
+    return A->isComplex ? buildFromDeviceImpl<zd>(A, dRowptr, dCol, dVal, colBegin, colFieldSize, colFieldGids, layout)
+                        : buildFromDeviceImpl<double>(A, dRowptr, dCol, dVal, colBegin, colFieldSize, colFieldGids, layout);
+  });
 }
 
 }  // namespace mxg
@@ -1959,24 +1836,9 @@ int mxg_crs_create_opts(mxg_map* row_map, mxg_map* domain_map, const int64_t* ro
   const int64_t nnz = rowptr[row_map->nLocal];
   MXG_REQUIRE(nnz == 0 || (col_gids && vals), "mxg_crs_create: NULL column / value array");
   MXG_REQUIRE(layout >= 0 && layout <= 1, "mxg_crs_create: unknown layout %d", layout);
-  mxg_ctx* ctx = row_map->ctx;
-  MXG_CUDA(cudaSetDevice(ctx->device));
-  mxg_crs* A = new mxg_crs;
-  A->ctx = ctx;
-  A->rowMap = row_map;
-  A->domMap = domain_map;
-  row_map->refs++;
-  domain_map->refs++;
-  A->isComplex = is_complex != 0;
-  A->nRows = row_map->nLocal;
-  A->nLoc = domain_map->nLocal;
-  int rc = A->isComplex ? buildImpl<zd>(A, rowptr, col_gids, vals, layout) : buildImpl<double>(A, rowptr, col_gids, vals, layout);
-  if (rc) {
-    mxg_crs_destroy(A);
-    return rc;
-  }
-  *out = A;
-  return MXG_OK;
+  return crsCreate(row_map, domain_map, is_complex, out, [&](mxg_crs* A) {
+    return A->isComplex ? buildImpl<zd>(A, rowptr, col_gids, vals, layout) : buildImpl<double>(A, rowptr, col_gids, vals, layout);
+  });
 }
 
 int mxg_crs_create(mxg_map* row_map, mxg_map* domain_map, const int64_t* rowptr, const int64_t* col_gids,

@@ -89,7 +89,7 @@ def solve_case(ctx, rank, world):
 def device_assembly_case(ctx, rank, world):
     """Operators assembled on every rank's device (include/mxasm.h), each rank keeping the rows of its slab; the layout is
     built on the device too (ghost discovery, halo plan, dictionary, sliced ELL). Applies must equal the oracle's global
-    apply bit for bit and the layout must be the one the host builder makes from the same rows."""
+    apply bit for bit, and the layout statistics must be those the same rows give when they come in as host CSR."""
     from maxwell_b200 import assembly as asm
     n = 24
     fine, coarse = asm.example_sim(ctx, "pillbox", n), asm.example_sim(ctx, "pillbox", n // 2)

@@ -1,7 +1,7 @@
 """Stand-alone body of tests/test_gpu_spmv.py::test_component_major_ordered_maps (own process: this path had not run on a
 GPU when it was written). Operators and vectors on component-major ordered maps (mxg_map_create_ordered) must give exactly
-the results of the reference order: bit-exact SpMM for square and rectangular operators, GID-keyed random vectors, field
-output, norms / Gram matrices up to summation order, and the same eigenvalues."""
+the results of the reference order: bit-exact SpMM for square and rectangular operators (also for an operator assembled on
+the device), GID-keyed random vectors, field output, norms / Gram matrices up to summation order, and the same eigenvalues."""
 import os
 import sys
 
@@ -34,6 +34,23 @@ def main():
             A.apply(x, y)
             xh = x.to_host()
             assert np.array_equal(op.apply(xh), y.to_host()), (name, nvec)
+    # a device-assembled operator on the ordered maps: mxg_crs_create_from_dcsr downloads its rows and lays them out as
+    # host CSR, so it must be the operator the oracle's rows make
+    from maxwell_b200 import assembly as asm
+    op = sim.op("curlCurl")
+    rowptr, col, val = op.arrays()
+    rg, cg = op.maps()
+    A = asm.to_crs(asm.example_sim(ctx, "pillbox", 20).op("curlCurl"), maps["bfield"], maps["bfield"])
+    H = mx.MxCrsMatrix.from_csr(maps["bfield"], maps["bfield"], rowptr, cg[col], val)
+    assert A.stats() == H.stats(), (A.stats(), H.stats())
+    x = mx.MxMultiVector(maps["bfield"], 3)
+    x.random(4242)
+    ys = []
+    for M in (A, H):
+        y = mx.MxMultiVector(maps["bfield"], 3)
+        M.apply(x, y)
+        ys.append(y.to_host())
+    assert np.array_equal(ys[0], ys[1]), "device-assembled operator on ordered maps"
     # random vectors are keyed by GID: identical to the reference-order map, column by column
     xo = mx.MxMultiVector(maps["bfield"], 2)
     xp = mx.MxMultiVector(plain["bfield"], 2)
