@@ -190,8 +190,13 @@ int mxg_crs_apply_host_batch(const mxg_crs* A, int count, const double* const* x
 /* y = alpha*A*x + beta*y fused into the SpMM epilogue (residuals r = b - A x of the
  * multigrid cycle, MxGeoMultigridPrec.cpp:312-314; shifted operators, MxMagWaveOp.cpp:247-256) */
 int mxg_crs_apply_axpby(const mxg_crs* A, const double alpha[2], const mxg_mv* x, const double beta[2], mxg_mv* y);
-/* one apply with CUDA events around each kernel class: ms[0] = dictionary-row kernel,
- * ms[1] = sliced-ELL kernel, ms[2] = halo pack + exchange wait, ms[3] = whole apply */
+/* one apply, on the path mxg_crs_apply takes, split into phases. ms[3] = whole apply (CUDA events) on every path.
+ * One rank (CUDA events): ms[0] = dictionary-row kernel, ms[1] = sliced-ELL kernel, ms[2] = time before the first kernel.
+ * Several ranks, single launch over peer memory (the %globaltimer roles of mxg_crs_trace): ms[0] = interior rows (roles 1
+ * and 2, first start to last end), ms[1] = boundary rows (role 4), ms[2] = pack + flag publish (role 0); a role that did
+ * not run counts 0.
+ * Several ranks, NCCL exchange (CUDA events): ms[0] = interior rows up to the end of the apply, ms[1] = boundary rows,
+ * ms[2] = NCCL send/recv. */
 int mxg_crs_apply_timed(const mxg_crs* A, const mxg_mv* x, mxg_mv* y, double ms[4]);
 /* %globaltimer timeline of ONE multi-rank apply (the single-launch path): call with enable = 1, apply once, call with
  * enable = 0 to read out[10] in ns relative to the earliest mark -- role r: out[2r] first start, out[2r+1] last end;

@@ -92,7 +92,7 @@ struct mxg_ctx {
   cudaEvent_t evA = nullptr, evB = nullptr;
   cudaEvent_t timer[16] = {};          // user timing slots (created lazily)
   cudaEvent_t prof[10] = {};           // per-kernel profiling events
-  bool profiling = false;
+  bool profiling = false;              // inside mxg_crs_apply_timed: record phase events, do not capture a graph
   ncclComm_t comm = nullptr;
   int rank = 0, nranks = 1;
   double* dScratch = nullptr;          // reduction partials / small device results
@@ -193,16 +193,14 @@ struct mxg_crs {
     int launches;
   };
   mutable std::vector<GraphEntry> graphs;
-  // Direct peer-memory halo exchange: boundary values are stored straight into the neighbour's ghost
-  // buffer over NVLink by the pack kernel, followed by an epoch flag; no NCCL call per apply.
+  // Direct peer-memory halo exchange: the whole apply is one launch (k_apply_fused) whose pack blocks store boundary values
+  // straight into the neighbour's ghost buffer over NVLink, followed by an epoch flag; no NCCL call per apply.
   struct P2P {
     bool on = false;
-    bool fused = true;                      // whole apply in one launch (k_apply_fused) instead of the multi-kernel graph
-    unsigned long long hostEpoch = 0;       // exchanges enqueued so far (= the device epoch once they have run)
+    unsigned long long hostEpoch = 0;       // exchanges enqueued so far
     int capCols = 0;
     void* ghost = nullptr;                  // [2][capCols][gTot] scalars, IPC-exported (double buffered by epoch parity)
     unsigned long long* flags = nullptr;    // [nranks] epochs written by the senders, IPC-exported
-    unsigned long long* epoch = nullptr;    // local apply counter
     unsigned int* done = nullptr;           // block-completion counter of the pack kernel
     void* dArgs = nullptr;                  // device copy of the peer tables (P2PArgs) for the single-launch kernel
     unsigned long long* trace = nullptr;    // %globaltimer marks of the fused apply (mxg_crs_trace), NULL = off

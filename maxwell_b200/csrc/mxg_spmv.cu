@@ -68,9 +68,6 @@ struct XSource {
   ColTable<T> x;       // local part of each column
   const T* ghost;      // [col][gLo + gHi]
   int64_t nLoc, gLo, gTot;
-  // peer-memory exchange: the ghost buffer is double buffered, the live half is (epoch & 1)
-  const unsigned long long* epoch;
-  int64_t halfStride;  // capCols * gTot
 };
 
 template <class T, bool GHOST>
@@ -369,46 +366,14 @@ __global__ void __launch_bounds__(kBlock) k_spmm_sell(int64_t genBegin, int64_t 
 }
 
 // Several row ranges (dictionary + sliced ELL, leading + trailing boundary) in ONE launch: for short
-// ranges the launch latency costs more than the rows. With W.n > 0 every block first waits until all
-// neighbour ranks have published the current halo epoch (peer-memory exchange); the wait depends only
-// on OTHER GPUs, never on blocks of this GPU, so it cannot dead-lock the device.
+// ranges the launch latency costs more than the rows.
 struct Segments {
   int64_t begin[4], end[4];   // 0,1: dictionary row ranges; 2,3: sliced-ELL (compacted) ranges
   int blockStart[5];          // first block of each segment
 };
-struct WaitArgs {
-  int n;
-  const unsigned long long* flags;
-  const unsigned long long* epoch;
-  int senderRank[8];
-  int* err;
-  long long timeoutTicks;   // 0 = wait for ever (MXG_HALO_TIMEOUT_S, default 120 s)
-};
-// A neighbour that never publishes its epoch means a dead or dead-locked rank. Continuing would compute boundary rows
-// from stale ghost values and return wrong numbers with a success code, so the wait records the fault in the mapped
-// error word and traps: every later call on the context fails loudly.
-__device__ __forceinline__ void haloWait(const WaitArgs& W, int k) {
-  const unsigned long long e = *W.epoch;
-  const volatile unsigned long long* f = W.flags + W.senderRank[k];
-  const long long t0 = clock64();
-  while (*f < e) {
-    if (W.timeoutTicks > 0 && clock64() - t0 > W.timeoutTicks) {
-      *W.err = 1;
-      __threadfence_system();
-      asm volatile("trap;");
-    }
-    __nanosleep(64);
-  }
-  __threadfence_system();
-}
 template <class T, bool GHOST, int NV>
 __global__ void __launch_bounds__(kBlock) k_spmm_multi(Segments G, DictArgs<T> D, SellArgs<T> S,
-                                                       XSource<T> X, ColTable<T> Y, int nvec, Epilogue<T> ep, WaitArgs W) {
-  if (GHOST && W.n > 0) {
-    if (threadIdx.x < W.n) haloWait(W, threadIdx.x);
-    __syncthreads();
-  }
-  if (GHOST && X.epoch) X.ghost += int64_t(*X.epoch & 1ull) * X.halfStride;
+                                                       XSource<T> X, ColTable<T> Y, int nvec, Epilogue<T> ep) {
   int seg = 0;
   while (seg < 3 && int(blockIdx.x) >= G.blockStart[seg + 1]) ++seg;
   const int64_t idx = G.begin[seg] + int64_t(int(blockIdx.x) - G.blockStart[seg]) * kBlock + threadIdx.x;
@@ -438,7 +403,7 @@ SellArgs<T> sellArgs(const mxg_crs* A) { return {A->dGenRow, A->dGenLen, A->dSli
 
 template <class T, bool GHOST>
 int launchSegments(const mxg_crs* A, const int64_t b[4], const int64_t e[4], const XSource<T>& X, const ColTable<T>& Y, int nvec,
-                   const Epilogue<T>& ep, cudaStream_t st, const WaitArgs& W) {
+                   const Epilogue<T>& ep, cudaStream_t st) {
   mxg_ctx* ctx = A->ctx;
   Segments G;
   int blocks = 0;
@@ -452,9 +417,9 @@ int launchSegments(const mxg_crs* A, const int64_t b[4], const int64_t e[4], con
   if (blocks == 0) return MXG_OK;
   const DictArgs<T> D = dictArgs<T>(A);
   const SellArgs<T> S = sellArgs<T>(A);
-  if (nvec == 1) k_spmm_multi<T, GHOST, 1><<<blocks, kBlock, 0, st>>>(G, D, S, X, Y, nvec, ep, W);
-  else if (nvec == 2) k_spmm_multi<T, GHOST, 2><<<blocks, kBlock, 0, st>>>(G, D, S, X, Y, nvec, ep, W);
-  else k_spmm_multi<T, GHOST, 4><<<blocks, kBlock, 0, st>>>(G, D, S, X, Y, nvec, ep, W);
+  if (nvec == 1) k_spmm_multi<T, GHOST, 1><<<blocks, kBlock, 0, st>>>(G, D, S, X, Y, nvec, ep);
+  else if (nvec == 2) k_spmm_multi<T, GHOST, 2><<<blocks, kBlock, 0, st>>>(G, D, S, X, Y, nvec, ep);
+  else k_spmm_multi<T, GHOST, 4><<<blocks, kBlock, 0, st>>>(G, D, S, X, Y, nvec, ep);
   LAUNCH_CHECK(ctx);
   return MXG_OK;
 }
@@ -493,17 +458,17 @@ int launchWin(const mxg_crs* A, int64_t rowBegin, int64_t rowEnd, const XSource<
   return MXG_OK;
 }
 
+// marks: record the per-kernel events of mxg_crs_apply_timed (prof[1..3]) around the launches
 template <class T, bool GHOST>
 int launchRange(const mxg_crs* A, int64_t rowBegin, int64_t rowEnd, int64_t genBegin, int64_t genEnd, const XSource<T>& X,
-                const ColTable<T>& Y, int nvec, const Epilogue<T>& ep, cudaStream_t st = nullptr) {
+                const ColTable<T>& Y, int nvec, const Epilogue<T>& ep, bool marks) {
   mxg_ctx* ctx = A->ctx;
-  if (!st) st = ctx->stream;
+  const cudaStream_t st = ctx->stream;
   // Two launches on purpose: a merged kernel carries the register footprint of the sliced-ELL path
   // (unrolled index/value arrays) and the lost occupancy costs the L1-bound dictionary rows ~35 %
   // (measured 0.406 ms vs 0.299 ms per apply on pillbox-256). Only the short boundary ranges use the
   // merged kernel (launchBoundary).
-  const bool prof = ctx->profiling;
-  if (prof) MXG_CUDA(cudaEventRecord(ctx->prof[1], ctx->stream));
+  if (marks) MXG_CUDA(cudaEventRecord(ctx->prof[1], st));
   // The windowed kernel wins for single vectors (0.232 vs 0.262 ms on pillbox-256); for blocks the gather kernels share
   // every pattern load between 4 vectors and stay ahead (profiles/README_r02.md), so they keep the block applies.
   if (A->dictRows > 0 && rowEnd > rowBegin && A->winR > 0 && nvec <= A->winMaxVec) {
@@ -524,7 +489,7 @@ int launchRange(const mxg_crs* A, int64_t rowBegin, int64_t rowEnd, int64_t genB
     }
     LAUNCH_CHECK(ctx);
   }
-  if (prof) MXG_CUDA(cudaEventRecord(ctx->prof[2], ctx->stream));
+  if (marks) MXG_CUDA(cudaEventRecord(ctx->prof[2], st));
   if (genEnd > genBegin) {
     const int64_t blocks = (genEnd - genBegin + kBlock - 1) / kBlock;
     const SellArgs<T> S = sellArgs<T>(A);
@@ -533,17 +498,16 @@ int launchRange(const mxg_crs* A, int64_t rowBegin, int64_t rowEnd, int64_t genB
     else k_spmm_sell<T, GHOST, 4><<<blocks, kBlock, 0, st>>>(genBegin, genEnd, S, X, Y, nvec, ep);
     LAUNCH_CHECK(ctx);
   }
-  if (prof) MXG_CUDA(cudaEventRecord(ctx->prof[3], ctx->stream));
+  if (marks) MXG_CUDA(cudaEventRecord(ctx->prof[3], st));
   return MXG_OK;
 }
 
 // leading + trailing boundary rows (dictionary and sliced ELL) in one launch on stream st
 template <class T>
-int launchBoundary(const mxg_crs* A, const XSource<T>& X, const ColTable<T>& Y, int nvec, const Epilogue<T>& ep, cudaStream_t st,
-                   const WaitArgs& W) {
+int launchBoundary(const mxg_crs* A, const XSource<T>& X, const ColTable<T>& Y, int nvec, const Epilogue<T>& ep, cudaStream_t st) {
   const int64_t b[4] = {0, A->intEnd, 0, A->genIntEnd};
   const int64_t e[4] = {A->dictRows > 0 ? A->intBegin : 0, A->dictRows > 0 ? A->nRows : A->intEnd, A->genIntBegin, A->nGen};
-  return launchSegments<T, true>(A, b, e, X, Y, nvec, ep, st, W);
+  return launchSegments<T, true>(A, b, e, X, Y, nvec, ep, st);
 }
 
 __host__ __device__ inline uint64_t mix64(uint64_t h, uint64_t v) {
@@ -553,6 +517,7 @@ __host__ __device__ inline uint64_t mix64(uint64_t h, uint64_t v) {
 }
 
 // ---- peer-memory halo exchange --------------------------------------------------------------
+// peer tables of the single-launch kernel, uploaded once per operator (mxg_crs::P2P::dArgs)
 struct P2PArgs {
   int n;
   void* ghost[8];
@@ -560,58 +525,8 @@ struct P2PArgs {
   int64_t sendOffset[8], sendCount[8], remoteStart[8], remoteGTot[8];
   int senderRank[8];
 };
-// sendBuf-less pack: x values go straight into the neighbours' ghost buffers (NVLink stores). The last
-// block to finish publishes the new epoch to every neighbour (release at system scope), so the
-// exchange is ONE kernel on the sender and no kernel on the receiver (the boundary-row kernel waits).
-template <class T>
-__global__ void __launch_bounds__(kBlock) k_pack_p2p(ColTable<T> x, const int32_t* __restrict__ idx, int64_t n, P2PArgs P,
-                                                     unsigned long long* epoch, unsigned int* done, int capCols) {
-  const T* __restrict__ c = x.p[blockIdx.y];
-  const unsigned long long e = *epoch + 1ull;
-  const unsigned long long par = e & 1ull;
-  for (int64_t i = blockIdx.x * int64_t(kBlock) + threadIdx.x; i < n; i += int64_t(gridDim.x) * kBlock) {
-    int k = 0;
-    while (k + 1 < P.n && i >= P.sendOffset[k] + P.sendCount[k]) ++k;
-    T* dst = static_cast<T*>(P.ghost[k]) + (int64_t(par) * capCols + blockIdx.y) * P.remoteGTot[k] + P.remoteStart[k] + (i - P.sendOffset[k]);
-    *dst = c[idx[i]];
-  }
-  __threadfence_system();
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    const unsigned int total = gridDim.x * gridDim.y;
-    if (atomicAdd(done, 1u) == total - 1u) {
-      *done = 0u;
-      __threadfence_system();
-      for (int k = 0; k < P.n; ++k) *reinterpret_cast<volatile unsigned long long*>(P.flag[k]) = e;
-      *epoch = e;
-      __threadfence_system();
-    }
-  }
-}
-
-// One warp waits until every neighbour has published this epoch (see haloWait for the timeout policy).
-// A separate tiny kernel on purpose: letting every boundary block spin instead keeps hundreds of blocks
-// resident while the interior rows want the SMs (measured: 0.22 ms vs 0.18 ms per apply at 2 GPUs).
-__global__ void k_wait(WaitArgs W) {
-  if (int(threadIdx.x) < W.n) haloWait(W, threadIdx.x);
-}
-
-template <class T>
-P2PArgs p2pArgs(const mxg_crs* A) {
-  P2PArgs P;
-  const auto& q = A->p2p;
-  P.n = q.npeers;
-  for (int k = 0; k < q.npeers; ++k) {
-    P.ghost[k] = q.peerGhost[k];
-    P.flag[k] = q.peerFlag[k];
-    P.remoteStart[k] = q.remoteStart[k];
-    P.remoteGTot[k] = q.remoteGTot[k];
-    P.senderRank[k] = q.peerRank[k];
-    for (const Peer& pr : A->peers)
-      if (pr.rank == q.peerRank[k]) { P.sendOffset[k] = pr.sendOffset; P.sendCount[k] = pr.sendCount; }
-  }
-  return P;
-}
+// the single launch serves this block: peer memory is set up and its ghost buffers are wide enough
+bool peerLaunch(const mxg_crs* A, int nvec) { return A->p2p.on && nvec <= A->p2p.capCols; }
 
 // ---- the whole multi-rank apply in ONE launch -------------------------------------------------------------------------------
 // Round 1 replayed a five-node graph (pack -> flag -> wait kernel -> boundary rows || interior rows) and measured ~100 us per
@@ -652,7 +567,7 @@ __device__ __forceinline__ void traceMark(unsigned long long* trace, int role, b
 }
 template <class T, int NV>
 __global__ void __launch_bounds__(kFusedBlock, (NV == 1 && sizeof(T) == 8) ? 5 : (NV <= 2 ? 4 : 3)) k_apply_fused(FusedPlan F, const P2PArgs* __restrict__ P, const int32_t* __restrict__ sendIdx,
-                                                             int64_t sendTotal, unsigned long long* epochDev, unsigned int* done, int capCols,
+                                                             int64_t sendTotal, unsigned int* done, int capCols,
                                                              DictArgs<T> D, SellArgs<T> S, XSource<T> X, ColTable<T> Y, int nvec,
                                                              Epilogue<T> ep, const unsigned long long* flags, int* err,
                                                              long long timeoutTicks) {
@@ -680,7 +595,6 @@ __global__ void __launch_bounds__(kFusedBlock, (NV == 1 && sizeof(T) == 8) ? 5 :
         *done = 0u;
         __threadfence_system();
         for (int k = 0; k < np; ++k) *reinterpret_cast<volatile unsigned long long*>(P->flag[k]) = F.epoch;
-        *epochDev = F.epoch;
         __threadfence_system();
       }
     }
@@ -705,7 +619,9 @@ __global__ void __launch_bounds__(kFusedBlock, (NV == 1 && sizeof(T) == 8) ? 5 :
     return;
   }
   b -= F.nDict;
-  // boundary rows
+  // boundary rows. A neighbour that never publishes this epoch means a dead or dead-locked rank. Continuing would compute
+  // boundary rows from stale ghost values and return wrong numbers with a success code, so the wait records the fault in the
+  // mapped error word and traps: every later call on the context fails loudly.
   traceMark(F.trace, 3, false);
   if (int(threadIdx.x) < P->n) {
     const volatile unsigned long long* f = flags + P->senderRank[threadIdx.x];
@@ -741,7 +657,17 @@ int launchFused(const mxg_crs* A, XSource<T> X, const ColTable<T>& Y, int nvec, 
   mxg_ctx* ctx = A->ctx;
   auto& q = A->p2p;
   if (!q.dArgs) {   // device copy of the (static) peer tables
-    const P2PArgs P = p2pArgs<T>(A);
+    P2PArgs P;
+    P.n = q.npeers;
+    for (int k = 0; k < q.npeers; ++k) {
+      P.ghost[k] = q.peerGhost[k];
+      P.flag[k] = q.peerFlag[k];
+      P.remoteStart[k] = q.remoteStart[k];
+      P.remoteGTot[k] = q.remoteGTot[k];
+      P.senderRank[k] = q.peerRank[k];
+      for (const Peer& pr : A->peers)
+        if (pr.rank == q.peerRank[k]) { P.sendOffset[k] = pr.sendOffset; P.sendCount[k] = pr.sendCount; }
+    }
     MXG_CUDA(cudaMalloc(&q.dArgs, sizeof(P2PArgs)));
     MXG_CUDA(cudaMemcpyAsync(q.dArgs, &P, sizeof(P2PArgs), cudaMemcpyHostToDevice, ctx->stream));
     MXG_CUDA(cudaStreamSynchronize(ctx->stream));
@@ -767,69 +693,25 @@ int launchFused(const mxg_crs* A, XSource<T> X, const ColTable<T>& Y, int nvec, 
   // the blocks after the interior rows are also what WAITS for the neighbours' flags: keep one even when nothing reads a ghost
   int sellBlocks = int((A->nGen - (F.sellIntEnd - F.sellIntBegin) + kFusedBlock - 1) / kFusedBlock);
   if (A->sendTotal > 0 && F.bndBlocks0 + F.bndBlocks1 + sellBlocks == 0) F.bndBlocks1 = 1;
-  X.halfStride = int64_t(q.capCols) * X.gTot;
-  X.ghost = static_cast<const T*>(q.ghost) + int64_t(F.epoch & 1ull) * X.halfStride;   // this epoch's half of the double buffer
-  X.epoch = nullptr;
+  X.ghost = static_cast<const T*>(q.ghost) + int64_t(F.epoch & 1ull) * q.capCols * X.gTot;   // this epoch's half of the double buffer
   const int grid = F.nPack + F.nSellInt + F.nDict + F.bndBlocks0 + F.bndBlocks1 + sellBlocks;
   const DictArgs<T> D = dictArgs<T>(A);
   const SellArgs<T> S = sellArgs<T>(A);
   const P2PArgs* dP = static_cast<const P2PArgs*>(q.dArgs);
   if (grid > 0) {
-    if (nvec == 1) k_apply_fused<T, 1><<<grid, kFusedBlock, 0, ctx->stream>>>(F, dP, A->dSendIdx, A->sendTotal, q.epoch, q.done, q.capCols, D, S, X, Y, nvec, ep, q.flags, ctx->dErr, ctx->haloTimeoutTicks);
-    else if (nvec == 2) k_apply_fused<T, 2><<<grid, kFusedBlock, 0, ctx->stream>>>(F, dP, A->dSendIdx, A->sendTotal, q.epoch, q.done, q.capCols, D, S, X, Y, nvec, ep, q.flags, ctx->dErr, ctx->haloTimeoutTicks);
-    else k_apply_fused<T, 4><<<grid, kFusedBlock, 0, ctx->stream>>>(F, dP, A->dSendIdx, A->sendTotal, q.epoch, q.done, q.capCols, D, S, X, Y, nvec, ep, q.flags, ctx->dErr, ctx->haloTimeoutTicks);
+    if (nvec == 1) k_apply_fused<T, 1><<<grid, kFusedBlock, 0, ctx->stream>>>(F, dP, A->dSendIdx, A->sendTotal, q.done, q.capCols, D, S, X, Y, nvec, ep, q.flags, ctx->dErr, ctx->haloTimeoutTicks);
+    else if (nvec == 2) k_apply_fused<T, 2><<<grid, kFusedBlock, 0, ctx->stream>>>(F, dP, A->dSendIdx, A->sendTotal, q.done, q.capCols, D, S, X, Y, nvec, ep, q.flags, ctx->dErr, ctx->haloTimeoutTicks);
+    else k_apply_fused<T, 4><<<grid, kFusedBlock, 0, ctx->stream>>>(F, dP, A->dSendIdx, A->sendTotal, q.done, q.capCols, D, S, X, Y, nvec, ep, q.flags, ctx->dErr, ctx->haloTimeoutTicks);
     LAUNCH_CHECK(ctx);
   }
   return MXG_OK;
 }
 
-// pack (remote stores) -> signal -> wait -> boundary rows on the communication stream || interior rows
-template <class T>
-int haloSequenceP2P(const mxg_crs* A, XSource<T> X, const ColTable<T>& Y, int nvec, const Epilogue<T>& ep) {
-  mxg_ctx* ctx = A->ctx;
-  const auto& q = A->p2p;
-  const P2PArgs P = p2pArgs<T>(A);
-  const bool prof = ctx->profiling;
-  MXG_CUDA(cudaEventRecord(ctx->evA, ctx->stream));
-  MXG_CUDA(cudaStreamWaitEvent(ctx->commStream, ctx->evA, 0));
-  if (prof) MXG_CUDA(cudaEventRecord(ctx->prof[1], ctx->commStream));
-  k_pack_p2p<T><<<dim3(gridFor(ctx, A->sendTotal, kBlock, 1), nvec), kBlock, 0, ctx->commStream>>>(X.x, A->dSendIdx, A->sendTotal, P, q.epoch, q.done, q.capCols);
-  LAUNCH_CHECK(ctx);
-  if (prof) MXG_CUDA(cudaEventRecord(ctx->prof[2], ctx->commStream));
-  X.ghost = static_cast<const T*>(q.ghost);
-  X.epoch = q.epoch;
-  X.halfStride = int64_t(q.capCols) * X.gTot;
-  WaitArgs W{};
-  W.n = P.n;
-  W.flags = q.flags;
-  W.epoch = q.epoch;
-  W.err = ctx->dErr;
-  W.timeoutTicks = ctx->haloTimeoutTicks;
-  for (int k = 0; k < P.n; ++k) W.senderRank[k] = P.senderRank[k];
-  k_wait<<<1, 32, 0, ctx->commStream>>>(W);
-  LAUNCH_CHECK(ctx);
-  ctx->profiling = false;
-  int rc;
-  { WaitArgs none{}; rc = launchBoundary<T>(A, X, Y, nvec, ep, ctx->commStream, none); }
-  ctx->profiling = prof;
-  if (rc) return rc;
-  MXG_CUDA(cudaEventRecord(ctx->evB, ctx->commStream));
-  if (prof) MXG_CUDA(cudaEventRecord(ctx->prof[3], ctx->commStream));
-  if (prof) MXG_CUDA(cudaEventRecord(ctx->prof[5], ctx->stream));
-  ctx->profiling = false;
-  rc = launchRange<T, false>(A, A->intBegin, A->intEnd, A->genIntBegin, A->genIntEnd, X, Y, nvec, ep);
-  ctx->profiling = prof;
-  if (rc) return rc;
-  if (prof) MXG_CUDA(cudaEventRecord(ctx->prof[8], ctx->stream));
-  MXG_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->evB, 0));
-  return MXG_OK;
-}
-
 // pack -> grouped ncclSend/ncclRecv on the communication stream || interior rows -> boundary rows
+// marks: record the phase events of mxg_crs_apply_timed (prof[1..3], prof[5])
 template <class T>
-int haloSequence(const mxg_crs* A, const XSource<T>& X, const ColTable<T>& Y, int nvec, const Epilogue<T>& ep) {
+int haloSequence(const mxg_crs* A, const XSource<T>& X, const ColTable<T>& Y, int nvec, const Epilogue<T>& ep, bool marks) {
   mxg_ctx* ctx = A->ctx;
-  if (A->p2p.on && nvec <= A->p2p.capCols) return haloSequenceP2P<T>(A, X, Y, nvec, ep);
   constexpr int w = sizeof(T) / sizeof(double);
   const int64_t gTot = A->gLo + A->gHi;
   // 1. pack boundary values and start the exchange on the communication stream
@@ -841,8 +723,7 @@ int haloSequence(const mxg_crs* A, const XSource<T>& X, const ColTable<T>& Y, in
   }
   MXG_CUDA(cudaEventRecord(ctx->evA, ctx->stream));
   MXG_CUDA(cudaStreamWaitEvent(ctx->commStream, ctx->evA, 0));
-  const bool prof = ctx->profiling;   // multi-rank phase timing (mxg_crs_apply_timed)
-  if (prof) MXG_CUDA(cudaEventRecord(ctx->prof[1], ctx->commStream));
+  if (marks) MXG_CUDA(cudaEventRecord(ctx->prof[1], ctx->commStream));
   MXG_NCCL(ncclGroupStart());
   for (const Peer& p : A->peers)
     for (int j = 0; j < nvec; ++j) {
@@ -852,21 +733,16 @@ int haloSequence(const mxg_crs* A, const XSource<T>& X, const ColTable<T>& Y, in
         MXG_NCCL(ncclRecv(ghost + j * gTot + p.recvStart, size_t(p.recvCount) * w, ncclDouble, p.rank, ctx->comm, ctx->commStream));
     }
   MXG_NCCL(ncclGroupEnd());
-  if (prof) MXG_CUDA(cudaEventRecord(ctx->prof[2], ctx->commStream));
+  if (marks) MXG_CUDA(cudaEventRecord(ctx->prof[2], ctx->commStream));
   // 2. boundary rows follow the receive ON THE COMMUNICATION STREAM, so exchange + boundary work
   //    overlap with the interior rows running on the compute stream (they write disjoint rows of y)
-  int rc = MXG_OK;
-  ctx->profiling = false;
-  { WaitArgs W{}; rc = launchBoundary<T>(A, X, Y, nvec, ep, ctx->commStream, W); }
-  if (rc) { ctx->profiling = prof; return rc; }
-  ctx->profiling = prof;
+  int rc = launchBoundary<T>(A, X, Y, nvec, ep, ctx->commStream);
+  if (rc) return rc;
   MXG_CUDA(cudaEventRecord(ctx->evB, ctx->commStream));
-  if (prof) MXG_CUDA(cudaEventRecord(ctx->prof[3], ctx->commStream));
+  if (marks) MXG_CUDA(cudaEventRecord(ctx->prof[3], ctx->commStream));
   // 3. rows that need no ghost values
-  if (prof) MXG_CUDA(cudaEventRecord(ctx->prof[5], ctx->stream));
-  ctx->profiling = false;   // launchRange's own single-rank markers would clobber ours
-  rc = launchRange<T, false>(A, A->intBegin, A->intEnd, A->genIntBegin, A->genIntEnd, X, Y, nvec, ep);
-  ctx->profiling = prof;
+  if (marks) MXG_CUDA(cudaEventRecord(ctx->prof[5], ctx->stream));
+  rc = launchRange<T, false>(A, A->intBegin, A->intEnd, A->genIntBegin, A->genIntEnd, X, Y, nvec, ep, false);
   if (rc) return rc;
   MXG_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->evB, 0));
   return MXG_OK;
@@ -878,8 +754,9 @@ int applyImpl(const mxg_crs* A, const mxg_mv* x, mxg_mv* y, const Epilogue<T>& e
   const int nvec = x->ncols;
   const int64_t gTot = A->gLo + A->gHi;
   const bool halo = ctx->nranks > 1 && (gTot > 0 || A->sendTotal > 0);
+  const bool timed = ctx->profiling;
   MXG_REQUIRE(*ctx->hErr == 0, "mxg_crs_apply: a previous halo exchange timed out waiting for a neighbour rank");
-  if (halo && A->haloCols < nvec && !(A->p2p.on && nvec <= A->p2p.capCols)) {
+  if (halo && A->haloCols < nvec && !peerLaunch(A, nvec)) {
     MXG_CUDA(cudaStreamSynchronize(ctx->stream));
     MXG_CUDA(cudaStreamSynchronize(ctx->commStream));
     if (A->dSendBuf) MXG_CUDA(cudaFree(A->dSendBuf));
@@ -897,24 +774,22 @@ int applyImpl(const mxg_crs* A, const mxg_mv* x, mxg_mv* y, const Epilogue<T>& e
   X.nLoc = A->nLoc;
   X.gLo = A->gLo;
   X.gTot = gTot;
-  X.epoch = nullptr;
-  X.halfStride = 0;
   ColTable<T> Y = tableOf<T>(y);
   if (!halo) {
     // MXG_FUSED_SELF=1 (profiling aid): run the single-launch kernel of the multi-rank path on one rank, with empty pack and
     // boundary roles, so that ncu can look at its interior role
     const bool fusedSelf = std::getenv("MXG_FUSED_SELF") != nullptr;
     if (fusedSelf && ctx->nranks == 1 && A->dictRows > 0) return launchFused<T>(A, X, Y, nvec, ep);
-    return launchRange<T, false>(A, 0, A->nRows, 0, A->nGen, X, Y, nvec, ep);
+    return launchRange<T, false>(A, 0, A->nRows, 0, A->nGen, X, Y, nvec, ep, timed);
   }
-  if (A->p2p.on && nvec <= A->p2p.capCols) {
-    ++A->p2p.hostEpoch;   // one epoch per exchange, on every path, so the device counter and all ranks stay in step
-    if (A->p2p.fused && !ctx->profiling) return launchFused<T>(A, X, Y, nvec, ep);
+  if (peerLaunch(A, nvec)) {
+    ++A->p2p.hostEpoch;   // one epoch per exchange, identical on all ranks
+    return launchFused<T>(A, X, Y, nvec, ep);
   }
 
   // The multi-rank apply is ~10 enqueues (pack, events, NCCL group, 2-6 kernels) for tens of
   // microseconds of GPU work, i.e. launch-bound. Capture it once per operand set and replay.
-  if (!ctx->graphsOff && !ctx->profiling) {
+  if (!ctx->graphsOff && !timed) {
     uint64_t key = mix64(0xC0FFEEull, uint64_t(nvec));
     for (int j = 0; j < nvec; ++j) { key = mix64(key, uint64_t(x->col[j])); key = mix64(key, uint64_t(y->col[j])); }
     uint64_t epBits[(sizeof(Epilogue<T>) + 7) / 8] = {};
@@ -929,7 +804,7 @@ int applyImpl(const mxg_crs* A, const mxg_mv* x, mxg_mv* y, const Epilogue<T>& e
     const int64_t before = ctx->launches;
     cudaGraph_t graph = nullptr;
     if (cudaStreamBeginCapture(ctx->stream, cudaStreamCaptureModeRelaxed) == cudaSuccess) {
-      const int rcCap = haloSequence<T>(A, X, Y, nvec, ep);
+      const int rcCap = haloSequence<T>(A, X, Y, nvec, ep, false);
       const cudaError_t endErr = cudaStreamEndCapture(ctx->stream, &graph);
       cudaGraphExec_t exec = nullptr;
       if (rcCap == MXG_OK && endErr == cudaSuccess && graph && cudaGraphInstantiate(&exec, graph, 0) == cudaSuccess) {
@@ -945,7 +820,7 @@ int applyImpl(const mxg_crs* A, const mxg_mv* x, mxg_mv* y, const Epilogue<T>& e
     ctx->launches = before;
     ctx->graphsOff = true;
   }
-  return haloSequence<T>(A, X, Y, nvec, ep);
+  return haloSequence<T>(A, X, Y, nvec, ep, timed);
 }
 
 // ---- host-side layout construction --------------------------------------------------------
@@ -997,11 +872,10 @@ int setupP2P(mxg_crs* A, int64_t gTot) {
   if (eligible) {
     const size_t gb = size_t(2) * cap * std::max<int64_t>(gTot, 1) * esz;
     bool ok = cudaMalloc(&q.ghost, gb) == cudaSuccess && cudaMalloc(&q.flags, sizeof(unsigned long long) * R) == cudaSuccess &&
-              cudaMalloc(&q.epoch, sizeof(unsigned long long)) == cudaSuccess && cudaMalloc(&q.done, sizeof(unsigned int)) == cudaSuccess;
+              cudaMalloc(&q.done, sizeof(unsigned int)) == cudaSuccess;
     if (ok) {
       cudaMemsetAsync(q.ghost, 0, gb, ctx->stream);
       cudaMemsetAsync(q.flags, 0, sizeof(unsigned long long) * R, ctx->stream);
-      cudaMemsetAsync(q.epoch, 0, sizeof(unsigned long long), ctx->stream);
       cudaMemsetAsync(q.done, 0, sizeof(unsigned int), ctx->stream);
       cudaStreamSynchronize(ctx->stream);
       ok = cudaIpcGetMemHandle(&mineH.ghost, q.ghost) == cudaSuccess && cudaIpcGetMemHandle(&mineH.flags, q.flags) == cudaSuccess;
@@ -1051,10 +925,6 @@ int setupP2P(mxg_crs* A, int64_t gTot) {
   MXG_CUDA(cudaFree(dflag));
   q.capCols = cap;
   q.on = opened == 1 && (gTot > 0 || A->sendTotal > 0);
-  {
-    const char* f = std::getenv("MXG_HALO_FUSED");   // 0: the multi-kernel graph of round 1
-    q.fused = !(f && std::strcmp(f, "0") == 0);
-  }
   return MXG_OK;
 }
 
@@ -1857,7 +1727,6 @@ int mxg_crs_destroy(mxg_crs* A) {
   for (void* o : A->p2p.opened) cudaIpcCloseMemHandle(o);
   if (A->p2p.ghost) cudaFree(A->p2p.ghost);
   if (A->p2p.flags) cudaFree(A->p2p.flags);
-  if (A->p2p.epoch) cudaFree(A->p2p.epoch);
   if (A->p2p.done) cudaFree(A->p2p.done);
   if (A->p2p.trace) cudaFree(A->p2p.trace);
   if (A->p2p.dArgs) cudaFree(A->p2p.dArgs);
@@ -1969,23 +1838,55 @@ int mxg_crs_apply_axpby(const mxg_crs* A, const double alpha[2], const mxg_mv* x
 }
 
 int mxg_crs_apply_timed(const mxg_crs* A, const mxg_mv* x, mxg_mv* y, double ms[4]) {
-  MXG_REQUIRE(A && ms, "mxg_crs_apply_timed: NULL argument");
+  MXG_REQUIRE(ms, "mxg_crs_apply_timed: NULL argument");
+  int rc = checkApply("mxg_crs_apply_timed", A, x, y);
+  if (rc) return rc;
   mxg_ctx* ctx = A->ctx;
   MXG_CUDA(cudaSetDevice(ctx->device));
   for (auto& e : ctx->prof)
     if (!e) MXG_CUDA(cudaEventCreate(&e));
-  MXG_CUDA(cudaEventRecord(ctx->prof[0], ctx->stream));
-  ctx->profiling = true;
-  int rc = mxg_crs_apply(A, x, y);
-  ctx->profiling = false;
+  // the single launch is one kernel: its phases come from the %globaltimer marks of its roles, not from events
+  const bool peer = peerLaunch(A, x->ncols);
+  if (peer) {
+    rc = mxg_crs_trace(A, 1, nullptr);
+    if (rc) return rc;
+  }
+  auto timedApply = [&]() -> int {
+    MXG_CUDA(cudaEventRecord(ctx->prof[0], ctx->stream));
+    ctx->profiling = true;
+    const int rcApply = mxg_crs_apply(A, x, y);
+    ctx->profiling = false;
+    if (rcApply) return rcApply;
+    MXG_CUDA(cudaEventRecord(ctx->prof[4], ctx->stream));
+    MXG_CUDA(cudaEventSynchronize(ctx->prof[4]));
+    MXG_CUDA(cudaStreamSynchronize(ctx->commStream));
+    return MXG_OK;
+  };
+  rc = timedApply();
+  double t[10];
+  if (peer) {   // read back and disarm, also when the apply failed
+    const int rcTrace = mxg_crs_trace(A, 0, t);
+    if (!rc) rc = rcTrace;
+  }
   if (rc) return rc;
-  MXG_CUDA(cudaEventRecord(ctx->prof[4], ctx->stream));
-  MXG_CUDA(cudaEventSynchronize(ctx->prof[4]));
-  MXG_CUDA(cudaStreamSynchronize(ctx->commStream));
   float f = 0;
   ms[0] = ms[1] = ms[2] = 0;
   const bool halo = ctx->nranks > 1 && (A->gLo + A->gHi > 0 || A->sendTotal > 0);
-  if (!halo) {
+  if (peer) {
+    // first start to last end over roles r0..r1, ns -> ms; a role that did not run (-1) counts 0
+    auto span = [&t](int r0, int r1) {
+      double lo = -1, hi = -1;
+      for (int r = r0; r <= r1; ++r) {
+        if (t[2 * r] < 0) continue;
+        if (lo < 0 || t[2 * r] < lo) lo = t[2 * r];
+        if (t[2 * r + 1] > hi) hi = t[2 * r + 1];
+      }
+      return lo < 0 ? 0.0 : (hi - lo) * 1e-6;
+    };
+    ms[0] = span(1, 2);   // interior dictionary + sliced-ELL rows
+    ms[1] = span(4, 4);   // boundary rows
+    ms[2] = span(0, 0);   // pack + flag publish
+  } else if (!halo) {
     MXG_CUDA(cudaEventElapsedTime(&f, ctx->prof[1], ctx->prof[2])); ms[0] = f;   // dictionary kernel
     MXG_CUDA(cudaEventElapsedTime(&f, ctx->prof[2], ctx->prof[3])); ms[1] = f;   // sliced-ELL kernel
     MXG_CUDA(cudaEventElapsedTime(&f, ctx->prof[0], ctx->prof[1])); ms[2] = f;

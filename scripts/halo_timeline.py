@@ -1,5 +1,5 @@
-"""Multi-rank apply: single-launch (fused) path vs the round-1 multi-kernel graph on the SAME box and operator, plus a
-%globaltimer timeline of the fused kernel's roles on every rank. Launch with torchrun (one process per GPU):
+"""Multi-rank apply: single-launch (fused) path vs the NCCL exchange on the SAME box and operator, plus a %globaltimer
+timeline of the fused kernel's roles on every rank. Launch with torchrun (one process per GPU):
   python -m torch.distributed.run --nproc-per-node N --master-addr 127.0.0.1 scripts/halo_timeline.py [--size 256] [--nvec 1]"""
 import argparse
 import json
@@ -41,9 +41,8 @@ cuts = bench.slab_ranges(rg, n_global, world, args.size)
 r0, r1 = cuts[rank], cuts[rank + 1]
 bmap = mx.MxMap(ctx, n_global, np.ascontiguousarray(rg[r0:r1]))
 ops = {}
-for name, env in (("fused", {"MXG_HALO_FUSED": "1"}), ("graph", {"MXG_HALO_FUSED": "0"}), ("nccl", {"MXG_HALO": "nccl"})):
-    for k in ("MXG_HALO_FUSED", "MXG_HALO"):
-        os.environ.pop(k, None)
+for name, env in (("fused", {}), ("nccl", {"MXG_HALO": "nccl"})):
+    os.environ.pop("MXG_HALO", None)
     os.environ.update(env)
     ops[name] = bench.upload_block(mx, m, bmap, bmap, r0, r1)
 out = {"world": world, "rows_rank0": int(r1 - r0)}

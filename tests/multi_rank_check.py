@@ -17,6 +17,15 @@ from maxwell_b200.partition import local_block, slab_cuts  # noqa: E402
 from oracle import oracle as orc  # noqa: E402
 
 
+def _assert_matches_global(got, ref, is_complex, what):
+    """bit for bit for real operators, to 1e-14 (relative 2-norm) for complex ones"""
+    if is_complex:
+        err = np.linalg.norm(got - ref) / np.linalg.norm(ref)
+        assert err < 1e-14, what + (err,)
+    else:
+        assert np.array_equal(got, ref), what + ("halo apply differs from the global apply",)
+
+
 def _block(m, cuts, rank):
     rowptr, col, val = m.arrays()
     rg, cg = m.maps()
@@ -174,12 +183,15 @@ def main():
             for rep in range(3):                      # repeated applies reuse the ghost buffers
                 A.apply(x, y)
             yg = op.apply(xg)
-            got = y.to_host()
-            if op.is_complex:
-                err = np.linalg.norm(got - yg[r0:r1]) / np.linalg.norm(yg[r0:r1])
-                assert err < 1e-14, (label, layout, err)
-            else:
-                assert np.array_equal(got, yg[r0:r1]), (label, layout, "halo apply differs from the global apply")
+            _assert_matches_global(y.to_host(), yg[r0:r1], op.is_complex, (label, layout))
+            # the timed apply takes the same path as apply, so it must compute the same y
+            ms = A.apply_timed(x, y)
+            _assert_matches_global(y.to_host(), yg[r0:r1], op.is_complex, (label, layout, "apply_timed"))
+            assert all(0 <= ms[k] <= ms["total_ms"] for k in ("dict_ms", "sell_ms", "pre_ms")), (label, layout, ms)
+            if not op.is_complex and os.environ.get("MXG_HALO") != "nccl":
+                # default path on one node: the single launch, whose pack and boundary-row roles both run on every rank here
+                tl = A.trace_apply(x, y)
+                assert -1 not in tl["pack"] and -1 not in tl["boundary_rows"], (label, layout, tl)
             np.testing.assert_allclose(x.norm2(), np.linalg.norm(xg, axis=0), rtol=1e-13)
             np.testing.assert_allclose(y.dot(x), np.einsum("ij,ij->j", xg.conj(), yg), rtol=1e-11, atol=1e-8)
             G = y.MvTransMv(1.0, x)
