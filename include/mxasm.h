@@ -88,25 +88,50 @@ int mxg_sim_make_map(mxg_sim* sim, const char* field, int64_t begin, int64_t end
  * factors of the chains (NULL: generated from the simulation's dielectric objects, identity without any). */
 int mxg_sim_op(mxg_sim* sim, const char* name, int is_complex, const mxg_dcsr* inv_eps, const mxg_dcsr* inv_eps_vol_ave,
                mxg_dcsr** out);
+/* The rows [row_begin, row_end) (positions in the row field's map) of mxg_sim_op's operator, bit for bit, assembled from
+ * the rows the chain needs only: each factor on the rows the factor to its left references (an x-slab +- the stencil
+ * reach, wrapping around on periodic-x grids), multiplied in the reference's association order (MxMagWaveOp.cpp:137-245,
+ * MxEMOps.cpp:39-168). inv_eps / inv_eps_vol_ave may be whole or partial; they must store the rows the chain needs.
+ * Out-of-range or inverted ranges return an error code. */
+int mxg_sim_op_rows(mxg_sim* sim, const char* name, int is_complex, const mxg_dcsr* inv_eps, const mxg_dcsr* inv_eps_vol_ave,
+                    int64_t row_begin, int64_t row_end, mxg_dcsr** out);
 int mxg_dcsr_upload(mxg_sim* sim, const char* row_field, const char* col_field, int64_t nrows, int64_t ncols,
                     const int64_t* rowptr, const int32_t* col, const double* vals, int is_complex, mxg_dcsr** out);
+/* A matrix may store only some rows of its map (mxg_dcsr_rows). multiply: rows of a x b on a's stored rows; b must store
+ * every row a's columns reference, otherwise an error ("a column of A has no stored row in B"). add: b must store a's rows. */
 int mxg_dcsr_multiply(const mxg_dcsr* a, const mxg_dcsr* b, mxg_dcsr** out);                     /* MxCrsMatrix.cpp:358-382 */
 int mxg_dcsr_add(const mxg_dcsr* a, const double sa[2], const mxg_dcsr* b, const double sb[2], int purge, mxg_dcsr** out); /* :401-430 */
 int mxg_dcsr_purge(const mxg_dcsr* a, mxg_dcsr** out);                                           /* MxCrsMatrix.cpp:84-117 */
 int mxg_dcsr_scale(mxg_dcsr* a, const double s[2]);
-int mxg_dcsr_transpose(const mxg_dcsr* a, mxg_dcsr** out); /* conjugate transpose, rows sorted by column */
+/* conjugate transpose, rows sorted by column; a must store all its rows (the rows of a restriction:
+ * mxg_sim_interpolator_transpose_rows) */
+int mxg_dcsr_transpose(const mxg_dcsr* a, mxg_dcsr** out);
 /* MxGridFieldInterpolator (MxGridFieldInterpolator.cpp:28-122): `field` of sim_from interpolated at the DOFs of sim_to --
  * the refiners / coarseners of MxGeoMultigridPrec (MxGeoMultigridPrec.cpp:98-240). Rows on sim_to, columns on sim_from. */
 int mxg_sim_interpolator(mxg_sim* sim_from, mxg_sim* sim_to, const char* field, int is_complex, mxg_dcsr** out);
-/* out = {rows, columns, entries, is_complex, row field, column field}; fields 0 B, 1 E, 2 psi, -1 unknown */
+/* rows [row_begin, row_end) of sim_to's map of the same interpolator (MxGridFieldInterpolator.cpp:28-122) */
+int mxg_sim_interpolator_rows(mxg_sim* sim_from, mxg_sim* sim_to, const char* field, int is_complex,
+                              int64_t row_begin, int64_t row_end, mxg_dcsr** out);
+/* rows [row_begin, row_end) of sim_from's map of its conjugate transpose (the restriction of MxGeoMultigridPrec.cpp:98-240
+ * before the 1/8 scaling): the interpolator is generated on the fine rows that can reach those coarse rows only */
+int mxg_sim_interpolator_transpose_rows(mxg_sim* sim_from, mxg_sim* sim_to, const char* field, int is_complex,
+                                        int64_t row_begin, int64_t row_end, mxg_dcsr** out);
+/* out = {rows, columns, entries, is_complex, row field, column field}; fields 0 B, 1 E, 2 psi, -1 unknown. rows counts
+ * the stored rows. */
 int mxg_dcsr_shape(const mxg_dcsr* a, int64_t out[6]);
-/* rows [row_begin, row_end) to the host; rowptr is rebased to 0; col / vals may be NULL */
+/* out = {first, end}: map positions of the stored rows (0 and the map size for a whole-map matrix) */
+int mxg_dcsr_rows(const mxg_dcsr* a, int64_t out[2]);
+/* stored rows [row_begin, row_end) to the host; rowptr is rebased to 0; col / vals may be NULL */
 int mxg_dcsr_download(const mxg_dcsr* a, int64_t row_begin, int64_t row_end, int64_t* rowptr, int32_t* col, double* vals);
 int mxg_dcsr_destroy(mxg_dcsr* a);
 
 /* MxCrsMatrix::fillComplete (MxCrsMatrix.cpp:325-342) for a device-assembled operator: the rows row_map owns become an
  * mxg_crs (layout: MXG_LAYOUT_* of mxgpu.h, 0 = default). Collective when the context has several ranks. */
 int mxg_crs_create_from_dcsr(mxg_map* row_map, mxg_map* domain_map, const mxg_dcsr* a, int layout, mxg_crs** out);
+
+/* Device bytes held by the assembly of a context's simulations (fractions, maps, matrices, temporaries):
+ * out = {current, peak}; reset_peak != 0 restarts the peak at the current value. */
+int mxg_asm_memory(mxg_ctx* ctx, int64_t out[2], int reset_peak);
 
 #ifdef __cplusplus
 }

@@ -41,6 +41,7 @@ class AssemblyAPI:
             "sim_map_copy": [vp, C.c_char_p, vp],
             "sim_fractions": [vp, C.c_char_p, vp],
             "sim_op": [vp, C.c_char_p, i32, vp, vp, pvp],
+            "sim_op_rows": [vp, C.c_char_p, i32, vp, vp, i64, i64, pvp],
             "dcsr_upload": [vp, C.c_char_p, C.c_char_p, i64, i64, vp, vp, vp, i32, pvp],
             "dcsr_multiply": [vp, vp, pvp],
             "dcsr_add": [vp, d3, vp, d3, i32, pvp],
@@ -48,7 +49,10 @@ class AssemblyAPI:
             "dcsr_scale": [vp, d3],
             "dcsr_transpose": [vp, pvp],
             "sim_interpolator": [vp, vp, C.c_char_p, i32, pvp],
+            "sim_interpolator_rows": [vp, vp, C.c_char_p, i32, i64, i64, pvp],
+            "sim_interpolator_transpose_rows": [vp, vp, C.c_char_p, i32, i64, i64, pvp],
             "dcsr_shape": [vp, C.POINTER(i64)],
+            "dcsr_rows": [vp, C.POINTER(i64)],
             "dcsr_download": [vp, i64, i64, vp, vp, vp],
             "dcsr_destroy": [vp],
             "shape_cylinder": [dbl, d3, d3, pvp],
@@ -245,26 +249,52 @@ class Sim:
         self.api.call("sim_fractions", self.handle, field.encode(), out.ctypes.data)
         return out
 
-    def op(self, name, is_complex=None, inv_eps=None, inv_eps_vol_ave=None):
+    def op(self, name, is_complex=None, inv_eps=None, inv_eps_vol_ave=None, rows=None):
+        """A named operator; rows=(begin, end) assembles only those rows of its row map (bit for bit the same rows)."""
         if not self._setup:
             self.setup()
         cplx = self.is_complex if is_complex is None else bool(is_complex)
         h = C.c_void_p()
-        self.api.call("sim_op", self.handle, name.encode(), 1 if cplx else 0, inv_eps.handle if inv_eps is not None else None,
-                      inv_eps_vol_ave.handle if inv_eps_vol_ave is not None else None, C.byref(h))
+        eps = (inv_eps.handle if inv_eps is not None else None, inv_eps_vol_ave.handle if inv_eps_vol_ave is not None else None)
+        if rows is None:
+            self.api.call("sim_op", self.handle, name.encode(), 1 if cplx else 0, *eps, C.byref(h))
+        else:
+            self.api.call("sim_op_rows", self.handle, name.encode(), 1 if cplx else 0, *eps, int(rows[0]), int(rows[1]), C.byref(h))
         return DeviceCsr(self, h)
 
-    def interpolator_from(self, coarse, field="bfield", is_complex=None):
-        """MxGridFieldInterpolator: `field` of the simulation `coarse` interpolated at this simulation's DOFs."""
+    def _setup_both(self, coarse):
         if not self._setup:
             self.setup()
         if not coarse._setup:
             coarse.setup()
+
+    def interpolator_from(self, coarse, field="bfield", is_complex=None, rows=None):
+        """MxGridFieldInterpolator: `field` of the simulation `coarse` interpolated at this simulation's DOFs (rows=(begin, end):
+        only those rows of this simulation's map)."""
+        self._setup_both(coarse)
         cplx = self.is_complex if is_complex is None else bool(is_complex)
         h = C.c_void_p()
-        self.api.call("sim_interpolator", coarse.handle, self.handle, field.encode(), 1 if cplx else 0, C.byref(h))
+        if rows is None:
+            self.api.call("sim_interpolator", coarse.handle, self.handle, field.encode(), 1 if cplx else 0, C.byref(h))
+        else:
+            self.api.call("sim_interpolator_rows", coarse.handle, self.handle, field.encode(), 1 if cplx else 0, int(rows[0]),
+                          int(rows[1]), C.byref(h))
         m = DeviceCsr(self, h)
         m.col_sim = coarse
+        return m
+
+    def interpolator_transpose(self, coarse, field="bfield", is_complex=None, rows=None):
+        """The rows (begin, end) of the coarse map of interpolator_from(coarse, field)'s conjugate transpose (the restriction
+        before its 1/8 scaling), generating the interpolator on the fine rows that reach them only. rows=None: all rows."""
+        self._setup_both(coarse)
+        cplx = self.is_complex if is_complex is None else bool(is_complex)
+        if rows is None:
+            rows = (0, coarse.map_size(field)[0])
+        h = C.c_void_p()
+        self.api.call("sim_interpolator_transpose_rows", coarse.handle, self.handle, field.encode(), 1 if cplx else 0, int(rows[0]),
+                      int(rows[1]), C.byref(h))
+        m = DeviceCsr(self, h)
+        m.row_sim, m.col_sim = coarse, self
         return m
 
     def upload(self, row_field, col_field, rowptr, col, val, ncols):
@@ -297,8 +327,12 @@ class DeviceCsr:
         self.nrows, self.ncols, self.nnz, self.is_complex = s[0], s[1], s[2], bool(s[3])
         self.row_field = FIELDS[s[4]] if s[4] >= 0 else None
         self.col_field = FIELDS[s[5]] if s[5] >= 0 else None
+        r = (C.c_int64 * 2)()
+        self.api.call("dcsr_rows", handle, r)
+        self.row_begin = r[0]          # map position of the first stored row (nrows counts the stored rows)
 
     def arrays(self, row_begin=0, row_end=None):
+        """Stored rows [row_begin, row_end): rowptr rebased to 0, column positions in the whole column map, values."""
         row_end = self.nrows if row_end is None else row_end
         rowptr = np.empty(row_end - row_begin + 1, dtype=np.int64)
         self.api.call("dcsr_download", self.handle, row_begin, row_end, rowptr.ctypes.data, None, None)
@@ -364,6 +398,8 @@ def gpu_api():
         L.mxg_crs_create_from_dcsr.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.POINTER(C.c_void_p)]
         L.mxg_sim_make_map.restype = C.c_int
         L.mxg_sim_make_map.argtypes = [C.c_void_p, C.c_char_p, C.c_int64, C.c_int64, C.POINTER(C.c_void_p)]
+        L.mxg_asm_memory.restype = C.c_int
+        L.mxg_asm_memory.argtypes = [C.c_void_p, C.POINTER(C.c_int64), C.c_int]
         _GPU_API = api
     return _GPU_API
 
@@ -388,6 +424,15 @@ def make_map(sim, field, begin=0, end=-1):
     gids = sim.map(field)
     m.gids = gids[begin:(len(gids) if end < 0 else end)]
     return m
+
+
+def asm_memory(ctx, reset_peak=False):
+    """(current, peak) device bytes held by the operator assembly of a context (include/mxasm.h: mxg_asm_memory)."""
+    api = gpu_api()
+    out = (C.c_int64 * 2)()
+    if api.lib.mxg_asm_memory(ctx.h, out, 1 if reset_peak else 0) != 0:
+        raise AssemblyError("mxg_asm_memory failed: %s" % api.lib.mxg_last_error().decode())
+    return out[0], out[1]
 
 
 def to_crs(dcsr, row_map, domain_map, layout=0):
@@ -486,7 +531,9 @@ class EigenProblem:
     (restriction = P^T / 8), divB / gradPsi / curlCurl on the fine grid and the mass diagonal dmA.
 
     sims: device simulations, fine to coarse. cuts(level, field, gids, num_global) -> (begin, end) selects this rank's
-    rows of a field map (x-slabs); None = the whole map (one rank)."""
+    rows of a field map (x-slabs); None = the whole map (one rank). Every operator, transfer and the mass diagonal is
+    assembled on this rank's rows only (each chain factor on the rows its left neighbour reaches), so a rank's assembly
+    memory and time shrink with the rank count; the rows are bit-identical to those of the global operators."""
 
     def __init__(self, ctx, sims, cuts=None, is_complex=False):
         import maxwell_b200 as mx
@@ -494,25 +541,29 @@ class EigenProblem:
         rng = {}
         for l, s in enumerate(sims):
             for f in ("bfield", "psifield"):
-                g = s.map(f)
-                rng[l, f] = (0, len(g)) if cuts is None else cuts(l, f, g, s.num_global(f))
+                if cuts is None:
+                    rng[l, f] = (0, s.map_size(f)[0])
+                else:
+                    rng[l, f] = cuts(l, f, s.map(f), s.num_global(f))
         self.bmaps = [make_map(s, "bfield", *rng[l, "bfield"]) for l, s in enumerate(sims)]
         self.pmaps = [make_map(s, "psifield", *rng[l, "psifield"]) for l, s in enumerate(sims)]
         cx = is_complex
-        self.vops = [to_crs(s.op("vecLapl", cx), self.bmaps[l], self.bmaps[l]) for l, s in enumerate(sims)]
-        self.sops = [to_crs(s.op("scaLapl", cx), self.pmaps[l], self.pmaps[l]) for l, s in enumerate(sims)]
+        self.vops = [to_crs(s.op("vecLapl", cx, rows=rng[l, "bfield"]), self.bmaps[l], self.bmaps[l]) for l, s in enumerate(sims)]
+        self.sops = [to_crs(s.op("scaLapl", cx, rows=rng[l, "psifield"]), self.pmaps[l], self.pmaps[l]) for l, s in enumerate(sims)]
         self.Rb, self.Pb, self.Rp, self.Pp = [], [], [], []
         for l in range(len(sims) - 1):
             for f, maps, Rl, Pl in (("bfield", self.bmaps, self.Rb, self.Pb), ("psifield", self.pmaps, self.Rp, self.Pp)):
-                p = sims[l].interpolator_from(sims[l + 1], f, cx)
+                p = sims[l].interpolator_from(sims[l + 1], f, cx, rows=rng[l, f])
                 Pl.append(to_crs(p, maps[l], maps[l + 1]))
-                Rl.append(to_crs(p.transpose(scale=0.125), maps[l + 1], maps[l]))
+                del p
+                r = sims[l].interpolator_transpose(sims[l + 1], f, cx, rows=rng[l + 1, f]).scale(0.125)
+                Rl.append(to_crs(r, maps[l + 1], maps[l]))
         s0 = sims[0]
-        self.divB = to_crs(s0.op("divB", cx), self.pmaps[0], self.bmaps[0])
-        self.gradPsi = to_crs(s0.op("gradPsi", cx), self.bmaps[0], self.pmaps[0])
-        self.curlCurl = to_crs(s0.op("curlCurl", cx), self.bmaps[0], self.bmaps[0])
         b0, b1 = rng[0, "bfield"]
-        fa = s0.op("dmA", False).arrays(b0, b1)[2]
+        self.divB = to_crs(s0.op("divB", cx, rows=rng[0, "psifield"]), self.pmaps[0], self.bmaps[0])
+        self.gradPsi = to_crs(s0.op("gradPsi", cx, rows=(b0, b1)), self.bmaps[0], self.pmaps[0])
+        self.curlCurl = to_crs(s0.op("curlCurl", cx, rows=(b0, b1)), self.bmaps[0], self.bmaps[0])
+        fa = s0.op("dmA", False, rows=(b0, b1)).arrays()[2]
         self.m_diag = mx.MxMultiVector(self.bmaps[0], 1, cx)
         self.m_diag.from_host(fa.astype(np.complex128) if cx else fa)
         self.fracs = fa

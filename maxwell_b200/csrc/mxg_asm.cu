@@ -8,6 +8,7 @@
 #include <algorithm>
 #include <cstring>
 #include <string>
+#include <unordered_map>
 
 #include "mxasm.h"
 #include "mxg_internal.h"
@@ -37,6 +38,7 @@ __global__ void __launch_bounds__(kAsmBlock) k_asm_max(const int32_t* __restrict
 
 struct DeviceExec {
   mxg_ctx* ctx;
+  std::unordered_map<void*, size_t> sizes;   // live allocations, counted into ctx->asmBytes / asmPeak
   explicit DeviceExec(mxg_ctx* c) : ctx(c) {
     if (!c) throw std::runtime_error("operator assembly needs a context (mxg_ctx_create)");
     cudaSetDevice(c->device);
@@ -44,11 +46,23 @@ struct DeviceExec {
   template <class T>
   T* alloc(int64_t n) {
     void* p = nullptr;
-    const cudaError_t e = cudaMalloc(&p, size_t(n > 0 ? n : 1) * sizeof(T));
+    const size_t bytes = size_t(n > 0 ? n : 1) * sizeof(T);
+    const cudaError_t e = cudaMalloc(&p, bytes);
     if (e != cudaSuccess) fail("device allocation of the operator assembly", e);
+    sizes[p] = bytes;
+    ctx->asmBytes += int64_t(bytes);
+    ctx->asmPeak = std::max(ctx->asmPeak, ctx->asmBytes);
     return static_cast<T*>(p);
   }
-  void free(void* p) { if (p) cudaFree(p); }
+  void free(void* p) {
+    if (!p) return;
+    const auto it = sizes.find(p);
+    if (it != sizes.end()) {
+      ctx->asmBytes -= int64_t(it->second);
+      sizes.erase(it);
+    }
+    cudaFree(p);
+  }
   void check(const char* what) {
     const cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) fail(what, e);
@@ -139,7 +153,7 @@ int mxg_crs_create_from_dcsr(mxg_map* row_map, mxg_map* domain_map, const mxg_dc
     mxa::Assembler<DeviceExec>& asC = *A->cols()->as;
     MXG_REQUIRE(domain_map->nGlobal == asC.numGlobal(cf) && row_map->nGlobal == asR.numGlobal(rf),
                 "mxg_crs_create_from_dcsr: maps do not span the simulation's GID space");
-    MXG_REQUIRE(asR.mapSize(rf) == A->nrows() && asC.mapSize(cf) == A->ncols(), "mxg_crs_create_from_dcsr: the matrix does not live on these field maps");
+    MXG_REQUIRE(asR.mapSize(rf) == A->mapRows() && asC.mapSize(cf) == A->ncols(), "mxg_crs_create_from_dcsr: the matrix does not live on these field maps");
     std::vector<int64_t> rowG(static_cast<size_t>(asR.mapSize(rf)), 0), colG(static_cast<size_t>(asC.mapSize(cf)), 0);
     asR.copyMap(rf, rowG.data());
     asC.copyMap(cf, colG.data());
@@ -152,6 +166,11 @@ int mxg_crs_create_from_dcsr(mxg_map* row_map, mxg_map* domain_map, const mxg_dc
                   "mxg_crs_create_from_dcsr: the row map is not a contiguous run of the simulation's %s map",
                   rf == mxy::FIELD_B ? "B" : (rf == mxy::FIELD_E ? "E" : "psi"));
     }
+    // ... which the matrix must store (a slab operator from mxg_sim_op_rows stores its rows only)
+    const int64_t s0 = r0 - A->rowBegin();
+    MXG_REQUIRE(r1 == r0 || (s0 >= 0 && s0 + (r1 - r0) <= A->nrows()),
+                "mxg_crs_create_from_dcsr: the matrix stores the rows [%lld, %lld) of its map, not the row map's [%lld, %lld)",
+                (long long)A->rowBegin(), (long long)(A->rowBegin() + A->nrows()), (long long)r0, (long long)r1);
     // this rank's columns: the run of the column field map its domain map owns
     int64_t c0 = 0;
     bool domIsRun = true;
@@ -161,7 +180,7 @@ int mxg_crs_create_from_dcsr(mxg_map* row_map, mxg_map* domain_map, const mxg_dc
                  std::memcmp(colG.data() + c0, domain_map->gids.data(), size_t(domain_map->nLocal) * sizeof(int64_t)) == 0;
     }
     if (domIsRun && row_map->perm.empty() && domain_map->perm.empty()) {
-      const int64_t* rp = (A->isComplex ? A->c.rowptr : A->r.rowptr) + r0;
+      const int64_t* rp = (A->isComplex ? A->c.rowptr : A->r.rowptr) + (r1 > r0 ? s0 : 0);
       const int32_t* col = A->isComplex ? A->c.col : A->r.col;
       const void* val = A->isComplex ? static_cast<const void*>(A->c.val) : static_cast<const void*>(A->r.val);
       return mxg::crsCreateFromDevice(row_map, domain_map, rp, col, val, c0, int64_t(colG.size()), colG.data(), A->isComplex, layout, out);
@@ -169,12 +188,13 @@ int mxg_crs_create_from_dcsr(mxg_map* row_map, mxg_map* domain_map, const mxg_dc
     // maps the device front end does not take: the rows pass through the host CSR entry point
     const int64_t n = r1 - r0;
     std::vector<int64_t> rowptr(static_cast<size_t>(n) + 1, 0);
-    int rc = mxg_dcsr_download(a, r0, r1, rowptr.data(), nullptr, nullptr);
+    const int64_t d0 = r1 > r0 ? s0 : 0;
+    int rc = mxg_dcsr_download(a, d0, d0 + n, rowptr.data(), nullptr, nullptr);
     if (rc) return rc;
     const int64_t cnt = rowptr[size_t(n)];
     std::vector<int32_t> col(static_cast<size_t>(std::max<int64_t>(cnt, 1)), 0);
     std::vector<double> val(static_cast<size_t>(std::max<int64_t>(cnt, 1)) * (A->isComplex ? 2 : 1), 0.0);
-    rc = mxg_dcsr_download(a, r0, r1, rowptr.data(), col.data(), val.data());
+    rc = mxg_dcsr_download(a, d0, d0 + n, rowptr.data(), col.data(), val.data());
     if (rc) return rc;
     std::vector<int64_t> gcol(static_cast<size_t>(std::max<int64_t>(cnt, 1)), 0);
     for (int64_t q = 0; q < cnt; ++q) gcol[size_t(q)] = colG[size_t(col[size_t(q)])];
@@ -202,6 +222,17 @@ int mxg_sim_make_map(mxg_sim* sim, const char* field, int64_t begin, int64_t end
   } catch (const std::exception& e) {
     MXG_REQUIRE(false, "mxg_sim_make_map: %s", e.what());
   }
+}
+
+// Device bytes the assembly executors of a context hold now (out[0]) and at most since the last reset (out[1]):
+// simulations (fractions, maps), matrices and the temporaries of the passes. reset_peak != 0 restarts the peak at the
+// current value.
+int mxg_asm_memory(mxg_ctx* ctx, int64_t out[2], int reset_peak) {
+  MXG_REQUIRE(ctx && out, "mxg_asm_memory: NULL argument");
+  if (reset_peak) ctx->asmPeak = ctx->asmBytes;
+  out[0] = ctx->asmBytes;
+  out[1] = ctx->asmPeak;
+  return 0;
 }
 
 }  // extern "C"

@@ -106,6 +106,7 @@ struct mxg_ctx {
   int* dErr = nullptr;
   long long haloTimeoutTicks = 0;      // device clock ticks a halo wait may spin (MXG_HALO_TIMEOUT_S; 0 = for ever)
   uint64_t randomEpoch = 0;            // advanced by mxg_ctx_random_epoch: successive MvRandom calls draw new numbers
+  int64_t asmBytes = 0, asmPeak = 0;   // device bytes held by the operator-assembly executors (mxg_asm_memory)
 };
 
 struct mxg_map {

@@ -362,22 +362,43 @@ struct GenRow {
 };
 
 // ---- CRS row algebra --------------------------------------------------------------------------------------------
+// The rows a CRS matrix stores: at most two runs of positions in its row field's map, stored one after the other
+// (a whole-map matrix: one run from 0). Two runs arise on periodic-x grids, where a slab's stencils reach the planes on
+// the far side of the wrap.
+struct RowRuns {
+  int64_t begin[2], count[2];
+  MXY_HD int64_t size() const { return count[0] + count[1]; }
+  MXY_HD int64_t pos(int64_t i) const { return i < count[0] ? begin[0] + i : begin[1] + (i - count[0]); }   // stored -> map
+  MXY_HD int64_t find(int64_t k) const {                                                                   // map -> stored, -1
+    if (k >= begin[0] && k - begin[0] < count[0]) return k - begin[0];
+    if (k >= begin[1] && k - begin[1] < count[1]) return count[0] + (k - begin[1]);
+    return -1;
+  }
+};
+MXY_HD RowRuns oneRun(int64_t begin, int64_t count) { return {{begin, 0}, {count, 0}}; }
+
 template <class S>
 struct CsrView {
   int64_t nrows, ncols;
   const int64_t* rowptr;
   const int32_t* col;
   const S* val;
+  RowRuns runs;             // which map positions the stored rows are
 };
 
+constexpr int kErrStencil = 1, kErrDomain = 2, kErrNotStored = 3;   // codes of Sim::err
+
 // Upper bound of the row length of A * B (before merging): the table size the product kernel is instantiated with.
+// B is read through its stored runs; a column of A that B does not store sets kErrNotStored.
 template <class S>
 struct ProductBound {
   CsrView<S> A, B;
+  int* err;
   MXY_HD int operator()(int64_t i) const {
     int64_t n = 0;
     for (int64_t p = A.rowptr[i]; p < A.rowptr[i + 1]; ++p) {
-      const int32_t k = A.col[p];
+      const int64_t k = B.runs.find(A.col[p]);
+      if (k < 0) { *err = kErrNotStored; continue; }
       n += B.rowptr[k + 1] - B.rowptr[k];
     }
     return n > 0x7fffffff ? 0x7fffffff : int(n);
@@ -390,10 +411,12 @@ template <class S, int MAXC>
 struct ProductRow {
   static constexpr int kMax = MAXC;
   CsrView<S> A, B;
+  int* err;
   MXY_HD int operator()(int64_t i, int32_t* cols, S* vals) const {
     int n = 0;
     for (int64_t p = A.rowptr[i]; p < A.rowptr[i + 1]; ++p) {
-      const int32_t k = A.col[p];
+      const int64_t k = B.runs.find(A.col[p]);
+      if (k < 0) { *err = kErrNotStored; continue; }
       const S a = A.val[p];
       for (int64_t q = B.rowptr[k]; q < B.rowptr[k + 1]; ++q) {
         const int32_t j = B.col[q];
@@ -450,6 +473,84 @@ struct PurgeRow {
     for (int64_t p = A.rowptr[i]; p < A.rowptr[i + 1]; ++p)
       if (survivesPurge(A.val[p]) && n < MAXC) { cols[n] = A.col[p]; vals[n] = A.val[p]; ++n; }
     return n;
+  }
+};
+
+// A row generator evaluated on the stored rows `runs` of its map: stored row i is map row runs.pos(i).
+template <class Fn>
+struct AtRows {
+  static constexpr int kMax = Fn::kMax;
+  Fn fn;
+  RowRuns runs;
+  template <class S>
+  MXY_HD int operator()(int64_t i, int32_t* cols, S* vals) const { return fn(runs.pos(i), cols, vals); }
+};
+
+// Which x-planes of the column field the map rows `over` of A reference: flag[plane] = 1 (GIDs are x-major, so a plane
+// is one run of the column field's map). `over` must be stored in A.
+template <class S>
+struct PlaneFlags {
+  CsrView<S> A;
+  RowRuns over;
+  const int64_t* colGids;   // column field map
+  int64_t planeGids;        // GIDs per x-plane: ncomp (N1 + 1) (N2 + 1)
+  int32_t* flag;
+  MXY_HD void operator()(int64_t i) const {
+    const int64_t s = A.runs.find(over.pos(i));
+    for (int64_t p = A.rowptr[s]; p < A.rowptr[s + 1]; ++p) flag[colGids[A.col[p]] / planeGids] = 1;
+  }
+};
+
+// How many entries of stored row i of A have a column that B does not store (checked before a product reads B).
+template <class S>
+struct MissingCols {
+  CsrView<S> A;
+  RowRuns bRuns;
+  MXY_HD int operator()(int64_t i) const {
+    int n = 0;
+    for (int64_t p = A.rowptr[i]; p < A.rowptr[i + 1]; ++p) n += bRuns.find(A.col[p]) < 0 ? 1 : 0;
+    return n;
+  }
+};
+
+// Copy of the map rows `over` of A (which stores them): row lengths, then entries.
+template <class S>
+struct SelectCount {
+  CsrView<S> A;
+  RowRuns over;
+  int32_t* count;
+  MXY_HD void operator()(int64_t i) const {
+    const int64_t s = A.runs.find(over.pos(i));
+    count[i] = int32_t(A.rowptr[s + 1] - A.rowptr[s]);
+  }
+};
+template <class S>
+struct SelectFill {
+  CsrView<S> A;
+  RowRuns over;
+  const int64_t* rowptr;
+  int32_t* col;
+  S* val;
+  MXY_HD void operator()(int64_t i) const {
+    const int64_t s = A.runs.find(over.pos(i));
+    int64_t o = rowptr[i];
+    for (int64_t p = A.rowptr[s]; p < A.rowptr[s + 1]; ++p, ++o) { col[o] = A.col[p]; val[o] = A.val[p]; }
+  }
+};
+
+// First map position of every x-plane: out[p] = lower bound of p * planeGids in the ascending map (p = 0 .. N0 + 1).
+struct PlaneStart {
+  const int64_t* gids;
+  int64_t n, planeGids;
+  int64_t* out;
+  MXY_HD void operator()(int64_t p) const {
+    const int64_t key = p * planeGids;
+    int64_t lo = 0, hi = n;
+    while (lo < hi) {
+      const int64_t mid = lo + (hi - lo) / 2;
+      if (gids[mid] < key) lo = mid + 1; else hi = mid;
+    }
+    out[p] = lo;
   }
 };
 
@@ -550,15 +651,21 @@ struct InterpRow {
 };
 
 // (conjugate) transpose in three passes: column counts, scattered fill, then every row sorted by column so that the
-// result does not depend on the order in which threads claimed their slots
+// result does not depend on the order in which threads claimed their slots. Only the columns of the window [c0, c1)
+// become rows (row j - c0); the columns of the result are A's map rows (A.runs.pos of the stored row).
 struct TransposeCount {
   const int32_t* col;
+  int32_t c0, c1;
   int32_t* count;
-  MXY_HD void operator()(int64_t q) const { fetchInc(count + col[q]); }
+  MXY_HD void operator()(int64_t q) const {
+    const int32_t j = col[q];
+    if (j >= c0 && j < c1) fetchInc(count + (j - c0));
+  }
 };
 template <class S>
 struct TransposeFill {
   CsrView<S> A;
+  int32_t c0, c1;
   const int64_t* tptr;
   int32_t* fill;
   int32_t* tcol;
@@ -566,10 +673,23 @@ struct TransposeFill {
   MXY_HD void operator()(int64_t i) const {
     for (int64_t p = A.rowptr[i]; p < A.rowptr[i + 1]; ++p) {
       const int32_t j = A.col[p];
-      const int64_t pos = tptr[j] + fetchInc(fill + j);
-      tcol[pos] = int32_t(i);
+      if (j < c0 || j >= c1) continue;
+      const int64_t pos = tptr[j - c0] + fetchInc(fill + (j - c0));
+      tcol[pos] = int32_t(A.runs.pos(i));
       tval[pos] = conjS(A.val[p]);
     }
+  }
+};
+// entries of stored row first + i of A whose column lies in [c0, c1)
+template <class S>
+struct WindowHits {
+  CsrView<S> A;
+  int64_t first;
+  int32_t c0, c1;
+  MXY_HD int operator()(int64_t i) const {
+    int n = 0;
+    for (int64_t p = A.rowptr[first + i]; p < A.rowptr[first + i + 1]; ++p) n += (A.col[p] >= c0 && A.col[p] < c1) ? 1 : 0;
+    return n;
   }
 };
 template <class S>
