@@ -15,6 +15,7 @@ import torch.distributed as dist  # noqa: E402
 import maxwell_b200 as mx  # noqa: E402
 from maxwell_b200.partition import local_block, slab_cuts  # noqa: E402
 from oracle import oracle as orc  # noqa: E402
+import gmg_reference  # noqa: E402
 
 
 def _assert_matches_global(got, ref, is_complex, what):
@@ -67,18 +68,36 @@ def solve_case(ctx, rank, world):
     cuts = B[0][2]
     md = mx.MxMultiVector(B[0][3], 1)
     md.from_host(fa[cuts[rank]:cuts[rank + 1]])
+
+    def matches_reference(prec, parts, name, field, b, what, **kw):
+        """This rank's slab of M^-1 b equals the matching rows of the float64 reference cycle on the global operators (run with
+        the all-reduced lambda_max of the GPU, which is the restated power iteration's to rounding) to 1e-12 per column."""
+        ops, R, P, gids = gmg_reference.oracle_hierarchy(orc, sims, name, field)
+        lam = [prec.info(l)["lambda_max"] for l in range(len(sims))]
+        ref = gmg_reference.from_oracle(ops, R, P, gids, lambda_max=lam, **kw)
+        for l in range(len(sims)):
+            want = gmg_reference.power_lambda_max(ref.A[l], ref.dinv[l], gids[l], l)
+            assert abs(lam[l] - want) <= 1e-12 * want, what + ("lambda_max", l, lam[l], want)
+        c0, c1 = parts[0][2][rank], parts[0][2][rank + 1]
+        bs = mx.MxMultiVector(parts[0][3], b.shape[1])
+        bs.from_host(b[c0:c1])
+        xs = bs.Clone(b.shape[1])
+        prec.ApplyInverse(bs, xs)
+        err = gmg_reference.column_errors(xs.to_host(), ref.apply(b)[c0:c1])
+        assert np.all(err < 1e-12), what + (err,)
+        return bs, xs
+
     for fmg in (True, False):
         prec = mx.MxGeoMultigridPrec(ctx, vops, Rb, Pb, smoother_sweeps=2, full_multigrid=fmg)
-        b = mx.MxMultiVector(B[0][3], 2)
-        b.random(21)
-        b.zero_unused(md)
-        x = b.Clone(2)
-        prec.ApplyInverse(b, x)
+        bg = gmg_reference.random_columns(21, B[0][0], 2, False) * (fa > 0)[:, None]
+        b, x = matches_reference(prec, B, "vecLapl", "bfield", bg, ("multigrid on %d ranks" % world, fmg), full_multigrid=fmg)
         r = b.CloneCopy()
         vops[0].apply_axpby(-1.0, x, 1.0, r)
         red = (r.norm2() / b.norm2()).max()
         assert red < 0.8, ("multigrid on %d ranks" % world, fmg, red)
     sprec = mx.MxGeoMultigridPrec(ctx, sops, Rp, Pp, smoother_sweeps=2, remove_const_field=True)
+    bg = gmg_reference.random_columns(23, Ps[0][0], 2, False)
+    matches_reference(sprec, Ps, "scaLapl", "psifield", bg, ("scalar multigrid on %d ranks" % world,), remove_const_field=True)
     nev = 6
     s = mx.MxSolver(ctx, vops[0], m_diag=md, prec=prec, nev=nev, block_size=10, tol=1e-9, max_iters=300,
                     projection={"divB": D, "gradPsi": G, "scaLapl": sops[0], "sca_prec": sprec})
