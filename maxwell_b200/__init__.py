@@ -325,19 +325,26 @@ class MxMultiVector:
     def getLocalLength(self):
         return self._L.mxg_mv_local_length(self.h)
 
-    def MvTimesMatAddMv(self, alpha, A, B, beta):
-        """this = alpha*A*B + beta*this; B: host (k x b) array."""
-        Bh = np.asfortranarray(np.asarray(B, dtype=self.dtype).reshape(A.GetNumberVecs(), -1))
+    def MvTimesMatAddMv(self, alpha, A, B, beta, ldb=None):
+        """this = alpha*A*B + beta*this; B: host (k x b) array, or with ldb an (ldb x b) array of which the first k rows
+        are read."""
+        k = A.GetNumberVecs()
+        Bh = np.asfortranarray(np.asarray(B, dtype=self.dtype).reshape(k if ldb is None else int(ldb), -1))
         _ck(self._L.mxg_mv_times_mat_add_mv(_scalar(alpha), A.h, Bh.ctypes.data, Bh.shape[0], _scalar(beta), self.h))
 
     def MvAddMv(self, alpha, A, beta, B):
         _ck(self._L.mxg_mv_add_mv(self.h, _scalar(alpha), A.h, _scalar(beta), B.h))
 
-    def MvTransMv(self, alpha, A):
-        """returns alpha * A^H * this as a host (k x b) array."""
+    def MvTransMv(self, alpha, A, ldb=None, out=None):
+        """returns alpha * A^H * this as a host (k x b) array. With ldb, the product fills the first k rows of an (ldb x b)
+        column-major array (`out`, whose other rows are left as they are, or a new zero array), which is returned."""
         k, b = A.GetNumberVecs(), self.GetNumberVecs()
-        out = np.zeros((k, b), dtype=self.dtype, order="F")
-        _ck(self._L.mxg_mv_trans_mv(_scalar(alpha), A.h, self.h, out.ctypes.data, k))
+        ldb = k if ldb is None else int(ldb)
+        if out is None:
+            out = np.zeros((ldb, b), dtype=self.dtype, order="F")
+        if out.shape != (ldb, b) or out.dtype != self.dtype or not out.flags.f_contiguous:
+            raise MxError("MvTransMv: out must be a column-major %d x %d %s array" % (ldb, b, np.dtype(self.dtype).name))
+        _ck(self._L.mxg_mv_trans_mv(_scalar(alpha), A.h, self.h, out.ctypes.data, ldb))
         return out
 
     def trans_mv(self, alpha, X):

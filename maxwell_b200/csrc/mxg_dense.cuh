@@ -1,16 +1,13 @@
 // Tall-skinny dense block products of the eigensolver (real FP64): the Gram product C = A^T X (MvTransMv,
 // src/MxAnasaziMV.cpp:114-149) and the update Y = alpha A B + beta Y (MvTimesMatAddMv, :8-33).
 //
-// ncu on the round-1 kernels (profiles/README_r02.md): k_gram_tiled moved every byte once but sat at 82 % of the
-// shared-memory wavefront limit with the FP64 pipe at 35 % (6 eight-byte shared loads per 9 FMAs), k_times_mat re-read A
-// once per 16 output columns and ran at 25 % occupancy on a register tile. Both kernels here stream A (and X) exactly
-// once through shared memory with 1-D TMA copies (one cp.async.bulk per column segment, double buffered behind
-// mbarriers) and feed the FP64 pipe from 16-byte shared loads laid out so that every warp-wide load is ONE wavefront:
-//   Gram  : 2 rows per load, thread tile RI x RJ  ->  (RI + RJ) wavefronts per 2 RI RJ FMAs
-//   update: 4 rows per thread x RC columns        ->  (2 + RC) wavefronts per 4 RC FMAs
-// so the kernels are bound by the FP64 pipe / HBM, not by the load pipe. tcgen05 has no FP64 kind and the DMMA path has
-// the same peak as the FMA pipe on B200, so the contraction stays on FMAs (north_star: tensor cores only if compute-bound
-// AND faster; neither holds here).
+// Both kernels stream A (and X) exactly once through shared memory: the rows are cut into chunks of kDenseRows, one 1-D TMA
+// copy (cp.async.bulk) per column segment fills a stage, two stages alternate behind mbarriers, and each CTA walks the
+// chunks ch = blockIdx, blockIdx + gridDim, ... The contraction runs on the FP64 tensor path (mma.sync.m8n8k4.f64, DMMA):
+// tcgen05 has no FP64 kind, and one 8-byte shared load per lane feeds 8 FMAs per lane, where the FMA-pipe kernels of
+// round 2 sat at 95 % of the shared-memory wavefront limit and were 1.3-2.0x slower on every timed shape
+// (profiles/README_r02.md section 2). The complex products and updates with more than kUpdateMaxK source columns run on the
+// register-tiled kernels of mxg_mvops.cu.
 #pragma once
 #include "mxg_internal.h"
 #include "mxg_spmm_win.cuh"
@@ -30,182 +27,8 @@ __device__ __forceinline__ void denseIssue(const double* col, int64_t r0, int ro
   bulkLoad(dst, col + r0, bytes, bar);
 }
 
-// ---- Gram: partial[(k0+ci) + (b0+cj) k][slice] = sum over this slice's rows of A_ci X_cj ---------------------------------
-// Block tile (16 RI) x (16 RJ); thread (ty, tx) owns A columns ty + 16 i and X columns tx + 16 j. A warp spans 4 ty x 8 tx.
-template <int RI, int RJ>
-__global__ void __launch_bounds__(kDenseThreads, 2) k_gram_tma(ColTable<double> A, int k, ColTable<double> X, int b, int64_t n, int tilesB,
-                                                               double* __restrict__ partial) {
-  constexpr int TI = 16 * RI, TJ = 16 * RJ, NC = TI + TJ;
-  extern __shared__ __align__(128) unsigned char smemRaw[];
-  uint64_t* bar = reinterpret_cast<uint64_t*>(smemRaw);                 // one per stage
-  double* stage0 = reinterpret_cast<double*>(smemRaw + 128);
-  constexpr int stageElems = NC * kDenseStride;
-  const int tk = blockIdx.x / tilesB, tb = blockIdx.x % tilesB;
-  const int k0 = tk * TI, b0 = tb * TJ;
-  const int kc = min(TI, k - k0), bc = min(TJ, b - b0);
-  const int nIssue = kc + bc;
-  const int t = threadIdx.x;
-  if (t == 0) {
-    mbarInit(&bar[0], nIssue);
-    mbarInit(&bar[1], nIssue);
-    mbarFenceInit();
-  }
-  __syncthreads();
-  const int64_t chunks = (n + kDenseRows - 1) / kDenseRows;
-  // column this thread feeds (A columns first, then X columns); column slots of unused tile columns stay untouched
-  const double* myCol = nullptr;
-  int mySlot = 0;
-  if (t < kc) { myCol = A.p[k0 + t]; mySlot = t; }
-  else if (t < nIssue) { myCol = X.p[b0 + (t - kc)]; mySlot = TI + (t - kc); }
-  auto issue = [&](int64_t ch, int s) {
-    if (myCol) {
-      const int64_t r0 = ch * kDenseRows;
-      const int rows = int(min(int64_t(kDenseRows), n - r0));
-      denseIssue(myCol, r0, rows, stage0 + s * stageElems + mySlot * kDenseStride, &bar[s]);
-    }
-  };
-  const int warp = t >> 5, lane = t & 31;
-  const int ty = (warp >> 1) * 4 + (lane >> 3), tx = (warp & 1) * 8 + (lane & 7);
-  double acc[RI][RJ];
-#pragma unroll
-  for (int i = 0; i < RI; ++i)
-#pragma unroll
-    for (int j = 0; j < RJ; ++j) acc[i][j] = 0.0;
-  int64_t ch = blockIdx.y;
-  if (ch < chunks) issue(ch, 0);
-  int it = 0;
-  for (; ch < chunks; ch += gridDim.y, ++it) {
-    const int s = it & 1;
-    const int64_t next = ch + gridDim.y;
-    if (next < chunks) issue(next, s ^ 1);                  // the other stage was released by the barrier below
-    mbarWait(&bar[s], (it >> 1) & 1);
-    double* sA = stage0 + s * stageElems;
-    const int64_t r0 = ch * kDenseRows;
-    if (n - r0 < kDenseRows) {                              // tail chunk: rows past the end contribute zero
-      const int valid = int(n - r0);
-      for (int e = t; e < NC * kDenseRows; e += kDenseThreads) {
-        const int c = e / kDenseRows, r = e % kDenseRows;
-        if (r >= valid) sA[c * kDenseStride + r] = 0.0;
-      }
-      __syncthreads();
-    }
-    const double* sX = sA + TI * kDenseStride;
-#pragma unroll 4
-    for (int rr = 0; rr < kDenseRows; rr += 2) {
-      double2 av[RI], xv[RJ];
-#pragma unroll
-      for (int i = 0; i < RI; ++i) av[i] = *reinterpret_cast<const double2*>(sA + (ty + 16 * i) * kDenseStride + rr);
-#pragma unroll
-      for (int j = 0; j < RJ; ++j) xv[j] = *reinterpret_cast<const double2*>(sX + (tx + 16 * j) * kDenseStride + rr);
-#pragma unroll
-      for (int i = 0; i < RI; ++i)
-#pragma unroll
-        for (int j = 0; j < RJ; ++j) {
-          acc[i][j] = fma(av[i].x, xv[j].x, acc[i][j]);
-          acc[i][j] = fma(av[i].y, xv[j].y, acc[i][j]);
-        }
-    }
-    __syncthreads();                                        // stage s may be refilled
-  }
-#pragma unroll
-  for (int i = 0; i < RI; ++i)
-#pragma unroll
-    for (int j = 0; j < RJ; ++j) {
-      const int ci = ty + 16 * i, cj = tx + 16 * j;
-      if (ci < kc && cj < bc) partial[(int64_t(k0 + ci) + int64_t(b0 + cj) * k) * gridDim.y + blockIdx.y] = acc[i][j];
-    }
-}
-
-// ---- update: Y(:, 0:b) = alpha A(:, 0:k) B + beta Y; B (k x b, column-major, ld k) in global memory ----------------------
-// A chunk is complete in shared memory before any of its rows is written, and different chunks are different rows, so Y
-// may share columns with A (in-place right-multiplication of a basis block).
-template <int RC>
-__global__ void __launch_bounds__(kDenseThreads, 2) k_update_tma(ColTable<double> A, int k, const double* __restrict__ Bg, int b, double alpha,
-                                                                 double beta, ColTable<double> Y, int64_t n) {
-  extern __shared__ __align__(128) unsigned char smemRaw[];
-  uint64_t* bar = reinterpret_cast<uint64_t*>(smemRaw);
-  double* sB = reinterpret_cast<double*>(smemRaw + 128);        // [k][16 RC], row i = coefficients of A column i
-  constexpr int BW = 16 * RC;
-  double* stage0 = sB + ((k * BW + 15) & ~15);
-  const int stageElems = k * kDenseStride;
-  const int t = threadIdx.x;
-  if (t == 0) {
-    mbarInit(&bar[0], k);
-    mbarInit(&bar[1], k);
-    mbarFenceInit();
-  }
-  for (int e = t; e < k * BW; e += kDenseThreads) {
-    const int i = e / BW, j = e % BW;
-    sB[e] = j < b ? Bg[i + int64_t(j) * k] : 0.0;
-  }
-  __syncthreads();
-  const int64_t chunks = (n + kDenseRows - 1) / kDenseRows;
-  auto issue = [&](int64_t ch, int s) {
-    for (int c = t; c < k; c += kDenseThreads) {
-      const int64_t r0 = ch * kDenseRows;
-      const int rows = int(min(int64_t(kDenseRows), n - r0));
-      denseIssue(A.p[c], r0, rows, stage0 + s * stageElems + c * kDenseStride, &bar[s]);
-    }
-  };
-  const int warp = t >> 5, lane = t & 31;
-  // rows 2 rg, 2 rg + 1, 32 + 2 rg, 33 + 2 rg of the chunk (the 8 row groups of a warp read 128 contiguous bytes per load)
-  const int rg = (warp & 1) * 8 + (lane & 7);
-  const int cg = (warp >> 1) * 4 + (lane >> 3);    // column group: columns cg + 16 j
-  int64_t ch = blockIdx.x;
-  if (ch < chunks) issue(ch, 0);
-  int it = 0;
-  for (; ch < chunks; ch += gridDim.x, ++it) {
-    const int s = it & 1;
-    const int64_t next = ch + gridDim.x;
-    if (next < chunks) issue(next, s ^ 1);
-    mbarWait(&bar[s], (it >> 1) & 1);
-    const double* sA = stage0 + s * stageElems + 2 * rg;
-    double acc[4][RC];
-#pragma unroll
-    for (int r = 0; r < 4; ++r)
-#pragma unroll
-      for (int j = 0; j < RC; ++j) acc[r][j] = 0.0;
-#pragma unroll 4
-    for (int i = 0; i < k; ++i) {
-      const double2 a01 = *reinterpret_cast<const double2*>(sA + i * kDenseStride);
-      const double2 a23 = *reinterpret_cast<const double2*>(sA + i * kDenseStride + 32);
-#pragma unroll
-      for (int j = 0; j < RC; ++j) {
-        const double bv = sB[i * BW + cg + 16 * j];
-        acc[0][j] = fma(a01.x, bv, acc[0][j]);
-        acc[1][j] = fma(a01.y, bv, acc[1][j]);
-        acc[2][j] = fma(a23.x, bv, acc[2][j]);
-        acc[3][j] = fma(a23.y, bv, acc[3][j]);
-      }
-    }
-    const int64_t r0 = ch * kDenseRows + 2 * rg;
-#pragma unroll
-    for (int j = 0; j < RC; ++j) {
-      const int c = cg + 16 * j;
-      if (c < b) {
-        double* y = Y.p[c];
-#pragma unroll
-        for (int r = 0; r < 4; ++r) {
-          const int64_t row = r0 + (r >> 1) * 32 + (r & 1);
-          if (row < n) {
-            double v = alpha * acc[r][j];
-            if (beta != 0.0) v += beta * y[row];
-            y[row] = v;
-          }
-        }
-      }
-    }
-    __syncthreads();
-  }
-}
-// ---- FP64 tensor-core variants (mma.sync.m8n8k4.f64) -----------------------------------------------------------------------
-// ncu on the FMA kernels above (profiles/README_r02.md): 95 % of the shared-memory wavefront limit, FP64 pipe at 29-48 % --
-// an FMA consumes two 8-byte operands and a (RI x RJ) register tile amortises them only (RI RJ)/(RI + RJ) times, while the
-// shared-memory pipe delivers 128 B/clk against 64 FMA/clk. A DMMA fragment is shared by the whole warp: one 8-byte shared
-// load per lane feeds 8 FMAs per lane, so the operand traffic drops 4x and the contraction becomes FP64-pipe / HBM bound.
-// This is the "only if ncu shows them compute-(pipe-)bound" case of north_star; tcgen05 has no FP64 kind, DMMA is the FP64
-// tensor path on sm_100a. Fragment layout (PTX ISA, m8n8k4): a0 = A[g][t], b0 = B[t][g], c0/c1 = C[g][2t], C[g][2t+1] with
-// g = lane / 4, t = lane % 4.
+// ---- FP64 tensor-core contraction (mma.sync.m8n8k4.f64) --------------------------------------------------------------------
+// Fragment layout (PTX ISA, m8n8k4): a0 = A[g][t], b0 = B[t][g], c0/c1 = C[g][2t], C[g][2t+1] with g = lane / 4, t = lane % 4.
 __device__ __forceinline__ void dmma884(double& c0, double& c1, double a, double b) {
   asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};" : "+d"(c0), "+d"(c1) : "d"(a), "d"(b));
 }

@@ -1,7 +1,6 @@
 // libmxgpu: multivector block operations (K5-K14 of SURVEY.md section 2.3). All kernels are
 // HBM-bound streaming or reduction kernels; grids are sized in multiples of the SM count.
 #include <cmath>
-#include <cstdlib>
 #include <cstring>
 
 #include "mxg_internal.h"
@@ -217,79 +216,9 @@ __global__ void __launch_bounds__(kBlock) k_trans_mv(ColTable<T> A, int k, ColTa
     }
 }
 
-// Real-valued Gram product with shared-memory staging: one block owns a 64 x 64 tile of C and
-// streams rows in chunks of kGramRows. Each chunk of the (up to) 64 A-columns and 64 X-columns is
-// loaded ONCE from global memory (coalesced, one column per warp-load) into shared memory and then
-// reused by all 256 threads, each of which keeps a 4 x 4 register tile of C. Column ownership is
-// interleaved (thread (ty, tx) owns A-columns ty + 16 i and X-columns tx + 16 j) and the shared
-// column stride is odd in 8-byte words, so every shared load is conflict-free or a broadcast.
-constexpr int kGramRows = 32;
-constexpr int kGramStride = kGramRows + 1;
-// RI x RJ = per-thread register tile; the block tile of C is (16 RI) x (16 RJ)
-template <int RI, int RJ>
-__global__ void __launch_bounds__(kBlock, 2) k_gram_tiled(ColTable<double> A, int k, ColTable<double> X, int b, int64_t n,
-                                                          int tilesB, double* __restrict__ partial /* [k*b][gridDim.y] */) {
-  constexpr int TI = 16 * RI, TJ = 16 * RJ;
-  __shared__ double sA[TI * kGramStride];
-  __shared__ double sX[TJ * kGramStride];
-  const int tk = blockIdx.x / tilesB, tb = blockIdx.x % tilesB;
-  const int k0 = tk * TI, b0 = tb * TJ;
-  const int kc = min(TI, k - k0), bc = min(TJ, b - b0);
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int ty = threadIdx.x >> 4, tx = threadIdx.x & 15;
-  double acc[RI][RJ];
-#pragma unroll
-  for (int i = 0; i < RI; ++i)
-#pragma unroll
-    for (int j = 0; j < RJ; ++j) acc[i][j] = 0.0;
-  const int64_t chunks = (n + kGramRows - 1) / kGramRows;
-  for (int64_t ch = blockIdx.y; ch < chunks; ch += gridDim.y) {
-    const int64_t r = ch * kGramRows + lane;
-    const bool ok = r < n;
-    // warp w stages columns w, w+8, ... of both operands; lane = row inside the chunk
-#pragma unroll
-    for (int c = 0; c < TI / 8; ++c) {
-      const int col = warp + 8 * c;
-      sA[col * kGramStride + lane] = (ok && col < kc) ? A.p[k0 + col][r] : 0.0;
-    }
-#pragma unroll
-    for (int c = 0; c < TJ / 8; ++c) {
-      const int col = warp + 8 * c;
-      sX[col * kGramStride + lane] = (ok && col < bc) ? X.p[b0 + col][r] : 0.0;
-    }
-    __syncthreads();
-#pragma unroll 8
-    for (int rr = 0; rr < kGramRows; ++rr) {
-      double av[RI], xv[RJ];
-#pragma unroll
-      for (int i = 0; i < RI; ++i) av[i] = sA[(ty + 16 * i) * kGramStride + rr];
-#pragma unroll
-      for (int j = 0; j < RJ; ++j) xv[j] = sX[(tx + 16 * j) * kGramStride + rr];
-#pragma unroll
-      for (int i = 0; i < RI; ++i)
-#pragma unroll
-        for (int j = 0; j < RJ; ++j) acc[i][j] = fma(av[i], xv[j], acc[i][j]);
-    }
-    __syncthreads();
-  }
-#pragma unroll
-  for (int i = 0; i < RI; ++i)
-#pragma unroll
-    for (int j = 0; j < RJ; ++j) {
-      const int ci = ty + 16 * i, cj = tx + 16 * j;
-      if (ci < kc && cj < bc) partial[(int64_t(k0 + ci) + int64_t(b0 + cj) * k) * gridDim.y + blockIdx.y] = acc[i][j];
-    }
-}
-
 // ---- tall-skinny update: Y = alpha * A * B + beta * Y ---------------------------------------
 // The small dense B rides in the kernel parameter block (constant bank): the FMAs take it as a
 // uniform operand, so the only memory instructions are the streaming loads of A and Y.
-// FP64 tensor-core (DMMA) variants of the Gram / update kernels unless MXG_DENSE=fma (mxg_dense.cuh)
-inline bool denseUseMma() {
-  static int v = -1;
-  if (v < 0) { const char* e = std::getenv("MXG_DENSE"); v = (e && std::strcmp(e, "fma") == 0) ? 0 : 1; }
-  return v == 1;
-}
 constexpr int kUpdateMaxK = 64;   // widest A the TMA-staged update kernel takes (shared memory: 2 stages of k columns + B)
 constexpr int kMaxBParam = 1536;  // doubles (12 KB of the 32 KB parameter space)
 struct DenseParam {
@@ -453,8 +382,8 @@ int transMvImpl(const double alpha[2], const mxg_mv* A, const mxg_mv* X, double*
   if (slices > maxSlices) slices = maxSlices;
   if (slices < 1) slices = 1;
   const size_t kb = size_t(k) * b;
-  // shared-memory tiled kernel (real case): the block tile of C is (16 ri) x (16 rj) with ri, rj in 1..4
-  // chosen to cover k and b with as little padding as possible
+  // TMA-staged DMMA kernel (real case): the block tile of C is (16 ri) x (16 rj) with ri, rj in 1..3, chosen to cover k and b
+  // with as little padding as possible
   const int ri = k >= 33 ? 3 : (k + 15) / 16, rj = b >= 33 ? 3 : (b + 15) / 16;   // block tile (16 ri) x (16 rj), at most 48 x 48
   const int gtB = (b + 16 * rj - 1) / (16 * rj), gtiles = ((k + 16 * ri - 1) / (16 * ri)) * gtB;
   int gs = (ctx->numSMs * 2 + gtiles - 1) / gtiles;
@@ -463,8 +392,7 @@ int transMvImpl(const double alpha[2], const mxg_mv* A, const mxg_mv* X, double*
     if (gs > chunks) gs = int(chunks);
     if (gs < 1) gs = 1;
   }
-  const bool useMma = denseUseMma();
-  if (w == 1) slices = useMma ? 2 * gs : gs;   // the DMMA kernel writes its two row halves as separate slices
+  if (w == 1) slices = 2 * gs;   // the DMMA kernel writes its two row halves as separate slices
   int rc = ensureScratch(ctx, sizeof(T) * (kb * slices + kb));
   if (rc) return rc;
   T* out = reinterpret_cast<T*>(ctx->dScratch);
@@ -478,12 +406,10 @@ int transMvImpl(const double alpha[2], const mxg_mv* A, const mxg_mv* X, double*
   {                                                                                                                   \
     static bool attr = false;                                                                                         \
     if (!attr) {                                                                                                      \
-      MXG_CUDA(cudaFuncSetAttribute(k_gram_tma<RI, RJ>, cudaFuncAttributeMaxDynamicSharedMemorySize, 110 * 1024));     \
       MXG_CUDA(cudaFuncSetAttribute(k_gram_mma<RI, RJ>, cudaFuncAttributeMaxDynamicSharedMemorySize, 110 * 1024));     \
       attr = true;                                                                                                    \
     }                                                                                                                 \
-    if (useMma) k_gram_mma<RI, RJ><<<grid, kDenseThreads, smem, ctx->stream>>>(ta, k, tx, b, A->ld, gtB, part);        \
-    else k_gram_tma<RI, RJ><<<grid, kDenseThreads, smem, ctx->stream>>>(ta, k, tx, b, A->ld, gtB, part);               \
+    k_gram_mma<RI, RJ><<<grid, kDenseThreads, smem, ctx->stream>>>(ta, k, tx, b, A->ld, gtB, part);                    \
   }
     switch (ri * 4 + rj) {
       case 5: MXG_GRAM(1, 1); break;  case 6: MXG_GRAM(1, 2); break;  case 7: MXG_GRAM(1, 3); break;
@@ -529,10 +455,8 @@ int timesMatImpl(const double alpha[2], const mxg_mv* A, const double* B, int ld
         for (int j = 0; j < cc; ++j) std::memcpy(&Bc[size_t(j) * k], B + size_t(c0 + j) * ldb, sizeof(double) * k);
         MXG_CUDA(cudaMemcpyAsync(ctx->dDense, Bc.data(), Bc.size() * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
         const int rc_ = (cc + 15) / 16;
-        const size_t smem = 128 + sizeof(double) * (((size_t(k) * 16 * rc_ + 15) & ~size_t(15)) + size_t(2) * k * kDenseStride);
         const size_t k4 = size_t((k + 3) & ~3);
-        const size_t smemMma = 128 + sizeof(double) * (((k4 * (16 * rc_ + 4) + 15) & ~size_t(15)) + size_t(2) * k4 * kDenseStride);
-        const bool useMma = denseUseMma();
+        const size_t smem = 128 + sizeof(double) * (((k4 * (16 * rc_ + 4) + 15) & ~size_t(15)) + size_t(2) * k4 * kDenseStride);
         const int64_t chunks = (Y->ld + kDenseRows - 1) / kDenseRows;
         const int grid = int(std::min<int64_t>(chunks, int64_t(ctx->numSMs) * 2));
         auto ta = tableOf<double>(A);
@@ -541,12 +465,10 @@ int timesMatImpl(const double alpha[2], const mxg_mv* A, const double* B, int ld
   {                                                                                                                    \
     static bool attr = false;                                                                                          \
     if (!attr) {                                                                                                       \
-      MXG_CUDA(cudaFuncSetAttribute(k_update_tma<RC>, cudaFuncAttributeMaxDynamicSharedMemorySize, 110 * 1024));        \
       MXG_CUDA(cudaFuncSetAttribute(k_update_mma<RC>, cudaFuncAttributeMaxDynamicSharedMemorySize, 110 * 1024));        \
       attr = true;                                                                                                     \
     }                                                                                                                  \
-    if (useMma) k_update_mma<RC><<<grid, kDenseThreads, smemMma, ctx->stream>>>(ta, k, ctx->dDense, cc, al, be, ty, Y->ld); \
-    else k_update_tma<RC><<<grid, kDenseThreads, smem, ctx->stream>>>(ta, k, ctx->dDense, cc, al, be, ty, Y->ld);       \
+    k_update_mma<RC><<<grid, kDenseThreads, smem, ctx->stream>>>(ta, k, ctx->dDense, cc, al, be, ty, Y->ld);            \
   }
         if (rc_ == 1) MXG_UPD(1) else if (rc_ == 2) MXG_UPD(2) else MXG_UPD(3)
 #undef MXG_UPD

@@ -114,6 +114,51 @@ def solve_case(ctx, rank, world):
         print("case multigrid + projected eigensolve ok on %d ranks" % world, flush=True)
 
 
+def dense_case(ctx, rank, world):
+    """Block products and reductions on ragged partitions: one rank owns no rows, or one owns fewer than 64 (a single tail
+    chunk). The data are small integers and the scalars dyadic, so every partial sum is an integer below 2^53: the all-reduced
+    Gram, dot, norm and mean and each rank's rows of the update must equal the global numpy result bit for bit, whatever
+    the rank count."""
+    n = 1 << 16                                       # a power of two: remove_const_field's 1/count is exact
+    rng = np.random.default_rng(64)                   # the same global data on every rank
+    Ag = rng.integers(-8, 9, size=(n, 72)).astype(np.float64)
+    Xg = rng.integers(-8, 9, size=(n, 24)).astype(np.float64)
+    Cg = rng.integers(-8, 9, size=(n, 5)) + 1j * rng.integers(-8, 9, size=(n, 5))
+    B = rng.integers(-4, 5, size=(72, 24)).astype(np.float64)
+    gids = np.arange(n, dtype=np.int64)
+
+    def even(total, parts):
+        return [total // parts + (1 if i < total % parts else 0) for i in range(parts)]
+
+    for label, sizes in (("rank 0 owns no rows", [0] + even(n, world - 1)),
+                         ("the last rank owns 37 rows", even(n - 37, world - 1) + [37])):
+        cuts = np.concatenate([[0], np.cumsum(sizes)])
+        r0, r1 = int(cuts[rank]), int(cuts[rank + 1])
+        m = mx.MxMap(ctx, n, gids[r0:r1])
+        A, X, Cx = mx.MxMultiVector(m, 72), mx.MxMultiVector(m, 24), mx.MxMultiVector(m, 5, True)
+        A.from_host(Ag[r0:r1])
+        X.from_host(Xg[r0:r1])
+        Cx.from_host(Cg[r0:r1])
+        what = (label, world)
+        assert np.array_equal(X.MvTransMv(-0.5, A.CloneView(list(range(40)))), -0.5 * (Ag[:, :40].T @ Xg)), what + ("gram",)
+        assert np.array_equal(X.MvTransMv(2.0, A), 2.0 * (Ag.T @ Xg)), what + ("gram, 72 columns",)
+        assert np.array_equal(Cx.MvTransMv(0.5 - 0.25j, Cx), (0.5 - 0.25j) * (Cg.conj().T @ Cg)), what + ("complex gram",)
+        for k in (40, 72):                            # the TMA-staged update and the parameter-block one
+            Y = mx.MxMultiVector(m, 24)
+            Y.from_host(Xg[r0:r1])
+            Y.MvTimesMatAddMv(0.75, A.CloneView(list(range(k))), B[:k], 2.0)
+            assert np.array_equal(Y.to_host(), 0.75 * (Ag[r0:r1, :k] @ B[:k]) + 2.0 * Xg[r0:r1]), what + ("update", k)
+        A24 = A.CloneView(list(range(24)))
+        assert np.array_equal(X.dot(A24), (Ag[:, :24] * Xg).sum(axis=0)), what + ("dot",)
+        assert np.array_equal(Cx.dot(Cx), (np.abs(Cg.real) ** 2 + np.abs(Cg.imag) ** 2).sum(axis=0).astype(complex)), what
+        assert np.array_equal(X.norm2(), np.sqrt((Xg * Xg).sum(axis=0))), what + ("norm2",)
+        X.remove_const_field()
+        assert np.array_equal(X.to_host(), Xg[r0:r1] - Xg.sum(axis=0) * (1.0 / n)), what + ("remove_const_field",)
+        del A, X, Cx, A24, Y
+    if rank == 0:
+        print("case dense block products on ragged partitions ok on %d ranks" % world, flush=True)
+
+
 def device_assembly_case(ctx, rank, world):
     """Operators assembled on every rank's device (include/mxasm.h), each rank keeping the rows of its slab; the layout is
     built on the device too (ghost discovery, halo plan, dictionary, sliced ELL). Applies must equal the oracle's global
@@ -218,6 +263,7 @@ def main():
             del A
         if rank == 0:
             print("case %s ok on %d ranks" % (label, world), flush=True)
+    dense_case(ctx, rank, world)
     device_assembly_case(ctx, rank, world)
     solve_case(ctx, rank, world)
     dist.barrier()
