@@ -77,14 +77,6 @@ void mxg_host_free(void* p);
  * A map is this rank's list of owned global DOF ids. GIDs must be ascending within a rank
  * and rank r's GIDs must all precede rank r+1's (x-slab partition; see DESIGN.md). */
 int mxg_map_create(mxg_ctx* ctx, int64_t n_global, const int64_t* my_gids, int64_t n_local, mxg_map** out);
-/* Same map with a component-major DEVICE ordering of the multivectors that live on it (component = GID mod ncomp, the
- * reference's globCompIndx = comp + ncomp * cell, MxGridField.hpp:142-145): consecutive device positions are
- * consecutive cells of one field component, which makes the gathers of the curl-curl SpMM contiguous. Single-rank
- * contexts only. mxg_mv_upload / mxg_mv_download / mxg_mv_col_ptr then use device order; mxg_map_get_order returns
- * perm[device position] = reference local index so callers can translate (returns 1 if ordered, 0 if identity).
- * Everything else (block operations, mxg_crs_create, mxg_mv_random, mxg_mv_to_grid) is order-agnostic. */
-int mxg_map_create_ordered(mxg_ctx* ctx, int64_t n_global, const int64_t* my_gids, int64_t n_local, int ncomp, mxg_map** out);
-int mxg_map_get_order(const mxg_map* map, int32_t* perm_out);
 int mxg_map_destroy(mxg_map* map);
 int64_t mxg_map_local_size(const mxg_map* map);    /* getNodeNumIndices   */
 int64_t mxg_map_global_size(const mxg_map* map);   /* getGlobalNumIndices */

@@ -56,8 +56,6 @@ def load_library():
         "mxg_host_free": (None, [vp]),
         "mxg_crs_apply_timed": (i32, [vp, vp, vp, dp]),
         "mxg_map_create": (i32, [vp, i64, vp, i64, pvp]),
-        "mxg_map_create_ordered": (i32, [vp, i64, vp, i64, i32, pvp]),
-        "mxg_map_get_order": (i32, [vp, vp]),
         "mxg_map_destroy": (i32, [vp]),
         "mxg_map_local_size": (i64, [vp]),
         "mxg_map_global_size": (i64, [vp]),
@@ -245,23 +243,12 @@ class Context:
 class MxMap:
     """MxMap(globalIndices, comm) (MxMap.hpp:22-103): this rank's owned GIDs, ascending."""
 
-    def __init__(self, ctx, num_global, my_gids, components=1):
-        """components > 1: multivectors on this map are stored component-major on the device (mxg_map_create_ordered;
-        GID = comp + components * cell). from_host / to_host translate, so callers keep the reference order."""
+    def __init__(self, ctx, num_global, my_gids):
         self.ctx = ctx
         self._L = ctx._L
         g = np.ascontiguousarray(my_gids, dtype=np.int64)
         h = C.c_void_p()
-        self.perm = None
-        if int(components) > 1:
-            _ck(self._L.mxg_map_create_ordered(ctx.h, int(num_global), g.ctypes.data, len(g), int(components), C.byref(h)))
-            perm = np.empty(len(g), dtype=np.int32)
-            rc = self._L.mxg_map_get_order(h, perm.ctypes.data)
-            _ck(min(rc, 0))
-            if rc == 1:
-                self.perm = perm.astype(np.int64)          # perm[device position] = reference local index
-        else:
-            _ck(self._L.mxg_map_create(ctx.h, int(num_global), g.ctypes.data, len(g), C.byref(h)))
+        _ck(self._L.mxg_map_create(ctx.h, int(num_global), g.ctypes.data, len(g), C.byref(h)))
         self.h = h
         self.gids = g
 
@@ -422,21 +409,10 @@ class MxMultiVector:
     def from_host(self, arr):
         n, b = self.getLocalLength(), self.GetNumberVecs()
         a = np.asfortranarray(np.asarray(arr, dtype=self.dtype).reshape(n, b))
-        perm = getattr(self.map, "perm", None)
-        if perm is not None:                               # ordered map: the device stores row perm[i] at position i
-            a = np.asfortranarray(a[perm, :])
         _ck(self._L.mxg_mv_upload(self.h, a.ctypes.data, n))
 
     def to_host(self, out=None):
         n, b = self.getLocalLength(), self.GetNumberVecs()
-        perm = getattr(self.map, "perm", None)
-        if perm is not None:
-            dev = np.empty((n, b), dtype=self.dtype, order="F")
-            _ck(self._L.mxg_mv_download(self.h, dev.ctypes.data, n))
-            if out is None:
-                out = np.empty((n, b), dtype=self.dtype, order="F")
-            out[perm, :] = dev
-            return out
         if out is None:
             out = np.empty((n, b), dtype=self.dtype, order="F")
         _ck(self._L.mxg_mv_download(self.h, out.ctypes.data, n))

@@ -420,7 +420,7 @@ def make_map(sim, field, begin=0, end=-1):
     if rc != 0:
         raise AssemblyError("mxg_sim_make_map failed (%d): %s" % (rc, api.lib.mxg_last_error().decode()))
     m = mx.MxMap.__new__(mx.MxMap)
-    m.ctx, m._L, m.h, m.perm = sim.ctx, sim.ctx._L, h, None
+    m.ctx, m._L, m.h = sim.ctx, sim.ctx._L, h
     gids = sim.map(field)
     m.gids = gids[begin:(len(gids) if end < 0 else end)]
     return m

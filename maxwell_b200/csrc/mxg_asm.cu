@@ -141,8 +141,8 @@ extern "C" {
 // MxCrsMatrix::fillComplete for an operator assembled on the device (MxCrsMatrix.cpp:325-342): the rows this rank's
 // row map owns become a device operator (pattern dictionary / sliced ELL, halo plan) without the host ever seeing
 // them: the layout is built by kernels too (mxg::crsCreateFromDevice). A domain map that is not a run of the column
-// field map, and ordered maps, take the host CSR route instead: the rows are downloaded and mxg_crs_create_opts lays
-// them out with the same kernels.
+// field map takes the host CSR route instead: the rows are downloaded and mxg_crs_create_opts lays them out with the
+// same kernels.
 int mxg_crs_create_from_dcsr(mxg_map* row_map, mxg_map* domain_map, const mxg_dcsr* a, int layout, mxg_crs** out) {
   const CsrHandle* A = reinterpret_cast<const CsrHandle*>(a);
   MXG_REQUIRE(row_map && domain_map && A && out, "mxg_crs_create_from_dcsr: NULL argument");
@@ -179,7 +179,7 @@ int mxg_crs_create_from_dcsr(mxg_map* row_map, mxg_map* domain_map, const mxg_dc
       domIsRun = c0 + domain_map->nLocal <= int64_t(colG.size()) &&
                  std::memcmp(colG.data() + c0, domain_map->gids.data(), size_t(domain_map->nLocal) * sizeof(int64_t)) == 0;
     }
-    if (domIsRun && row_map->perm.empty() && domain_map->perm.empty()) {
+    if (domIsRun) {
       const int64_t* rp = (A->isComplex ? A->c.rowptr : A->r.rowptr) + (r1 > r0 ? s0 : 0);
       const int32_t* col = A->isComplex ? A->c.col : A->r.col;
       const void* val = A->isComplex ? static_cast<const void*>(A->c.val) : static_cast<const void*>(A->r.val);

@@ -3,7 +3,6 @@
 #include <cstring>
 
 #include "mxg_internal.h"
-#include "mxg_order.h"
 
 namespace mxg {
 static thread_local char g_err[1024] = "";
@@ -244,45 +243,6 @@ int mxg_map_create(mxg_ctx* ctx, int64_t n_global, const int64_t* my_gids, int64
   }
   *out = m;
   return MXG_OK;
-}
-
-// Same map, but multivectors on it are stored component-major on the device (all DOFs of component 0, then 1, ...;
-// component = GID mod ncomp as in the reference's globCompIndx, MxGridField.hpp:142-145). Single-rank contexts only.
-// mxg_mv_upload / download / col_ptr then speak DEVICE order: the caller permutes with mxg_map_get_order
-// (the C++ / Python veneers do). Operators built on ordered maps are re-indexed inside mxg_crs_create.
-int mxg_map_create_ordered(mxg_ctx* ctx, int64_t n_global, const int64_t* my_gids, int64_t n_local, int ncomp, mxg_map** out) {
-  MXG_REQUIRE(ncomp >= 1 && ncomp <= 16, "mxg_map_create_ordered: ncomp %d outside 1..16", ncomp);
-  int rc = mxg_map_create(ctx, n_global, my_gids, n_local, out);
-  if (rc || ncomp == 1 || n_local == 0) return rc;
-  mxg_map* m = *out;
-  try {
-    m->perm = mxg::componentMajorOrder(my_gids, n_local, ncomp);
-  } catch (const std::exception& e) {   // nothing may unwind through the C boundary
-    mxg_map_destroy(m);
-    *out = nullptr;
-    MXG_REQUIRE(false, "mxg_map_create_ordered: %s", e.what());
-  }
-  bool identity = true;
-  for (int64_t i = 0; i < n_local && identity; ++i) identity = m->perm[size_t(i)] == int32_t(i);
-  if (identity) { m->perm.clear(); return MXG_OK; }
-  m->inv = mxg::inversePermutation(m->perm);
-  std::vector<int64_t> dev(static_cast<size_t>(n_local), 0);
-  for (int64_t i = 0; i < n_local; ++i) dev[size_t(i)] = my_gids[m->perm[size_t(i)]];
-  cudaError_t e = cudaMemcpyAsync(m->dGids, dev.data(), size_t(n_local) * sizeof(int64_t), cudaMemcpyHostToDevice, ctx->stream);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-  if (e != cudaSuccess) {
-    mxg_map_destroy(m);
-    *out = nullptr;
-    MXG_REQUIRE(false, "mxg_map_create_ordered: %s", cudaGetErrorString(e));
-  }
-  return MXG_OK;
-}
-// perm_out[device position] = reference local index (n_local entries); returns 1 if the map is ordered, 0 if the
-// device order is the reference order (perm_out then receives the identity), < 0 on error.
-int mxg_map_get_order(const mxg_map* map, int32_t* perm_out) {
-  MXG_REQUIRE(map && perm_out, "mxg_map_get_order: NULL argument");
-  for (int64_t i = 0; i < map->nLocal; ++i) perm_out[i] = map->perm.empty() ? int32_t(i) : map->perm[size_t(i)];
-  return map->perm.empty() ? 0 : 1;
 }
 
 static void mapRelease(mxg_map* m) {

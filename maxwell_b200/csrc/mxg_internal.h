@@ -114,10 +114,7 @@ struct mxg_map {
   int64_t nGlobal = 0, nLocal = 0;      // size of the GID space / DOFs owned by this rank
   int64_t nMapGlobal = -1;             // DOFs in the map over all ranks (lazily all-reduced: mxg::mapGlobalCount)
   std::vector<int64_t> gids;           // host copy (ascending)
-  int64_t* dGids = nullptr;            // device copy (RNG keys, halo plans); in DEVICE order when the map is ordered
-  // Optional component-major device ordering (mxg_map_create_ordered): perm[device position] = reference local index,
-  // inv = its inverse. Empty = device order is the reference order (ascending GID).
-  std::vector<int32_t> perm, inv;
+  int64_t* dGids = nullptr;            // device copy (RNG keys, halo plans)
   int refs = 1;
 };
 

@@ -24,7 +24,6 @@
 
 #include "mxg_internal.h"
 #include "mxg_ilv_model.h"
-#include "mxg_order.h"
 #include "mxg_spmm_win.cuh"
 #include "mxg_scan.cuh"
 
@@ -1542,25 +1541,6 @@ int buildImpl(mxg_crs* A, const int64_t* rowptr, const int64_t* colGids, const d
     rp[r + 1] = int64_t(ext.size());
   }
   A->nnz = int64_t(ext.size());
-  // Ordered maps (mxg_map_create_ordered): rows move to their device positions and owned columns are translated; the
-  // entry order inside a row stays the reference's ascending local column, so sums keep Epetra's order bit for bit.
-  if (!A->rowMap->perm.empty() || !A->domMap->perm.empty()) {
-    MXG_REQUIRE(ctx->nranks == 1 && ghosts.empty(), "mxg_crs_create: ordered maps are supported on single-rank contexts only");
-    std::vector<int32_t> rowPerm = A->rowMap->perm, colInv = A->domMap->inv;
-    if (rowPerm.empty()) { rowPerm.resize(size_t(nRows)); for (int64_t i = 0; i < nRows; ++i) rowPerm[size_t(i)] = int32_t(i); }
-    if (colInv.empty()) { colInv.resize(size_t(nLoc)); for (int64_t i = 0; i < nLoc; ++i) colInv[size_t(i)] = int32_t(i); }
-    std::vector<int64_t> rp2;
-    std::vector<int32_t> ext2;
-    std::vector<T> val2;
-    try {
-      mxg::permuteCsr(rp, ext, val, rowPerm, colInv, nLoc, rp2, ext2, val2);
-    } catch (const std::exception& e) {   // nothing may unwind through the C boundary
-      MXG_REQUIRE(false, "mxg_crs_create: %s", e.what());
-    }
-    rp.swap(rp2);
-    ext.swap(ext2);
-    val.swap(val2);
-  }
   setInterior(A, needsGhost);
 
   // the merged rows go to the device for the common back end
@@ -1687,7 +1667,6 @@ int crsCreateFromDevice(mxg_map* rowMap, mxg_map* domMap, const int64_t* dRowptr
   MXG_REQUIRE(rowMap && domMap && dRowptr && out, "mxg_crs_create_from_dcsr: NULL argument");
   MXG_REQUIRE(rowMap->ctx == domMap->ctx, "mxg_crs_create_from_dcsr: maps live on different contexts");
   MXG_REQUIRE(layout >= 0 && layout <= 1, "mxg_crs_create_from_dcsr: unknown layout %d", layout);
-  MXG_REQUIRE(rowMap->perm.empty() && domMap->perm.empty(), "mxg_crs_create_from_dcsr: ordered maps are not supported by the device front end");
   return crsCreate(rowMap, domMap, isComplex, out, [&](mxg_crs* A) {
     return A->isComplex ? buildFromDeviceImpl<zd>(A, dRowptr, dCol, dVal, colBegin, colFieldSize, colFieldGids, layout)
                         : buildFromDeviceImpl<double>(A, dRowptr, dCol, dVal, colBegin, colFieldSize, colFieldGids, layout);
@@ -1773,7 +1752,6 @@ int mxg_crs_apply_host_batch(const mxg_crs* A, int count, const double* const* x
   if (count == 0) return MXG_OK;
   for (int i = 0; i < count; ++i) MXG_REQUIRE(x_host[i] && y_host[i], "mxg_crs_apply_host_batch: NULL buffer %d", i);
   mxg_ctx* ctx = A->ctx;
-  MXG_REQUIRE(A->rowMap->perm.empty() && A->domMap->perm.empty(), "mxg_crs_apply_host_batch: operator lives on ordered maps");
   MXG_CUDA(cudaSetDevice(ctx->device));
   const size_t esz = A->isComplex ? 16 : 8;
   mxg_mv *xs[2] = {nullptr, nullptr}, *ys[2] = {nullptr, nullptr};

@@ -1,6 +1,5 @@
 // extern "C" wrapper so the Python tests can feed REAL operator patterns (from the oracle) to the cost model.
 #include "mxg_ilv_model.h"
-#include "mxg_order.h"
 
 extern "C" int ilv_model_eval(const int32_t* rowPat, const int32_t* patOff, const int32_t* delta, int64_t rowBegin, int64_t rowEnd,
                               int xBytes, int patEntryBytes, double out[5]) {
@@ -12,23 +11,4 @@ extern "C" int ilv_model_wins(const double cost[5]) {
   mxg::IlvCost c;
   c.pat[0] = cost[0]; c.pat[1] = cost[1]; c.col[0] = cost[2]; c.col[1] = cost[3]; c.tiles = int(cost[4]);
   return mxg::ilvWins(c) ? 1 : 0;
-}
-
-// component-major ordering helpers (mxg_order.h)
-extern "C" int order_component_major(const int64_t* gids, int64_t n, int ncomp, int32_t* perm, int32_t* inv) {
-  const std::vector<int32_t> p = mxg::componentMajorOrder(gids, n, ncomp);
-  const std::vector<int32_t> q = mxg::inversePermutation(p);
-  for (int64_t i = 0; i < n; ++i) { perm[i] = p[size_t(i)]; inv[i] = q[size_t(i)]; }
-  return 0;
-}
-extern "C" int order_permute_csr(int64_t nRows, const int64_t* rowptr, const int32_t* col, const double* val, const int32_t* rowPerm,
-                                 const int32_t* colInv, int64_t nLoc, int64_t* outRowptr, int32_t* outCol, double* outVal) {
-  std::vector<int64_t> rp(rowptr, rowptr + nRows + 1), orp;
-  std::vector<int32_t> c(col, col + rp[size_t(nRows)]), oc, rperm(rowPerm, rowPerm + nRows), cinv(colInv, colInv + nLoc);
-  std::vector<double> v(val, val + rp[size_t(nRows)]), ov;
-  mxg::permuteCsr(rp, c, v, rperm, cinv, nLoc, orp, oc, ov);
-  std::copy(orp.begin(), orp.end(), outRowptr);
-  std::copy(oc.begin(), oc.end(), outCol);
-  std::copy(ov.begin(), ov.end(), outVal);
-  return 0;
 }

@@ -117,7 +117,6 @@ def test_error_convention_without_gpu(mx):
     assert L.mxg_crs_apply(None, None, None) < 0 and b"mxg_crs_apply" in L.mxg_last_error()
     h = C.c_void_p()
     assert L.mxg_map_create(None, 10, None, 0, C.byref(h)) < 0
-    assert L.mxg_map_create_ordered(None, 10, None, 0, 99, C.byref(h)) < 0 and b"ncomp" in L.mxg_last_error()
     assert L.mxg_mv_to_grid(None, 0, 0, 0, None, None) < 0
     assert L.mxg_crs_apply_host_batch(None, 1, None, None) < 0
     assert L.mxg_gmg_apply(None, None, None) < 0

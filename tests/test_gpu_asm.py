@@ -204,6 +204,31 @@ def test_host_and_device_rows_make_the_same_layout(asm, mx, ctx, orc, case, name
     assert H.stats()["rows"] == d.nrows
 
 
+def test_domain_map_that_is_not_a_run_of_the_field_map(asm, mx, ctx, orc):
+    """A domain map that is not a contiguous run of the column field's map (here every GID of the B field's space) sends
+    mxg_crs_create_from_dcsr through its download route: the rows come to the host and mxg_crs_create lays them out, so
+    the operator must be the one the oracle's rows make on the same two maps."""
+    o, p = orc.pillbox(20), asm.example_sim(ctx, "pillbox", 20)
+    op = o.op("curlCurl")
+    bmap = asm.make_map(p, "bfield")
+    n = o.num_global("bfield")
+    assert len(bmap.gids) < n
+    dense = mx.MxMap(ctx, n, np.arange(n))
+    for layout in (0, 1):
+        A = asm.to_crs(p.op("curlCurl"), bmap, dense, layout=layout)
+        H = mx.MxCrsMatrix.from_csr(bmap, dense, *_global(op), layout=layout)
+        assert A.stats() == H.stats(), (layout, A.stats(), H.stats())
+        x = mx.MxMultiVector(dense, 3)
+        x.random(4242)
+        ys = []
+        for M in (A, H):
+            y = mx.MxMultiVector(bmap, 3)
+            M.apply(x, y)
+            ys.append(y.to_host())
+        assert np.array_equal(ys[0], ys[1]), layout
+        assert np.array_equal(ys[0], op.apply(x.to_host()[op.maps()[1]])), layout
+
+
 def _global(op):
     rowptr, col, val = op.arrays()
     _, cg = op.maps()

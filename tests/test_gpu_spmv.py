@@ -178,18 +178,6 @@ def test_host_buffer_batch_apply(mx, ctx, orc, is_complex):
     A.apply_host_batch([], [])
 
 
-def test_component_major_ordered_maps():
-    """mxg_map_create_ordered: vectors stored component-major on the device, operators re-indexed at creation. Results must
-    equal the reference order bit for bit. Runs in its own process (tests/ordered_map_check.py)."""
-    import os
-    import subprocess
-    import sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    res = subprocess.run([sys.executable, os.path.join(root, "tests", "ordered_map_check.py")], capture_output=True, text=True,
-                         timeout=600)
-    assert res.returncode == 0 and "ORDERED MAPS OK" in res.stdout, res.stdout[-2000:] + res.stderr[-2000:]
-
-
 def test_literal_reference_operator_r13(mx, ctx, orc):
     """DESIGN.md R13: read literally, MxYeeFitEField::getCompFactor (MxYeeFitEField.cpp:90-98) drops curlE's wrap-around
     entries on a periodic upper boundary (MxGridField.cpp:64-74). The oracle can generate that operator too

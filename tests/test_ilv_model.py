@@ -68,56 +68,3 @@ def test_model_on_real_operators(tmp_path, orc):
     assert not got["vecLapl"][0] and got["vecLapl"][1] > 1.3, got
     assert not got["scaLapl"][0] and not got["curlE"][0], got
 
-
-def _table_from_arrays(rowptr, col, val, min_count=4):
-    class _Op:
-        pass
-    o = _Op()
-    o.nrows = len(rowptr) - 1
-    o.arrays = lambda: (rowptr, col, val)
-    return _pattern_table(o, min_count)
-
-
-def test_component_major_order_keeps_results_and_cuts_lines(tmp_path, orc):
-    """mxg_order.h (host half of the planned component-major device ordering): the re-indexed CSR gives bit-identical
-    results through the permutation, and the line-count model rates it at roughly half the L1 lines of today's order
-    for curl-curl without hurting the vector Laplacian."""
-    so = str(tmp_path / "libilv.so")
-    subprocess.check_call([CXX, "-std=c++17", "-O2", "-shared", "-fPIC", "-I", INC, os.path.join(ROOT, "tests", "cpp", "ilv_model_capi.cpp"),
-                           "-o", so])
-    L = C.CDLL(so)
-    vp = C.c_void_p
-    sim = orc.pillbox(32)
-    gids = np.ascontiguousarray(sim.map("bfield"), dtype=np.int64)
-    n = len(gids)
-    perm, inv = np.empty(n, np.int32), np.empty(n, np.int32)
-    L.order_component_major(gids.ctypes.data_as(vp), C.c_int64(n), 3, perm.ctypes.data_as(vp), inv.ctypes.data_as(vp))
-    assert sorted(perm.tolist()) == list(range(n)) and np.array_equal(inv[perm], np.arange(n))
-    comp = gids[perm] % 3
-    assert np.all(np.diff(comp) >= 0)                                   # grouped by component ...
-    for c in range(3):
-        assert np.all(np.diff(gids[perm][comp == c]) > 0)               # ... ascending cell inside a group
-    ratios = {}
-    for name in ("curlCurl", "vecLapl"):
-        op = sim.op(name)
-        rowptr, col, val = op.arrays()
-        rowptr = np.ascontiguousarray(rowptr, dtype=np.int64)
-        col = np.ascontiguousarray(col, dtype=np.int32)
-        val = np.ascontiguousarray(val, dtype=np.float64)
-        orp, oc, ov = np.empty_like(rowptr), np.empty_like(col), np.empty_like(val)
-        L.order_permute_csr(C.c_int64(n), rowptr.ctypes.data_as(vp), col.ctypes.data_as(vp), val.ctypes.data_as(vp),
-                            perm.ctypes.data_as(vp), inv.ctypes.data_as(vp), C.c_int64(n), orp.ctypes.data_as(vp),
-                            oc.ctypes.data_as(vp), ov.ctypes.data_as(vp))
-        x = np.random.default_rng(5).uniform(-1, 1, n)
-        y = op.apply(x)
-        y_dev = orc.csr_apply(orp, oc, ov, x[perm])                     # device order in, device order out
-        assert np.array_equal(y_dev, y[perm]), name                     # bit-identical through the permutation
-        costs = []
-        for rp_, c_, v_ in ((rowptr, col, val), (orp, oc, ov)):
-            t = _table_from_arrays(rp_, c_, v_)
-            out = (C.c_double * 5)()
-            L.ilv_model_eval(t[0].ctypes.data_as(vp), t[1].ctypes.data_as(vp), t[2].ctypes.data_as(vp), C.c_int64(0), C.c_int64(n), 8, 16, out)
-            costs.append(out[0] + out[2])                               # plain thread -> row assignment
-        ratios[name] = costs[1] / costs[0]
-    assert ratios["curlCurl"] < 0.65, ratios
-    assert ratios["vecLapl"] < 1.05, ratios
