@@ -140,9 +140,8 @@ extern "C" {
 
 // MxCrsMatrix::fillComplete for an operator assembled on the device (MxCrsMatrix.cpp:325-342): the rows this rank's
 // row map owns become a device operator (pattern dictionary / sliced ELL, halo plan) without the host ever seeing
-// them: the layout is built by kernels too (mxg::crsCreateFromDevice). A domain map that is not a run of the column
-// field map takes the host CSR route instead: the rows are downloaded and mxg_crs_create_opts lays them out with the
-// same kernels.
+// them: the layout is built by kernels too (mxg::crsCreateFromDevice), which find the columns the domain map owns
+// from the column field map's device GIDs.
 int mxg_crs_create_from_dcsr(mxg_map* row_map, mxg_map* domain_map, const mxg_dcsr* a, int layout, mxg_crs** out) {
   const CsrHandle* A = reinterpret_cast<const CsrHandle*>(a);
   MXG_REQUIRE(row_map && domain_map && A && out, "mxg_crs_create_from_dcsr: NULL argument");
@@ -154,9 +153,8 @@ int mxg_crs_create_from_dcsr(mxg_map* row_map, mxg_map* domain_map, const mxg_dc
     MXG_REQUIRE(domain_map->nGlobal == asC.numGlobal(cf) && row_map->nGlobal == asR.numGlobal(rf),
                 "mxg_crs_create_from_dcsr: maps do not span the simulation's GID space");
     MXG_REQUIRE(asR.mapSize(rf) == A->mapRows() && asC.mapSize(cf) == A->ncols(), "mxg_crs_create_from_dcsr: the matrix does not live on these field maps");
-    std::vector<int64_t> rowG(static_cast<size_t>(asR.mapSize(rf)), 0), colG(static_cast<size_t>(asC.mapSize(cf)), 0);
+    std::vector<int64_t> rowG(static_cast<size_t>(asR.mapSize(rf)), 0);
     asR.copyMap(rf, rowG.data());
-    asC.copyMap(cf, colG.data());
     // the rank's rows: one contiguous run of the field map (x-slabs)
     int64_t r0 = 0, r1 = 0;
     if (row_map->nLocal > 0) {
@@ -171,35 +169,10 @@ int mxg_crs_create_from_dcsr(mxg_map* row_map, mxg_map* domain_map, const mxg_dc
     MXG_REQUIRE(r1 == r0 || (s0 >= 0 && s0 + (r1 - r0) <= A->nrows()),
                 "mxg_crs_create_from_dcsr: the matrix stores the rows [%lld, %lld) of its map, not the row map's [%lld, %lld)",
                 (long long)A->rowBegin(), (long long)(A->rowBegin() + A->nrows()), (long long)r0, (long long)r1);
-    // this rank's columns: the run of the column field map its domain map owns
-    int64_t c0 = 0;
-    bool domIsRun = true;
-    if (domain_map->nLocal > 0) {
-      c0 = int64_t(std::lower_bound(colG.begin(), colG.end(), domain_map->gids.front()) - colG.begin());
-      domIsRun = c0 + domain_map->nLocal <= int64_t(colG.size()) &&
-                 std::memcmp(colG.data() + c0, domain_map->gids.data(), size_t(domain_map->nLocal) * sizeof(int64_t)) == 0;
-    }
-    if (domIsRun) {
-      const int64_t* rp = (A->isComplex ? A->c.rowptr : A->r.rowptr) + (r1 > r0 ? s0 : 0);
-      const int32_t* col = A->isComplex ? A->c.col : A->r.col;
-      const void* val = A->isComplex ? static_cast<const void*>(A->c.val) : static_cast<const void*>(A->r.val);
-      return mxg::crsCreateFromDevice(row_map, domain_map, rp, col, val, c0, int64_t(colG.size()), colG.data(), A->isComplex, layout, out);
-    }
-    // maps the device front end does not take: the rows pass through the host CSR entry point
-    const int64_t n = r1 - r0;
-    std::vector<int64_t> rowptr(static_cast<size_t>(n) + 1, 0);
-    const int64_t d0 = r1 > r0 ? s0 : 0;
-    int rc = mxg_dcsr_download(a, d0, d0 + n, rowptr.data(), nullptr, nullptr);
-    if (rc) return rc;
-    const int64_t cnt = rowptr[size_t(n)];
-    std::vector<int32_t> col(static_cast<size_t>(std::max<int64_t>(cnt, 1)), 0);
-    std::vector<double> val(static_cast<size_t>(std::max<int64_t>(cnt, 1)) * (A->isComplex ? 2 : 1), 0.0);
-    rc = mxg_dcsr_download(a, d0, d0 + n, rowptr.data(), col.data(), val.data());
-    if (rc) return rc;
-    std::vector<int64_t> gcol(static_cast<size_t>(std::max<int64_t>(cnt, 1)), 0);
-    for (int64_t q = 0; q < cnt; ++q) gcol[size_t(q)] = colG[size_t(col[size_t(q)])];
-    std::vector<int32_t>().swap(col);
-    return mxg_crs_create_opts(row_map, domain_map, rowptr.data(), gcol.data(), val.data(), A->isComplex, layout, out);
+    const int64_t* rp = (A->isComplex ? A->c.rowptr : A->r.rowptr) + (r1 > r0 ? s0 : 0);
+    const int32_t* col = A->isComplex ? A->c.col : A->r.col;
+    const void* val = A->isComplex ? static_cast<const void*>(A->c.val) : static_cast<const void*>(A->r.val);
+    return mxg::crsCreateFromDevice(row_map, domain_map, rp, col, val, asC.mapSize(cf), asC.mapGids(cf), A->isComplex, layout, out);
   } catch (const std::exception& e) {
     MXG_REQUIRE(false, "mxg_crs_create_from_dcsr: %s", e.what());
   }

@@ -310,6 +310,7 @@ class Assembler {
   int64_t mapSize(int kind) const { return h_.f[kind].nLoc; }
   int64_t numGlobal(int kind) const { return mxy::numNodes(h_.g) * h_.f[kind].ncomp; }
   void copyMap(int kind, int64_t* out) { x_.toHost(out, h_.f[kind].gids, size_t(h_.f[kind].nLoc) * sizeof(int64_t)); }
+  const int64_t* mapGids(int kind) const { return h_.f[kind].gids; }   // executor memory, mapSize(kind) ascending GIDs
   void copyFractions(int kind, double* out) {
     const mxy::Field& f = h_.f[kind];
     if (!f.region) throw std::runtime_error("field has no PEC fractions");

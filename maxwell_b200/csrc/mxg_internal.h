@@ -230,9 +230,9 @@ int mapGlobalCount(mxg_map* map, int64_t* out);
 int checkHaloFault(const mxg_ctx* ctx, const char* where);
 // Device layout builder (mxg_spmv.cu): rows of a CRS matrix that already sits in device memory -> operator. dRowptr
 // points at the first row of rowMap and holds offsets into dCol / dVal; columns are positions in the column field's map,
-// of which domMap owns [colBegin, colBegin + nLocal). colFieldGids: host copy of that field map.
-int crsCreateFromDevice(mxg_map* rowMap, mxg_map* domMap, const int64_t* dRowptr, const int32_t* dCol, const void* dVal, int64_t colBegin,
-                        int64_t colFieldSize, const int64_t* colFieldGids, int isComplex, int layout, mxg_crs** out);
+// whose K GIDs (ascending) keyGids holds in device memory. domMap owns the columns whose GIDs it lists.
+int crsCreateFromDevice(mxg_map* rowMap, mxg_map* domMap, const int64_t* dRowptr, const int32_t* dCol, const void* dVal, int64_t K,
+                        const int64_t* keyGids, int isComplex, int layout, mxg_crs** out);
 inline int gridFor(const mxg_ctx* ctx, int64_t work, int block, int perSM) {
   int64_t need = (work + block - 1) / block;
   int64_t cap = int64_t(ctx->numSMs) * perSM;

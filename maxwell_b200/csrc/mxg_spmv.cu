@@ -928,7 +928,7 @@ int setupP2P(mxg_crs* A, int64_t gTot) {
 }
 
 // Who owns which ghost: every rank publishes its ghost GID list, owners answer with send lists.
-int planHalo(mxg_crs* A, const std::vector<int64_t>& ghosts, const std::vector<int32_t>& domLookup, int64_t domLo, int64_t domHi) {
+int planHalo(mxg_crs* A, const std::vector<int64_t>& ghosts, int64_t domLo, int64_t domHi) {
   mxg_ctx* ctx = A->ctx;
   const int P = ctx->nranks;
   if (P == 1) return MXG_OK;
@@ -967,6 +967,7 @@ int planHalo(mxg_crs* A, const std::vector<int64_t>& ghosts, const std::vector<i
   MXG_CUDA(cudaStreamSynchronize(ctx->stream));
   MXG_CUDA(cudaFree(dRange));
 
+  const std::vector<int64_t>& dom = A->domMap->gids;
   std::vector<int32_t> sendIdx;
   A->peers.clear();
   for (int q = 0; q < P; ++q) {
@@ -978,10 +979,10 @@ int planHalo(mxg_crs* A, const std::vector<int64_t>& ghosts, const std::vector<i
     for (int64_t i = 0; i < cnt[q]; ++i) {
       const int64_t g = all[size_t(q) * maxCnt + i];
       if (g >= domLo && g <= domHi) {
-        const int32_t l = domLookup[g];
-        MXG_REQUIRE(l >= 0, "mxg_crs_create: rank %d asks for GID %lld which lies in rank %d's range but is not in its map",
+        const auto it = std::lower_bound(dom.begin(), dom.end(), g);
+        MXG_REQUIRE(*it == g, "mxg_crs_create: rank %d asks for GID %lld which lies in rank %d's range but is not in its map",
                     q, (long long)g, ctx->rank);
-        sendIdx.push_back(l);
+        sendIdx.push_back(int32_t(it - dom.begin()));
       }
     }
     peer.sendCount = int64_t(sendIdx.size()) - peer.sendOffset;
@@ -1070,11 +1071,12 @@ int planKernels(mxg_crs* A, const std::vector<int32_t>& rowPat, const std::vecto
 }
 
 // ---- layout construction ----------------------------------------------------------------------------------------------
-// Two front ends bring a rank's rows into extended local columns: buildImpl from host CSR with global column ids
-// (mxg_crs_create), buildFromDeviceImpl from CRS rows that already sit in device memory (the operator assembly, mxg_asm.cu).
-// One back end, layoutFromDeviceRows, lays those rows out: the pattern dictionary (a device hash table), sliced ELL and the
-// inverse diagonal are kernels; the host keeps what is small or collective -- pattern ordering (a few thousand
-// candidates), the halo plan and the tile planner on a downloaded row -> pattern map.
+// One front end, frontEnd, brings a rank's device rows into extended local columns: rows from host CSR (mxg_crs_create,
+// merged on the host and uploaded with the GIDs as column keys) and rows the operator assembly left in device memory
+// (mxg_asm.cu, column keys = positions in the column field's map). One back end, layoutFromDeviceRows, lays those rows out:
+// the pattern dictionary (a device hash table), sliced ELL and the inverse diagonal are kernels; the host keeps what is
+// small or collective -- pattern ordering (a few thousand candidates), the halo plan and the tile planner on a downloaded
+// row -> pattern map.
 struct Scratch {
   std::vector<void*> p;
   ~Scratch() { for (void* q : p) if (q) cudaFree(q); }
@@ -1089,31 +1091,52 @@ struct Scratch {
 
 constexpr unsigned long long kLbEmpty = 0xFFFFFFFFFFFFFFFFull;
 
-__global__ void k_lb_mark_ghosts(const int32_t* __restrict__ col, int64_t cnt, int64_t c0, int64_t c1, int32_t* __restrict__ flag) {
-  for (int64_t q = int64_t(blockIdx.x) * blockDim.x + threadIdx.x; q < cnt; q += int64_t(gridDim.x) * blockDim.x) {
-    const int64_t l = col[q];
-    if (l < c0 || l >= c1) flag[l] = 1;
+__device__ __forceinline__ int64_t lbKeyGid(const int64_t* keyGids, int64_t k) { return keyGids ? keyGids[k] : k; }
+// lid[k] = position of key k's GID in the domain map's ascending GIDs, or -1 when the map does not own it
+__global__ void k_lb_lid(const int64_t* __restrict__ keyGids, int64_t K, const int64_t* __restrict__ domGids, int64_t nLoc,
+                         int32_t* __restrict__ lid) {
+  for (int64_t k = int64_t(blockIdx.x) * blockDim.x + threadIdx.x; k < K; k += int64_t(gridDim.x) * blockDim.x) {
+    const int64_t g = lbKeyGid(keyGids, k);
+    int64_t lo = 0, hi = nLoc;
+    while (lo < hi) {
+      const int64_t m = (lo + hi) >> 1;
+      if (domGids[m] < g) lo = m + 1;
+      else hi = m;
+    }
+    lid[k] = lo < nLoc && domGids[lo] == g ? int32_t(lo) : -1;
   }
 }
-__global__ void k_lb_compact(const int32_t* __restrict__ flag, const int64_t* __restrict__ off, int64_t n, int32_t* __restrict__ list) {
-  for (int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x; i < n; i += int64_t(gridDim.x) * blockDim.x)
-    if (flag[i]) list[off[i]] = int32_t(i);
+__global__ void k_lb_mark_ghosts(const int32_t* __restrict__ key, int64_t cnt, const int32_t* __restrict__ lid, int32_t* __restrict__ flag) {
+  for (int64_t q = int64_t(blockIdx.x) * blockDim.x + threadIdx.x; q < cnt; q += int64_t(gridDim.x) * blockDim.x) {
+    const int32_t k = key[q];
+    if (lid[k] < 0) flag[k] = 1;
+  }
 }
-// extended local column of every entry (owned: 0 .. nLoc-1; ghosts below / above the owned range: negative / >= nLoc)
-__global__ void k_lb_ext(const int64_t* __restrict__ rp, const int32_t* __restrict__ colG, int64_t nRows, int64_t base, int64_t c0,
-                         int64_t c1, int64_t nLoc, int64_t gLo, const int64_t* __restrict__ ghostOff, int32_t* __restrict__ ext,
-                         uint8_t* __restrict__ needs, int* __restrict__ err) {
+// GIDs of the flagged keys, ascending because the keys are
+__global__ void k_lb_compact(const int32_t* __restrict__ flag, const int64_t* __restrict__ off, int64_t K, const int64_t* __restrict__ keyGids,
+                             int64_t* __restrict__ ghosts) {
+  for (int64_t k = int64_t(blockIdx.x) * blockDim.x + threadIdx.x; k < K; k += int64_t(gridDim.x) * blockDim.x)
+    if (flag[k]) ghosts[off[k]] = lbKeyGid(keyGids, k);
+}
+// extended local column of every entry (owned: 0 .. nLoc-1; ghosts below / above the owned range: negative / >= nLoc).
+// Without ghostOff (one rank) a key the domain map does not own is an error: the smallest such GID lands in *bad.
+__global__ void k_lb_ext(const int64_t* __restrict__ rp, const int32_t* __restrict__ key, int64_t nRows, int64_t base,
+                         const int32_t* __restrict__ lid, const int64_t* __restrict__ keyGids, int64_t nLoc, int64_t gLo,
+                         const int64_t* __restrict__ ghostOff, int32_t* __restrict__ ext, uint8_t* __restrict__ needs,
+                         unsigned long long* __restrict__ bad) {
   for (int64_t r = int64_t(blockIdx.x) * blockDim.x + threadIdx.x; r < nRows; r += int64_t(gridDim.x) * blockDim.x) {
     bool ghost = false;
     for (int64_t q = rp[r]; q < rp[r + 1]; ++q) {
-      const int64_t l = colG[q];
-      int32_t e;
-      if (l >= c0 && l < c1) e = int32_t(l - c0);
-      else if (ghostOff) {
-        const int64_t pos = ghostOff[l];
+      const int32_t k = key[q];
+      int32_t e = lid[k];
+      if (e < 0 && ghostOff) {
+        const int64_t pos = ghostOff[k];
         e = pos < gLo ? int32_t(pos - gLo) : int32_t(nLoc + (pos - gLo));
         ghost = true;
-      } else { *err = 1; e = 0; }
+      } else if (e < 0) {
+        atomicMin(bad, (unsigned long long)lbKeyGid(keyGids, k));
+        e = 0;
+      }
       ext[q - base] = e;
     }
     if (needs) needs[r] = ghost ? 1 : 0;
@@ -1470,60 +1493,100 @@ int layoutFromDeviceRows(mxg_crs* A, const int64_t* dRp, const int32_t* dExt, co
   return MXG_OK;
 }
 
-// Host front end (mxg_crs_create): host CSR rows with global column ids.
+// Front end of every operator: the rows of a CRS in device memory (dRp: nRows + 1 offsets into dKey / dVal, which index
+// entries from dRp[0]; rows merged) whose columns are keys in [0, K), ascending in GID: the GID itself (keyGids == nullptr)
+// or a position in a field map whose device GIDs keyGids holds. A key's GID is owned (its position in the domain map) or a
+// ghost; ghosts and the halo plan come first, then the extended local columns and the layout.
 template <class T>
-int buildImpl(mxg_crs* A, const int64_t* rowptr, const int64_t* colGids, const double* valsIn, int layout) {
-  const char* fn = "mxg_crs_create";
+int frontEnd(mxg_crs* A, const int64_t* dRp, const int32_t* dKey, int64_t K, const int64_t* keyGids, const T* dVal, int layout,
+             const char* fn) {
   mxg_ctx* ctx = A->ctx;
-  const T* vals = reinterpret_cast<const T*>(valsIn);
+  cudaStream_t st = ctx->stream;
   const int64_t nRows = A->nRows, nLoc = A->nLoc;
-  const int64_t nnzIn = rowptr[nRows];
   const mxg_map* dom = A->domMap;
-  MXG_REQUIRE(dom->nGlobal < (int64_t(1) << 31), "mxg_crs_create: global size must fit in 31 bits");
-
-  // GID -> local id of the domain map
-  std::vector<int32_t> lookup(size_t(dom->nGlobal), -1);
-  for (int64_t i = 0; i < nLoc; ++i) lookup[dom->gids[i]] = int32_t(i);
+  const bool multi = ctx->nranks > 1;
+  Scratch tmp;
+  int64_t ends[2] = {0, 0};
+  MXG_CUDA(cudaMemcpyAsync(&ends[0], dRp, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+  MXG_CUDA(cudaMemcpyAsync(&ends[1], dRp + nRows, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+  MXG_CUDA(cudaStreamSynchronize(st));
+  const int64_t base = ends[0], cnt = ends[1] - ends[0];
+  A->nnz = cnt;
   const int64_t domLo = nLoc ? dom->gids.front() : 0, domHi = nLoc ? dom->gids.back() : -1;
 
-  // ghosts = referenced GIDs that are not local
+  MXG_LB_ALLOC(dLid, int32_t, K);
+  if (K > 0) k_lb_lid<<<lbGrid(K), 256, 0, st>>>(keyGids, K, dom->dGids, nLoc, dLid);
+  ctx->launches++;
+
+  // ---- ghosts: referenced keys the domain map does not own (several ranks; on one rank they are an error)
   std::vector<int64_t> ghosts;
-  for (int64_t q = 0; q < nnzIn; ++q) {
-    const int64_t g = colGids[q];
-    MXG_REQUIRE(g >= 0 && g < dom->nGlobal, "mxg_crs_create: column GID %lld out of range", (long long)g);
-    if (lookup[g] < 0) ghosts.push_back(g);
+  int64_t* dGhostOff = nullptr;
+  if (multi) {
+    MXG_LB_ALLOC(dFlag, int32_t, K);
+    MXG_LB_ALLOC(dOff, int64_t, K + 1);
+    MXG_CUDA(cudaMemsetAsync(dFlag, 0, size_t(K) * sizeof(int32_t), st));
+    if (cnt > 0) k_lb_mark_ghosts<<<lbGrid(cnt), 256, 0, st>>>(dKey + base, cnt, dLid, dFlag);
+    int64_t ng = 0;
+    MXG_CUDA(exclusiveScan(ctx, dFlag, dOff, K, &ng));
+    if (ng > 0) {
+      MXG_LB_ALLOC(dGhosts, int64_t, ng);
+      k_lb_compact<<<lbGrid(K), 256, 0, st>>>(dFlag, dOff, K, keyGids, dGhosts);
+      ghosts.resize(static_cast<size_t>(ng));
+      MXG_CUDA(cudaMemcpyAsync(ghosts.data(), dGhosts, size_t(ng) * sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+      MXG_CUDA(cudaStreamSynchronize(st));
+    }
+    dGhostOff = dOff;
+    ctx->launches += 2;
   }
-  std::sort(ghosts.begin(), ghosts.end());
-  ghosts.erase(std::unique(ghosts.begin(), ghosts.end()), ghosts.end());
-  MXG_REQUIRE(ghosts.empty() || ctx->nranks > 1, "mxg_crs_create: column GID %lld is not in the domain map",
-              (long long)(ghosts.empty() ? 0 : ghosts[0]));
   A->gLo = int64_t(std::lower_bound(ghosts.begin(), ghosts.end(), domLo) - ghosts.begin());
   if (nLoc == 0) A->gLo = 0;
   A->gHi = int64_t(ghosts.size()) - A->gLo;
-  int rc = planHalo(A, ghosts, lookup, domLo, domHi);
-  if (rc) return rc;
+  const int rcH = planHalo(A, ghosts, domLo, domHi);
+  if (rcH) return rcH;
 
-  // extended local column index of every entry; rows sorted, duplicates merged
+  // ---- extended local columns, rows that need ghost values
+  MXG_LB_ALLOC(dExt, int32_t, cnt);
+  MXG_LB_ALLOC(dBad, unsigned long long, 1);
+  uint8_t* dNeeds = nullptr;
+  if (multi) { MXG_LB_ALLOC(needs_, uint8_t, nRows); dNeeds = needs_; }
+  MXG_CUDA(cudaMemsetAsync(dBad, 0xFF, sizeof(unsigned long long), st));
+  if (nRows > 0)
+    k_lb_ext<<<lbGrid(nRows), 256, 0, st>>>(dRp, dKey, nRows, base, dLid, keyGids, nLoc, A->gLo, dGhostOff, dExt, dNeeds, dBad);
+  ctx->launches++;
+  unsigned long long bad = 0;
+  MXG_CUDA(cudaMemcpyAsync(&bad, dBad, sizeof(bad), cudaMemcpyDeviceToHost, st));
+  std::vector<uint8_t> needs;
+  if (dNeeds) {
+    needs.resize(static_cast<size_t>(nRows));
+    MXG_CUDA(cudaMemcpyAsync(needs.data(), dNeeds, size_t(nRows), cudaMemcpyDeviceToHost, st));
+  }
+  MXG_CUDA(cudaStreamSynchronize(st));
+  MXG_REQUIRE(bad == ~0ull, "%s: column GID %lld is not in the domain map", fn, (long long)bad);
+  setInterior(A, needs);
+  return layoutFromDeviceRows<T>(A, dRp, dExt, dVal, base, layout, fn);
+}
+
+// Host CSR rows with global column ids (mxg_crs_create): each row in GID order with duplicates summed in insertion order,
+// uploaded with the GIDs as column keys.
+template <class T>
+int buildFromHost(mxg_crs* A, const int64_t* rowptr, const int64_t* colGids, const double* valsIn, int layout) {
+  const char* fn = "mxg_crs_create";
+  const T* vals = reinterpret_cast<const T*>(valsIn);
+  const int64_t nRows = A->nRows, nGlobal = A->domMap->nGlobal;
   std::vector<int64_t> rp(nRows + 1, 0);
-  std::vector<int32_t> ext;
+  std::vector<int32_t> key;
   std::vector<T> val;
-  ext.reserve(nnzIn);
-  val.reserve(nnzIn);
-  std::vector<uint8_t> needsGhost(nRows, 0);
+  key.reserve(rowptr[nRows]);
+  val.reserve(rowptr[nRows]);
   std::vector<std::pair<int32_t, T>> rowBuf;
   for (int64_t r = 0; r < nRows; ++r) {
     rowBuf.clear();
     bool sorted = true;
     for (int64_t q = rowptr[r]; q < rowptr[r + 1]; ++q) {
       const int64_t g = colGids[q];
-      int32_t e = lookup[g];
-      if (e < 0) {
-        const int64_t pos = std::lower_bound(ghosts.begin(), ghosts.end(), g) - ghosts.begin();
-        e = pos < A->gLo ? int32_t(pos - A->gLo) : int32_t(nLoc + (pos - A->gLo));
-        needsGhost[r] = 1;
-      }
-      if (!rowBuf.empty() && e <= rowBuf.back().first) sorted = false;
-      rowBuf.emplace_back(e, vals[q]);
+      MXG_REQUIRE(g >= 0 && g < nGlobal, "mxg_crs_create: column GID %lld out of range", (long long)g);
+      if (!rowBuf.empty() && g <= rowBuf.back().first) sorted = false;
+      rowBuf.emplace_back(int32_t(g), vals[q]);
     }
     if (!sorted) {
       std::stable_sort(rowBuf.begin(), rowBuf.end(), [](auto& a, auto& b) { return a.first < b.first; });
@@ -1537,105 +1600,27 @@ int buildImpl(mxg_crs* A, const int64_t* rowptr, const int64_t* colGids, const d
       }
       rowBuf.resize(o);
     }
-    for (auto& t : rowBuf) { ext.push_back(t.first); val.push_back(t.second); }
-    rp[r + 1] = int64_t(ext.size());
+    for (auto& t : rowBuf) { key.push_back(t.first); val.push_back(t.second); }
+    rp[r + 1] = int64_t(key.size());
   }
-  A->nnz = int64_t(ext.size());
-  setInterior(A, needsGhost);
 
-  // the merged rows go to the device for the common back end
   Scratch tmp;
   MXG_LB_ALLOC(dRp, int64_t, nRows + 1);
-  MXG_LB_ALLOC(dExt, int32_t, A->nnz);
-  MXG_LB_ALLOC(dVal, T, A->nnz);
-  cudaStream_t st = ctx->stream;
+  MXG_LB_ALLOC(dKey, int32_t, int64_t(key.size()));
+  MXG_LB_ALLOC(dVal, T, int64_t(val.size()));
+  cudaStream_t st = A->ctx->stream;
   MXG_CUDA(cudaMemcpyAsync(dRp, rp.data(), rp.size() * sizeof(int64_t), cudaMemcpyHostToDevice, st));
-  if (A->nnz > 0) {
-    MXG_CUDA(cudaMemcpyAsync(dExt, ext.data(), ext.size() * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+  if (!key.empty()) {
+    MXG_CUDA(cudaMemcpyAsync(dKey, key.data(), key.size() * sizeof(int32_t), cudaMemcpyHostToDevice, st));
     MXG_CUDA(cudaMemcpyAsync(dVal, val.data(), val.size() * sizeof(T), cudaMemcpyHostToDevice, st));
   }
-  return layoutFromDeviceRows<T>(A, dRp, dExt, dVal, 0, layout, fn);
-}
-
-// Device front end (mxg_crs_create_from_dcsr): rows [base, base + nnz) of a device CRS whose columns are positions in
-// the column field's map, of which this rank owns [c0, c0 + nLoc).
-template <class T>
-int buildFromDeviceImpl(mxg_crs* A, const int64_t* dRp, const int32_t* dColG, const void* dValRaw, int64_t c0, int64_t colFieldSize,
-                        const int64_t* colFieldGids, int layout) {
-  const char* fn = "mxg_crs_create_from_dcsr";
-  mxg_ctx* ctx = A->ctx;
-  cudaStream_t st = ctx->stream;
-  const int64_t nRows = A->nRows, nLoc = A->nLoc, c1 = c0 + nLoc;
-  const mxg_map* dom = A->domMap;
-  MXG_REQUIRE(dom->nGlobal < (int64_t(1) << 31), "mxg_crs_create: global size must fit in 31 bits");
-  Scratch tmp;
-  int64_t ends[2] = {0, 0};
-  MXG_CUDA(cudaMemcpyAsync(&ends[0], dRp, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
-  MXG_CUDA(cudaMemcpyAsync(&ends[1], dRp + nRows, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
-  MXG_CUDA(cudaStreamSynchronize(st));
-  const int64_t base = ends[0], cnt = ends[1] - ends[0];
-  A->nnz = cnt;
-  const int64_t domLo = nLoc ? dom->gids.front() : 0, domHi = nLoc ? dom->gids.back() : -1;
-
-  // ---- ghosts: referenced columns outside this rank's run of the column field map
-  std::vector<int64_t> ghosts;
-  int64_t* dGhostOff = nullptr;
-  if (ctx->nranks > 1) {
-    MXG_LB_ALLOC(dFlag, int32_t, colFieldSize);
-    MXG_LB_ALLOC(dOff, int64_t, colFieldSize + 1);
-    MXG_CUDA(cudaMemsetAsync(dFlag, 0, size_t(colFieldSize) * sizeof(int32_t), st));
-    if (cnt > 0) k_lb_mark_ghosts<<<lbGrid(cnt), 256, 0, st>>>(dColG + base, cnt, c0, c1, dFlag);
-    int64_t ng = 0;
-    MXG_CUDA(exclusiveScan(ctx, dFlag, dOff, colFieldSize, &ng));
-    if (ng > 0) {
-      MXG_LB_ALLOC(dList, int32_t, ng);
-      k_lb_compact<<<lbGrid(colFieldSize), 256, 0, st>>>(dFlag, dOff, colFieldSize, dList);
-      std::vector<int32_t> list(static_cast<size_t>(ng), 0);
-      MXG_CUDA(cudaMemcpyAsync(list.data(), dList, size_t(ng) * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-      MXG_CUDA(cudaStreamSynchronize(st));
-      ghosts.resize(static_cast<size_t>(ng));
-      for (int64_t i = 0; i < ng; ++i) ghosts[size_t(i)] = colFieldGids[list[size_t(i)]];   // ascending: the field map is
-    }
-    dGhostOff = dOff;
-    ctx->launches += 2;
-  }
-  A->gLo = int64_t(std::lower_bound(ghosts.begin(), ghosts.end(), domLo) - ghosts.begin());
-  if (nLoc == 0) A->gLo = 0;
-  A->gHi = int64_t(ghosts.size()) - A->gLo;
-  {
-    std::vector<int32_t> lookup;
-    if (ctx->nranks > 1) {
-      lookup.assign(size_t(dom->nGlobal), -1);
-      for (int64_t i = 0; i < nLoc; ++i) lookup[size_t(dom->gids[size_t(i)])] = int32_t(i);
-    }
-    const int rcH = planHalo(A, ghosts, lookup, domLo, domHi);
-    if (rcH) return rcH;
-  }
-
-  // ---- extended local columns, rows that need ghost values
-  MXG_LB_ALLOC(dExt, int32_t, cnt);
-  MXG_LB_ALLOC(dErr, int, 1);
-  uint8_t* dNeeds = nullptr;
-  if (ctx->nranks > 1) { MXG_LB_ALLOC(needs_, uint8_t, nRows); dNeeds = needs_; }
-  MXG_CUDA(cudaMemsetAsync(dErr, 0, sizeof(int), st));
-  if (nRows > 0) k_lb_ext<<<lbGrid(nRows), 256, 0, st>>>(dRp, dColG, nRows, base, c0, c1, nLoc, A->gLo, dGhostOff, dExt, dNeeds, dErr);
-  ctx->launches++;
-  int hErr = 0;
-  MXG_CUDA(cudaMemcpyAsync(&hErr, dErr, sizeof(int), cudaMemcpyDeviceToHost, st));
-  std::vector<uint8_t> needs;
-  if (dNeeds) {
-    needs.resize(static_cast<size_t>(nRows));
-    MXG_CUDA(cudaMemcpyAsync(needs.data(), dNeeds, size_t(nRows), cudaMemcpyDeviceToHost, st));
-  }
-  MXG_CUDA(cudaStreamSynchronize(st));
-  MXG_REQUIRE(hErr == 0, "mxg_crs_create: a column is not in the domain map (single-rank context)");
-  setInterior(A, needs);
-  return layoutFromDeviceRows<T>(A, dRp, dExt, static_cast<const T*>(dValRaw), base, layout, fn);
+  return frontEnd<T>(A, dRp, dKey, nGlobal, nullptr, dVal, layout, fn);
 }
 
 // A new operator on (rowMap, domMap), laid out by `build`; released again when that fails.
 template <class Build>
 int crsCreate(mxg_map* rowMap, mxg_map* domMap, int isComplex, mxg_crs** out, Build build) {
+  MXG_REQUIRE(domMap->nGlobal < (int64_t(1) << 31), "mxg_crs_create: global size must fit in 31 bits");
   mxg_ctx* ctx = rowMap->ctx;
   MXG_CUDA(cudaSetDevice(ctx->device));
   mxg_crs* A = new mxg_crs;
@@ -1660,16 +1645,15 @@ int crsCreate(mxg_map* rowMap, mxg_map* domMap, int isComplex, mxg_crs** out, Bu
 
 namespace mxg {
 
-// rows [r0, r0 + rowMap->nLocal) of a device CRS (dRowptr points at row r0 and holds offsets into dCol / dVal; columns are
-// positions in the column field's map, of which domMap owns [colBegin, colBegin + nLocal)) -> device operator
-int crsCreateFromDevice(mxg_map* rowMap, mxg_map* domMap, const int64_t* dRowptr, const int32_t* dCol, const void* dVal, int64_t colBegin,
-                        int64_t colFieldSize, const int64_t* colFieldGids, int isComplex, int layout, mxg_crs** out) {
+int crsCreateFromDevice(mxg_map* rowMap, mxg_map* domMap, const int64_t* dRowptr, const int32_t* dCol, const void* dVal, int64_t K,
+                        const int64_t* keyGids, int isComplex, int layout, mxg_crs** out) {
   MXG_REQUIRE(rowMap && domMap && dRowptr && out, "mxg_crs_create_from_dcsr: NULL argument");
   MXG_REQUIRE(rowMap->ctx == domMap->ctx, "mxg_crs_create_from_dcsr: maps live on different contexts");
   MXG_REQUIRE(layout >= 0 && layout <= 1, "mxg_crs_create_from_dcsr: unknown layout %d", layout);
+  const char* fn = "mxg_crs_create_from_dcsr";
   return crsCreate(rowMap, domMap, isComplex, out, [&](mxg_crs* A) {
-    return A->isComplex ? buildFromDeviceImpl<zd>(A, dRowptr, dCol, dVal, colBegin, colFieldSize, colFieldGids, layout)
-                        : buildFromDeviceImpl<double>(A, dRowptr, dCol, dVal, colBegin, colFieldSize, colFieldGids, layout);
+    return A->isComplex ? frontEnd<zd>(A, dRowptr, dCol, K, keyGids, static_cast<const zd*>(dVal), layout, fn)
+                        : frontEnd<double>(A, dRowptr, dCol, K, keyGids, static_cast<const double*>(dVal), layout, fn);
   });
 }
 
@@ -1686,7 +1670,7 @@ int mxg_crs_create_opts(mxg_map* row_map, mxg_map* domain_map, const int64_t* ro
   MXG_REQUIRE(nnz == 0 || (col_gids && vals), "mxg_crs_create: NULL column / value array");
   MXG_REQUIRE(layout >= 0 && layout <= 1, "mxg_crs_create: unknown layout %d", layout);
   return crsCreate(row_map, domain_map, is_complex, out, [&](mxg_crs* A) {
-    return A->isComplex ? buildImpl<zd>(A, rowptr, col_gids, vals, layout) : buildImpl<double>(A, rowptr, col_gids, vals, layout);
+    return A->isComplex ? buildFromHost<zd>(A, rowptr, col_gids, vals, layout) : buildFromHost<double>(A, rowptr, col_gids, vals, layout);
   });
 }
 

@@ -205,9 +205,9 @@ def test_host_and_device_rows_make_the_same_layout(asm, mx, ctx, orc, case, name
 
 
 def test_domain_map_that_is_not_a_run_of_the_field_map(asm, mx, ctx, orc):
-    """A domain map that is not a contiguous run of the column field's map (here every GID of the B field's space) sends
-    mxg_crs_create_from_dcsr through its download route: the rows come to the host and mxg_crs_create lays them out, so
-    the operator must be the one the oracle's rows make on the same two maps."""
+    """A domain map that is not a contiguous run of the column field's map (here every GID of the B field's space): the
+    device rows find their owned columns by GID, so the operator must be the one the oracle's rows make on the same two
+    maps."""
     o, p = orc.pillbox(20), asm.example_sim(ctx, "pillbox", 20)
     op = o.op("curlCurl")
     bmap = asm.make_map(p, "bfield")
@@ -227,6 +227,21 @@ def test_domain_map_that_is_not_a_run_of_the_field_map(asm, mx, ctx, orc):
             ys.append(y.to_host())
         assert np.array_equal(ys[0], ys[1]), layout
         assert np.array_equal(ys[0], op.apply(x.to_host()[op.maps()[1]])), layout
+
+
+def test_columns_outside_a_one_rank_domain_map_are_refused_on_both_routes(asm, mx, ctx, orc):
+    """On one rank every referenced column must be in the domain map. A domain map that owns only the first half of the
+    B field refuses pillbox-20 curlCurl from device rows and from host CSR alike, naming the smallest GID it lacks."""
+    o, p = orc.pillbox(20), asm.example_sim(ctx, "pillbox", 20)
+    op = o.op("curlCurl")
+    bmap = asm.make_map(p, "bfield")
+    half = asm.make_map(p, "bfield", 0, len(bmap.gids) // 2)
+    used = np.unique(_global(op)[1])
+    msg = "column GID %d is not in the domain map" % used[~np.isin(used, half.gids)].min()
+    with pytest.raises(asm.AssemblyError, match=msg):
+        asm.to_crs(p.op("curlCurl"), bmap, half)
+    with pytest.raises(mx.MxError, match=msg):
+        mx.MxCrsMatrix.from_csr(bmap, half, *_global(op))
 
 
 def _global(op):
