@@ -192,10 +192,11 @@ class MxEMSim {
     mx::check(mxg_sim_op(h_, name.c_str(), isComplex ? 1 : 0, nullptr, nullptr, &o));
     return MxDeviceCrs(o, comm_);
   }
-  // MxGridFieldInterpolator (MxGridFieldInterpolator.cpp:28-122): `field` of the coarser simulation at this one's DOFs
-  MxDeviceCrs interpolatorFrom(const MxEMSim& coarse, const std::string& field) const {
+  // MxGridFieldInterpolator (MxGridFieldInterpolator.cpp:28-122): `field` of the coarser simulation at this one's DOFs.
+  // bloch: Bloch factors across periodic faces (MXG_INTERP_BLOCH, DESIGN.md GMG-bloch).
+  MxDeviceCrs interpolatorFrom(const MxEMSim& coarse, const std::string& field, bool bloch = false) const {
     mxg_dcsr* o = nullptr;
-    mx::check(mxg_sim_interpolator(coarse.h_, h_, field.c_str(), complex_ ? 1 : 0, &o));
+    mx::check(mxg_sim_interpolator_ex(coarse.h_, h_, field.c_str(), complex_ ? 1 : 0, bloch ? MXG_INTERP_BLOCH : 0, &o));
     return MxDeviceCrs(o, comm_);
   }
   bool isComplex() const { return complex_; }

@@ -116,6 +116,17 @@ int mxg_sim_interpolator_rows(mxg_sim* sim_from, mxg_sim* sim_to, const char* fi
  * before the 1/8 scaling): the interpolator is generated on the fine rows that can reach those coarse rows only */
 int mxg_sim_interpolator_transpose_rows(mxg_sim* sim_from, mxg_sim* sim_to, const char* field, int is_complex,
                                         int64_t row_begin, int64_t row_end, mxg_dcsr** out);
+/* The same three with flags (the plain ones are flags = 0). MXG_INTERP_BLOCH: a stencil cell that wraps across a periodic
+ * face of sim_from carries that direction's Bloch factor, e^{+i phi} from the top and e^{-i phi} from below, so that the
+ * prolongator maps a coarse Bloch-periodic field onto the fine one (MxGridFieldInterpolator.cpp:28-122 applies none;
+ * DESIGN.md deviation GMG-bloch). Both simulations must have the same phase shifts; a real (is_complex = 0) transfer with
+ * a non-zero phase is an error; with all phases 0 the result equals the plain transfer bit for bit. */
+#define MXG_INTERP_BLOCH 1
+int mxg_sim_interpolator_ex(mxg_sim* sim_from, mxg_sim* sim_to, const char* field, int is_complex, int flags, mxg_dcsr** out);
+int mxg_sim_interpolator_rows_ex(mxg_sim* sim_from, mxg_sim* sim_to, const char* field, int is_complex,
+                                 int64_t row_begin, int64_t row_end, int flags, mxg_dcsr** out);
+int mxg_sim_interpolator_transpose_rows_ex(mxg_sim* sim_from, mxg_sim* sim_to, const char* field, int is_complex,
+                                           int64_t row_begin, int64_t row_end, int flags, mxg_dcsr** out);
 /* out = {rows, columns, entries, is_complex, row field, column field}; fields 0 B, 1 E, 2 psi, -1 unknown. rows counts
  * the stored rows. */
 int mxg_dcsr_shape(const mxg_dcsr* a, int64_t out[6]);

@@ -11,6 +11,7 @@ import numpy as np
 
 PERIODIC, ZERO, CONSTANT, PEC, PMC = 0, 1, 2, 3, 4
 FIELDS = ("bfield", "efield", "psifield")
+INTERP_BLOCH = 1          # include/mxasm.h: MXG_INTERP_BLOCH
 
 
 class AssemblyError(RuntimeError):
@@ -51,6 +52,9 @@ class AssemblyAPI:
             "sim_interpolator": [vp, vp, C.c_char_p, i32, pvp],
             "sim_interpolator_rows": [vp, vp, C.c_char_p, i32, i64, i64, pvp],
             "sim_interpolator_transpose_rows": [vp, vp, C.c_char_p, i32, i64, i64, pvp],
+            "sim_interpolator_ex": [vp, vp, C.c_char_p, i32, i32, pvp],
+            "sim_interpolator_rows_ex": [vp, vp, C.c_char_p, i32, i64, i64, i32, pvp],
+            "sim_interpolator_transpose_rows_ex": [vp, vp, C.c_char_p, i32, i64, i64, i32, pvp],
             "dcsr_shape": [vp, C.POINTER(i64)],
             "dcsr_rows": [vp, C.POINTER(i64)],
             "dcsr_download": [vp, i64, i64, vp, vp, vp],
@@ -142,7 +146,10 @@ class AssemblyAPI:
         self.call("sim_create", ctx_handle, _i3(n), _d3(origin), _d3(size), _i3(lower or (PERIODIC,) * 3),
                   _i3(upper or (PERIODIC,) * 3), _d3(phase_shifts or (0.0, 0.0, 0.0)), float(dm_frac),
                   1 if literal_upper_periodic_e else 0, C.byref(h))
-        return Sim(self, h, n, phase_shifts is not None and any(p != 0 for p in phase_shifts))
+        sim = Sim(self, h, n, phase_shifts is not None and any(p != 0 for p in phase_shifts))
+        sim.lower, sim.upper = tuple(lower or (PERIODIC,) * 3), tuple(upper or (PERIODIC,) * 3)
+        sim.phase_shifts = tuple(float(p) for p in (phase_shifts or (0.0, 0.0, 0.0)))
+        return sim
 
 
 class Shape:
@@ -268,31 +275,40 @@ class Sim:
         if not coarse._setup:
             coarse.setup()
 
-    def interpolator_from(self, coarse, field="bfield", is_complex=None, rows=None):
+    def interpolator_from(self, coarse, field="bfield", is_complex=None, rows=None, bloch=False):
         """MxGridFieldInterpolator: `field` of the simulation `coarse` interpolated at this simulation's DOFs (rows=(begin, end):
-        only those rows of this simulation's map)."""
+        only those rows of this simulation's map). bloch: stencil cells that wrap across a periodic face carry the Bloch
+        factor, so that the transfer maps a coarse Bloch-periodic field onto the fine one (include/mxasm.h: MXG_INTERP_BLOCH)."""
         self._setup_both(coarse)
         cplx = self.is_complex if is_complex is None else bool(is_complex)
         h = C.c_void_p()
-        if rows is None:
-            self.api.call("sim_interpolator", coarse.handle, self.handle, field.encode(), 1 if cplx else 0, C.byref(h))
+        args = (coarse.handle, self.handle, field.encode(), 1 if cplx else 0)
+        if rows is None and not bloch:
+            self.api.call("sim_interpolator", *args, C.byref(h))
+        elif rows is None:
+            self.api.call("sim_interpolator_ex", *args, INTERP_BLOCH, C.byref(h))
+        elif not bloch:
+            self.api.call("sim_interpolator_rows", *args, int(rows[0]), int(rows[1]), C.byref(h))
         else:
-            self.api.call("sim_interpolator_rows", coarse.handle, self.handle, field.encode(), 1 if cplx else 0, int(rows[0]),
-                          int(rows[1]), C.byref(h))
+            self.api.call("sim_interpolator_rows_ex", *args, int(rows[0]), int(rows[1]), INTERP_BLOCH, C.byref(h))
         m = DeviceCsr(self, h)
         m.col_sim = coarse
         return m
 
-    def interpolator_transpose(self, coarse, field="bfield", is_complex=None, rows=None):
-        """The rows (begin, end) of the coarse map of interpolator_from(coarse, field)'s conjugate transpose (the restriction
-        before its 1/8 scaling), generating the interpolator on the fine rows that reach them only. rows=None: all rows."""
+    def interpolator_transpose(self, coarse, field="bfield", is_complex=None, rows=None, bloch=False):
+        """The rows (begin, end) of the coarse map of interpolator_from(coarse, field, bloch=bloch)'s conjugate transpose (the
+        restriction before its 1/8 scaling), generating the interpolator on the fine rows that reach them only. rows=None:
+        all rows."""
         self._setup_both(coarse)
         cplx = self.is_complex if is_complex is None else bool(is_complex)
         if rows is None:
             rows = (0, coarse.map_size(field)[0])
         h = C.c_void_p()
-        self.api.call("sim_interpolator_transpose_rows", coarse.handle, self.handle, field.encode(), 1 if cplx else 0, int(rows[0]),
-                      int(rows[1]), C.byref(h))
+        args = (coarse.handle, self.handle, field.encode(), 1 if cplx else 0, int(rows[0]), int(rows[1]))
+        if bloch:
+            self.api.call("sim_interpolator_transpose_rows_ex", *args, INTERP_BLOCH, C.byref(h))
+        else:
+            self.api.call("sim_interpolator_transpose_rows", *args, C.byref(h))
         m = DeviceCsr(self, h)
         m.row_sim, m.col_sim = coarse, self
         return m
@@ -525,17 +541,35 @@ def example_sim(ctx, workload, n, phase_shifts=None):
     return sim.setup()
 
 
+def scalar_laplacian_has_constant_null_vector(sim):
+    """Whether the constant psi field is a null vector of the simulation's scalar Laplacian, i.e. whether a multigrid cycle on
+    it should run with remove_const_field: every periodic direction has a phase shift that is 0 modulo 2 pi (a Bloch phase
+    couples the constant to its neighbour image with e^{i phi} != 1), and no wall holds psi at zero (a PMC wall or a ZERO
+    boundary: psi is Dirichlet there, MxYeePsiField.cpp:84-93). PEC shapes and PEC walls keep the constant."""
+    import math
+    for lo, up, phi in zip(sim.lower, sim.upper, sim.phase_shifts):
+        if lo == PERIODIC and up == PERIODIC:
+            if abs(math.remainder(phi, 2.0 * math.pi)) > 1e-12:
+                return False
+        elif lo in (ZERO, PMC) or up in (ZERO, PMC):
+            return False
+    return True
+
+
 class EigenProblem:
     """Everything MxSolver needs for the projected eigensolve, assembled on the device: the re-discretisation hierarchy
     of MxEMSimHierarchy (MxEMSimHierarchy.cpp:37-76) for the vector and the scalar Laplacian, trilinear transfers
-    (restriction = P^T / 8), divB / gradPsi / curlCurl on the fine grid and the mass diagonal dmA.
+    (restriction = P^H / 8), divB / gradPsi / curlCurl on the fine grid and the mass diagonal dmA.
 
     sims: device simulations, fine to coarse. cuts(level, field, gids, num_global) -> (begin, end) selects this rank's
     rows of a field map (x-slabs); None = the whole map (one rank). Every operator, transfer and the mass diagonal is
     assembled on this rank's rows only (each chain factor on the rows its left neighbour reaches), so a rank's assembly
-    memory and time shrink with the rank count; the rows are bit-identical to those of the global operators."""
+    memory and time shrink with the rank count; the rows are bit-identical to those of the global operators.
 
-    def __init__(self, ctx, sims, cuts=None, is_complex=False):
+    bloch_transfers: the transfers carry the Bloch factor across periodic faces (Sim.interpolator_from(bloch=True)), which
+    makes the V-cycle converge on Bloch-periodic levels; it needs is_complex when a phase is non-zero."""
+
+    def __init__(self, ctx, sims, cuts=None, is_complex=False, bloch_transfers=False):
         import maxwell_b200 as mx
         self.sims = sims
         rng = {}
@@ -553,10 +587,10 @@ class EigenProblem:
         self.Rb, self.Pb, self.Rp, self.Pp = [], [], [], []
         for l in range(len(sims) - 1):
             for f, maps, Rl, Pl in (("bfield", self.bmaps, self.Rb, self.Pb), ("psifield", self.pmaps, self.Rp, self.Pp)):
-                p = sims[l].interpolator_from(sims[l + 1], f, cx, rows=rng[l, f])
+                p = sims[l].interpolator_from(sims[l + 1], f, cx, rows=rng[l, f], bloch=bloch_transfers)
                 Pl.append(to_crs(p, maps[l], maps[l + 1]))
                 del p
-                r = sims[l].interpolator_transpose(sims[l + 1], f, cx, rows=rng[l + 1, f]).scale(0.125)
+                r = sims[l].interpolator_transpose(sims[l + 1], f, cx, rows=rng[l + 1, f], bloch=bloch_transfers).scale(0.125)
                 Rl.append(to_crs(r, maps[l + 1], maps[l]))
         s0 = sims[0]
         b0, b1 = rng[0, "bfield"]

@@ -12,6 +12,7 @@
 #include <cstring>
 #include <stdexcept>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "mxg_yee.h"
@@ -152,6 +153,7 @@ class Assembler {
     std::complex<double> phase[3];
     for (int i = 0; i < 3; ++i) phase[i] = std::exp(std::complex<double>(0.0, 1.0) * phaseShifts[i]);   // MxGridField.cpp:34-38
     complex_ = phaseShifts[0] != 0 || phaseShifts[1] != 0 || phaseShifts[2] != 0;
+    for (int i = 0; i < 3; ++i) phase_[i] = phaseShifts[i];
     for (int k = 0; k < mxy::NUM_ALL_FIELDS; ++k) {
       mxy::Field& f = h_.f[k];
       f.kind = k;
@@ -495,18 +497,20 @@ class Assembler {
 
   // MxGridFieldInterpolator.cpp:28-122: `field` of the simulation `from` interpolated at the DOFs of this simulation
   // (rows: this simulation's map, columns: from's map). Both live on the same executor.
+  // bloch: stencil cells that wrap across a periodic face carry the Bloch factor (mxy::InterpRow; DESIGN.md GMG-bloch).
   template <class S>
-  Csr<S> interpolatorFrom(Assembler& from, int field) {
+  Csr<S> interpolatorFrom(Assembler& from, int field, bool bloch = false) {
     requireSetUp();
-    return interpolatorRows<S>(from, field, mxy::oneRun(0, h_.f[field].nLoc));
+    return interpolatorRows<S>(from, field, mxy::oneRun(0, h_.f[field].nLoc), bloch);
   }
   // ... on the rows `rows` of this simulation's map
   template <class S>
-  Csr<S> interpolatorRows(Assembler& from, int field, const mxy::RowRuns& rows) {
+  Csr<S> interpolatorRows(Assembler& from, int field, const mxy::RowRuns& rows, bool bloch = false) {
     requireSetUp();
     from.requireSetUp();
+    if (bloch) checkBlochTransfer(from, std::is_same<S, double>::value);
     using Fn = mxy::AtRows<mxy::InterpRow<S>>;
-    Csr<S> m = buildRows<S>(rows.size(), from.h_.f[field].nLoc, Fn{mxy::InterpRow<S>{from.dSim_, dSim_, field}, rows});
+    Csr<S> m = buildRows<S>(rows.size(), from.h_.f[field].nLoc, Fn{mxy::InterpRow<S>{from.dSim_, dSim_, field, bloch ? 1 : 0}, rows});
     m.setRuns(rows, h_.f[field].nLoc);
     m.rowField = field;
     m.colField = field;
@@ -518,9 +522,10 @@ class Assembler {
   // each side, and only its entries in the columns [c0, c1) are transposed. The margin planes must contribute nothing
   // to the window; if they do, the derivation of the fine rows was wrong and the rows would be short.
   template <class S>
-  Csr<S> interpolatorTransposeRows(Assembler& from, int field, int64_t c0, int64_t c1) {
+  Csr<S> interpolatorTransposeRows(Assembler& from, int field, int64_t c0, int64_t c1, bool bloch = false) {
     requireSetUp();
     from.requireSetUp();
+    if (bloch) checkBlochTransfer(from, std::is_same<S, double>::value);
     const mxy::Grid& gf = h_.g;
     const mxy::Grid& gc = from.h_.g;
     const mxy::Field& ff = h_.f[field];
@@ -556,7 +561,7 @@ class Assembler {
     } else if (len > 0) {
       first = 0; len = P;
     }
-    Csr<S> p = interpolatorRows<S>(from, field, planeRows(field, first, len));
+    Csr<S> p = interpolatorRows<S>(from, field, planeRows(field, first, len), bloch);
     struct Owned {
       Assembler* a; Csr<S>* x;
       ~Owned() { a->destroy(*x); }
@@ -800,6 +805,13 @@ class Assembler {
     x_.toExec(d, shape.nodes.data(), shape.nodes.size() * sizeof(ShapeNode));
     return d;
   }
+  // A Bloch-consistent transfer needs complex entries unless every phase is 0 (then it equals the plain transfer bit for
+  // bit), and both grids must carry the same phases.
+  void checkBlochTransfer(const Assembler& from, bool realScalar) const {
+    for (int i = 0; i < 3; ++i)
+      if (from.phase_[i] != phase_[i]) throw std::runtime_error("Bloch transfer: the two simulations have different phase shifts");
+    if (realScalar && from.complex_) throw std::runtime_error("Bloch transfer: non-zero phase shifts need a complex interpolator");
+  }
   void requireSetUp() const {
     if (!setUp_) throw std::runtime_error("the simulation has not been set up (mxg_sim_setup)");
   }
@@ -815,6 +827,7 @@ class Assembler {
   Shape pec_;             // kept for the D-field fractions a later dielectric needs
   std::vector<int64_t> planeStart_[mxy::NUM_FIELDS];   // first map position of x-planes 0 .. N0 + 1, per field
   bool hasPEC_ = false, setUp_ = false, complex_ = false;
+  double phase_[3] = {0.0, 0.0, 0.0};   // Bloch phase shifts per direction
 };
 
 }  // namespace mxa

@@ -604,12 +604,19 @@ MXY_HD int32_t fetchInc(int32_t* p) {
 // a field of the `from` grid at the component positions of the `to` grid. Entries whose column is not a DOF are
 // dropped, then the row is divided by the sum of the magnitudes of what is left. (The reference's unset stencil point
 // and never-zeroed row-sum accumulator are not reproduced, DESIGN.md R12.)
+//
+// bloch != 0 (DESIGN.md GMG-bloch, not in the reference): a stencil cell that wraps across a PERIODIC face of the coarse
+// grid carries that direction's Bloch factor, e^{+i phi} from the top (cell >= N, ACT_MUL) and e^{-i phi} from below
+// (cell < 0, ACT_DIV), looked up in the coarse field's factor table, so that P maps a coarse Bloch-periodic field onto
+// the fine one. PEC / PMC images get no factor here. The row-sum normalisation still uses the weights, and entries of
+// weight 0 keep the value +0 (a factor would give them the signs of its parts).
 template <class S>
 struct InterpRow {
   static constexpr int kMax = 8;
   const Sim* from;
   const Sim* to;
   int kind;
+  int bloch;
   MXY_HD int operator()(int64_t row, int32_t* cols, S* vals) const {
     const Sim& sf = *from;
     const Sim& st = *to;
@@ -641,6 +648,16 @@ struct InterpRow {
           if (l < 0) continue;
           cols[n] = l;
           vals[n] = fromParts<S>(w, 0.0);
+          if (bloch && w != 0.0) {            // a zero weight stays (+0, +0), whatever the factor's signs
+            int code = 0;
+            for (int i = 0; i < 3; ++i) {
+              int act = ACT_NONE;
+              if (cell[i] < 0) { if (ff.lbc[comp][i] == PERIODIC) act = ACT_DIV; }
+              else if (cell[i] >= sf.g.N[i]) { if (ff.ubc[comp][i] == PERIODIC) act = ACT_MUL; }
+              code = code * 5 + act;
+            }
+            vals[n] = mulS(fromParts<S>(ff.facRe[code], ff.facIm[code]), vals[n]);
+          }
           ++n;
           sum += absD(w);
         }
